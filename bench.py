@@ -4,6 +4,8 @@
     python bench.py --gpus N --steps K --warmup W                    # this repo's CUDA path (default config: africa)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's own code on the host CPU
     python bench.py --config fern|lego ...                           # BASELINE.json configs[3] / configs[4]
+    python bench.py ... --dump-outputs DIR                           # + the last timed step's maps as DIR/*.npy
+                                                                     # (rank 0's rays only when N > 1)
 
 Configs (BASELINE.json `configs`; SURVEY §8(d)):
   africa  configs[1]: 512x512 image, N=128 samples, K=32, one image per GPU per step (weak scaling, no collective), plus
@@ -44,6 +46,7 @@ sys.path.insert(0, ROOT)
 # limits it (scripts/experiments/k1_precision_sim.py).
 RENDER_PRECISION = "fp16"
 N_VIEWS_LEGO = 200
+DUMP_BYTES = 64_000_000          # --dump-outputs: all files together stay below this
 
 CONFIGS = {
     "africa": dict(H=512, W=512, focal=443.4, near=1.2, far=8.0, ndc=False, Nc=128, Nf=0, K=32, white_bkgd=False,
@@ -166,6 +169,27 @@ def ncu_dram_traffic(summary_csv: str, block: int = 0):
         if max(blocks, 0) == block and len(f) == 3 and f[0] in ("dram__bytes_read.sum", "dram__bytes_write.sum"):
             tot += float(f[2]) * mult.get(f[1], 1.0)
     return tot or None
+
+
+def dump_outputs(out_dir: str, chunks, limit: int = DUMP_BYTES, seed: int = 0) -> tuple[int, int]:
+    """Write what one render step returned (the dicts of its render_rays calls, concatenated along the ray axis) as
+    <out_dir>/<key>.npy in float32.  When the arrays together would exceed `limit` bytes, every array keeps the same
+    rows: a fixed, seeded, sorted sample of the rays, so that two builds run with the same arguments write the same
+    rays.  Returns (rays written, rays rendered)."""
+    import numpy as np
+    keys = sorted(chunks[0])
+    B = sum(c[keys[0]].shape[0] for c in chunks)
+    per_ray = sum(4 * math.prod(chunks[0][k].shape[1:]) for k in keys)
+    n = min(B, (limit - 4096) // per_ray)          # 4096: room for the .npy headers
+    rows = None if n == B else torch.randperm(B, generator=torch.Generator().manual_seed(seed))[:n].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    for k in keys:
+        a = torch.cat([c[k] for c in chunks], 0)
+        assert a.is_floating_point(), (k, a.dtype)
+        if rows is not None:
+            a = a[rows.to(a.device)]
+        np.save(os.path.join(out_dir, k + ".npy"), a.float().cpu().numpy())
+    return n, B
 
 
 def host_threads() -> int:
@@ -433,8 +457,13 @@ def main():
                     help="GEMM engine of the training legs: bf16 storage + kind::f16 (BASELINE configs[2] wording), "
                          "tf32 over fp32 storage, or the fp32 CUDA-core check engine")
     ap.add_argument("--no-graph", action="store_true", help="launch the training step eagerly instead of replaying CUDA graphs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed render steps, write the maps the last one returned as DIR/<name>.npy (float32; "
+                         f"rank 0; a fixed seeded sample of the rays when all of them exceed {DUMP_BYTES / 1e6:.0f} MB)")
     args = ap.parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the CUDA path; it has no meaning with --impl reference")
         return run_reference(args)
 
     import torch.distributed as dist
@@ -505,13 +534,19 @@ def main():
     barrier()
     timer.on = True
     ev0.record()
+    outs = None
     for s in range(args.steps):
-        render_device(views_dev[(W_ + s) % len(views_dev)])
+        del outs            # the previous step's maps go back to the allocator first, as in the warm-up loop
+        outs = render_device(views_dev[(W_ + s) % len(views_dev)])
     ev1.record()
     barrier()
     timer.on = False
     ms = ev0.elapsed_time(ev1)
     k1_ms, k1_points, n_k1 = timer.total_ms(), timer.points, len(timer.events)
+    if args.dump_outputs and rank == 0 and outs:
+        n, n_all = dump_outputs(args.dump_outputs, outs)
+        sys.stderr.write(f"bench: wrote the maps of {n} of the {n_all} rays of the last timed step to {args.dump_outputs}\n")
+    del outs
 
     # ---- end to end through the public API: pinned host rays in, K fields + statistics out ----
     out_host = None

@@ -153,6 +153,33 @@ def test_bench_workloads_and_flop_accounting():
     assert abs(float(p[:, 3].norm()) - 4.0) < 1e-4                                                     # radius of pose_spherical
 
 
+def test_bench_dump_outputs_sample_is_seeded_and_bounded(tmp_path):
+    """bench.py --dump-outputs: the chunks of one step concatenated along the rays, float32; over the byte limit every
+    array keeps the same seeded sample of rows, identical from run to run."""
+    import numpy as np
+
+    import bench
+    g = torch.Generator().manual_seed(0)
+    chunks = [{"rgb_map": torch.rand(n, 3, 4, generator=g), "depth_map": torch.rand(n, 4, generator=g),
+               "kstats": torch.rand(n, 8, generator=g)} for n in (5, 7)]
+    full = {k: torch.cat([c[k] for c in chunks], 0).numpy() for k in chunks[0]}
+    assert bench.dump_outputs(str(tmp_path / "all"), chunks) == (12, 12)
+    for k, v in full.items():
+        a = np.load(tmp_path / "all" / f"{k}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, v), k
+    per_ray = 4 * (12 + 4 + 8)
+    limit = 4096 + 5 * per_ray
+    dirs = [tmp_path / "a", tmp_path / "b"]
+    for d in dirs:
+        assert bench.dump_outputs(str(d), chunks, limit=limit) == (5, 12)
+    assert sum(f.stat().st_size for f in dirs[0].iterdir()) <= limit
+    rows = [int(np.nonzero((full["kstats"] == r).all(-1))[0][0]) for r in np.load(dirs[0] / "kstats.npy")]
+    assert rows == sorted(set(rows)) and len(rows) == 5
+    for k, v in full.items():
+        a, b = np.load(dirs[0] / f"{k}.npy"), np.load(dirs[1] / f"{k}.npy")
+        assert np.array_equal(a, b) and np.array_equal(a, v[rows]), k
+
+
 def test_oracle_ref_staging_is_byte_identical():
     """oracle/_ref (git-ignored) is a byte-for-byte copy of the reference's *.py files when it exists."""
     from oracle import build_ref

@@ -598,6 +598,40 @@ def test_bench_dtype_network_stage_on_the_stressed_golden(cf, dev):
     assert e_mine <= max(5e-2, 100 * e_ref)      # per-(point, k) values; the rendered statistics carry the 2e-3 bar above
 
 
+def test_bench_times_the_given_steps_and_dumps_what_they_rendered(cf, dev, tmp_path):
+    """bench.py --steps 2 times two render steps (one network launch per chunk each) and --dump-outputs writes the maps of
+    the last one: a seeded sample of the image's rays within the byte limit, equal to rendering those rays here."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    import bench
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = tmp_path / "dump"
+    res = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "1", "--no-train",
+                          "--no-kernels", "--no-cpu-baseline", "--dump-outputs", str(out)],
+                         capture_output=True, text=True, timeout=900)
+    assert res.returncode == 0, res.stderr[-4000:]
+    line = json.loads(res.stdout.strip().splitlines()[-1])
+    B, chunk = line["config"]["rays_per_step_per_gpu"], line["config"]["chunk_rays"]
+    assert line["steps"] == 2 and line["roofline"]["launches_timed"] == 2 * ((B + chunk - 1) // chunk)
+    files = {f.stem: np.load(f) for f in out.iterdir()}
+    assert set(files) == {"rgb_map", "disp_map", "depth_map", "kstats"}
+    assert sum(f.stat().st_size for f in out.iterdir()) <= bench.DUMP_BYTES
+    n = files["kstats"].shape[0]
+    assert 0 < n < B and all(a.dtype == np.float32 and a.shape[0] == n for a in files.values())
+    rows = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:n].sort().values
+    cfg = O.CfnConfig(K=bench.CONFIGS["africa"]["K"])
+    net = make_net(cf, cfg, O.make_params(cfg, 0, "default"), *O.make_latents(cfg, 0), dev)
+    rays = bench.image_rays_host("africa", 0).to(dev)
+    mine = [cf.render_rays(rays[i:i + chunk], net, None, 128, False, False, K_samples=cfg.K,
+                           precision=bench.RENDER_PRECISION, want_kstats=True) for i in range(0, B, chunk)]
+    for k, a in files.items():
+        full = torch.cat([m[k] for m in mine], 0)[rows.to(dev)].cpu()
+        assert (full - torch.from_numpy(a)).abs().max().item() <= 1e-6, k
+
+
 # ------------------------------------------------------------------------------------------------
 # F2: ray generation from a pose (render(..., c2w=pose))
 # ------------------------------------------------------------------------------------------------
