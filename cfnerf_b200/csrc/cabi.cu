@@ -1,8 +1,6 @@
 // C-ABI entry points (include/cfnerf_b200.h): handle lifetime, parameter table, argument checking and
 // dispatch to the kernels.  No torch types, no hidden device allocation outside create/pack.
 #include <stdarg.h>
-#include <stdlib.h>
-#include <string.h>
 
 #include "handle.h"
 
@@ -19,7 +17,7 @@ void set_error(const char* fmt, ...) {
 using namespace cfn;
 
 extern "C" const char* cfn_last_error(void) { return g_err; }
-extern "C" int cfn_version(void) { return 100; }
+extern "C" int cfn_version(void) { return 101; }
 
 static void add_slot(CfnHandle* h, const std::string& name, int rows, int cols) {
   ParamSlot s;
@@ -58,22 +56,16 @@ extern "C" int cfn_create(const CfnConfig* cfg, CfnHandle** out) {
   h->packed = false;
   h->tc = nullptr;
   h->tc_dirty = 0;
-  h->zero_lo = h->zero_hi = nullptr;
   h->deterministic = 0;
   h->det_scratch = nullptr;
   h->det_floats = 0;
   h->gemm_tc = (cfg->precision != CFN_PREC_FP32) ? 1 : 0;
-  if (const char* e = getenv("CFN_TRAIN_GEMM")) {   // experiments: "fp32" forces the CUDA-core GEMMs, "tf32" the tensor cores
-    if (!strcmp(e, "fp32")) h->gemm_tc = 0;
-    if (!strcmp(e, "tf32")) h->gemm_tc = 1;
-  }
   h->gp = (h->in_pos + 7) & ~7;
   h->gd = (h->in_dir + 7) & ~7;
   // bf16 storage of the layer-by-layer chain (training in CFN_PREC_BF16): every row stride / column offset must be a
   // multiple of 8 elements (16 bytes); other widths keep the fp32-storage tf32 chain
   h->chain_bf16 = (h->gemm_tc && cfg->precision == CFN_PREC_BF16 && cfg->W % 16 == 0 && cfg->h_alpha % 8 == 0 &&
                    cfg->h_rgb % 8 == 0) ? 1 : 0;
-  if (const char* e = getenv("CFN_TRAIN_GEMM")) if (!strcmp(e, "tf32") || !strcmp(e, "fp32")) h->chain_bf16 = 0;
   h->wg = h->amA_g = h->amC_g = nullptr;
   const int W = cfg->W, F = cfg->F;
   add_slot(h, "alpha_mean", 1, 1);
@@ -302,21 +294,6 @@ extern "C" int cfn_network_bwd(CfnHandle* h, const float* g_flow_params, int64_t
     return CFN_ENOMEM;
   }
   return chain_network_bwd(h, g_flow_params, B, N, (float*)workspace, grads, (cudaStream_t)stream);
-}
-
-extern "C" int cfn_network_bwd_part(CfnHandle* h, const float* g_flow_params, int64_t B, int N, void* workspace,
-                                    size_t workspace_bytes, float* const* grads, int n_params, int part, int split_layer,
-                                    void* stream) {
-  CFN_CHECK_ARG(h && g_flow_params && grads && workspace, "cfn_network_bwd_part: null argument");
-  CFN_CHECK_ARG(n_params == (int)h->slots.size(), "cfn_network_bwd_part: expected %d tensors", (int)h->slots.size());
-  CFN_CHECK_ARG(part == 1 || part == 2, "cfn_network_bwd_part: part must be 1 or 2");
-  size_t need = 0;
-  cfn_workspace_bytes(h, B * N, 1, &need);
-  if (workspace_bytes < need) {
-    set_error("cfn_network_bwd_part: workspace %zu bytes < required %zu", workspace_bytes, need);
-    return CFN_ENOMEM;
-  }
-  return chain_network_bwd(h, g_flow_params, B, N, (float*)workspace, grads, (cudaStream_t)stream, part, split_layer);
 }
 
 extern "C" int cfn_flow_composite_fwd(CfnHandle* h, const float* flow_params, const float* z_vals,

@@ -463,9 +463,8 @@ int launch_flow_composite_fwd(int fast_math, int F, int K, const float* globals,
   size_t smem = fwd_smem_bytes(F, N);
   unsigned grid = (unsigned)((B + 3) / 4);
   const bool train = logdet_sums != nullptr;
-  // small training batches: four warps per ray (see flow_composite_fwd_seg4_kernel); CFN_K2_SEG4=0 keeps one warp per ray
-  static const int seg4_env = [] { const char* e = getenv("CFN_K2_SEG4"); return e ? atoi(e) : 1; }();
-  if (train && seg4_env && trans && seg_sums && n_seg == 4 && N % 4 == 0 && !weights && !kstats && B <= 1536 && F <= 4) {
+  // small training batches: four warps per ray (see flow_composite_fwd_seg4_kernel)
+  if (train && trans && seg_sums && n_seg == 4 && N % 4 == 0 && !weights && !kstats && B <= 1536 && F <= 4) {
     const size_t sm4 = ((size_t)4 * ((kChunk * 18 * F + 3) & ~3) + 2 * (size_t)N + 4 * 32 + 4 * 5 * 32 + 8) * sizeof(float);
 #define CFN_SEG4_LAUNCH(FASTM, FTT)                                                                                  \
     do {                                                                                                             \

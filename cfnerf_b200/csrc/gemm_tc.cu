@@ -24,7 +24,6 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 
-#include <cstdlib>
 #include <math.h>
 
 #include "common.cuh"
@@ -601,11 +600,9 @@ bool tgemm_supported(const GemmArgs& g) {
 
 // tile / split / stage geometry of one GEMM
 static void plan_tgemm(const GemmArgs& g, TgParams& p, int& CG, bool& a_mn, bool& b_mn, size_t& smem) {
-  static int cg_env = -1;
-  if (cg_env < 0) { const char* e = getenv("CFN_TG_CTA_GROUP"); cg_env = e ? atoi(e) : 2; if (cg_env != 1) cg_env = 2; }
   a_mn = (g.a_cs != 1);
   b_mn = (g.b_rs != 1);
-  CG = (g.M <= 128) ? 1 : cg_env;
+  CG = (g.M <= 128) ? 1 : 2;
   p = TgParams{};
   p.C = g.C; p.c_rs = g.c_rs; p.bias = g.bias; p.aux = g.aux; p.aux_rs = g.aux_rs;
   p.M = g.M; p.N = g.N; p.K = g.K;

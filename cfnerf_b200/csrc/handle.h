@@ -63,9 +63,6 @@ struct CfnHandle {
   std::vector<int64_t> wg_offset;   // in 4-byte slots
   float* amA_g; float* amC_g;   // operand copies of amA / amC (tf32-rounded when gemm_tc, else aliases)
 
-  // transient, set by chain_network_bwd: the gradient range that one memset already zeroed (flat gradient buckets)
-  const float* zero_lo; const float* zero_hi;
-
   // opt-in deterministic weight gradients (cfn_set_deterministic): scratch for the split-K slabs of one wgrad
   int deterministic;
   float* det_scratch; int64_t det_floats;
@@ -79,10 +76,8 @@ namespace cfn {
 size_t chain_workspace_floats(const CfnHandle* h, int64_t n_points, int save);
 int chain_network_fwd(CfnHandle* h, const float* rays, const float* z_vals, const float* pts, const float* viewdirs,
                      int64_t B, int N, float* flow_params, float* ws, int save, cudaStream_t s);
-// part 0: the whole backward.  part 1: everything down to and including the weight gradient of trunk layer `split_layer`
-// (then the gradients of every parameter from that layer on are final); part 2: the rest (trunk layers below it).
-int chain_network_bwd(CfnHandle* h, const float* g_flow_params, int64_t B, int N, float* ws, float* const* grads,
-                     cudaStream_t s, int part = 0, int split_layer = 0);
+int chain_network_bwd(const CfnHandle* h, const float* g_flow_params, int64_t B, int N, float* ws, float* const* grads,
+                      cudaStream_t s);
 int pack_fp32(CfnHandle* h, const float* const* params, cudaStream_t s);
 
 // tensor-core path (mlp_tc.cu)

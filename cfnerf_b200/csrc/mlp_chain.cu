@@ -410,13 +410,17 @@ static int colsum(const float* g, int64_t ld, int64_t M, int N, float* out, cuda
   return CFN_OK;
 }
 
+// gradient range [lo, hi) that a single memset at the start of chain_network_bwd already zeroed (flat gradient buckets)
+struct Zeroed {
+  const float* lo = nullptr; const float* hi = nullptr;
+  bool has(const float* q) const { return lo && q >= lo && q < hi; }
+};
+
 // dW(out x in) = G(M x out)^T X(M x in), split over the point dimension, atomically accumulated into zeroed dW
 // db (optional): the bias gradient = column sums of G, fused into the tensor-core GEMM when possible
 static int wgrad(const CfnHandle* h, const float* G, int64_t ldg, int out_f, const float* X, int64_t ldx, int in_f, int64_t M,
-                 float* dW, float* db, cudaStream_t s) {
-  // gradient tensors that sit in one flat buffer were zeroed by a single memset at the start of chain_network_bwd
-  auto prezeroed = [&](const float* q) { return h->zero_lo && q >= h->zero_lo && q < h->zero_hi; };
-  if (!h->deterministic && !prezeroed(dW)) CFN_CUDA(cudaMemsetAsync(dW, 0, (size_t)out_f * in_f * sizeof(float), s));
+                 float* dW, float* db, const Zeroed& zeroed, cudaStream_t s) {
+  if (!h->deterministic && !zeroed.has(dW)) CFN_CUDA(cudaMemsetAsync(dW, 0, (size_t)out_f * in_f * sizeof(float), s));
   GemmArgs g{};
   g.A = G; g.a_rs = 1; g.a_cs = ldg;        // A(m=o, k=pt) = G[pt*ldg + o]
   g.B = X; g.b_rs = ldx; g.b_cs = 1;        // B(k=pt, n=i) = X[pt*ldx + i]
@@ -444,7 +448,7 @@ static int wgrad(const CfnHandle* h, const float* G, int64_t ldg, int out_f, con
   if (h->deterministic) { g.partials = h->det_scratch; g.partials_floats = h->det_floats; }
   if (db) {
     if (h->gemm_tc && tgemm_can_rowsum(g)) {
-      if (!h->deterministic && !prezeroed(db)) CFN_CUDA(cudaMemsetAsync(db, 0, (size_t)out_f * sizeof(float), s));
+      if (!h->deterministic && !zeroed.has(db)) CFN_CUDA(cudaMemsetAsync(db, 0, (size_t)out_f * sizeof(float), s));
       g.rowsum = db;
     } else if (h->chain_bf16) {
       set_error("bf16 chain: the bias gradient could not be fused into the wgrad (out %d in %d)", out_f, in_f);
@@ -460,11 +464,11 @@ static int wgrad(const CfnHandle* h, const float* G, int64_t ldg, int out_f, con
 // weight gradient of parameter slot `slot` (an nn.Linear whose input rows are X): straight into grads[slot] when the
 // operand view is unpadded, otherwise through the padded scratch and two strided copies that drop the pad columns
 static int wgrad_slot(const CfnHandle* h, int slot, const float* G, int64_t ldg, const float* X, int64_t ldx, int64_t M,
-                      float* dW, float* db, float* scratch, cudaStream_t s) {
+                      float* dW, float* db, float* scratch, const Zeroed& zeroed, cudaStream_t s) {
   const ParamSlot& w = h->slots[slot];
   const WView& v = h->wv[slot];
-  if (v.ld == w.cols) return wgrad(h, G, ldg, w.rows, X, ldx, w.cols, M, dW, db, s);
-  int rc = wgrad(h, G, ldg, w.rows, X, ldx, v.ld, M, scratch, db, s);
+  if (v.ld == w.cols) return wgrad(h, G, ldg, w.rows, X, ldx, w.cols, M, dW, db, zeroed, s);
+  int rc = wgrad(h, G, ldg, w.rows, X, ldx, v.ld, M, scratch, db, zeroed, s);
   if (rc) return rc;
   const int first = v.gap_at < w.cols ? v.gap_at : w.cols;
   if (first > 0)
@@ -509,12 +513,9 @@ __global__ void scatter_rows_kernel(const float* __restrict__ dAm, const float* 
   if (gb && threadIdx.x == 0) gb[row] = dAb[r];
 }
 
-int chain_network_bwd(CfnHandle* h, const float* g_flow_params, int64_t B, int N, float* ws, float* const* grads,
-                     cudaStream_t s, int part, int split_layer) {
+int chain_network_bwd(const CfnHandle* h, const float* g_flow_params, int64_t B, int N, float* ws, float* const* grads,
+                      cudaStream_t s) {
   const int64_t M = B * N;
-  CFN_CHECK_ARG(part >= 0 && part <= 2 && (part == 0 || (split_layer >= 1 && split_layer < h->cfg.D)),
-                "cfn_network_bwd_part: part %d / split layer %d out of range (1..%d)", part, split_layer, h->cfg.D - 1);
-  const bool head_phase = part != 2;      // parts 0 and 1 start at the flow records; part 2 resumes inside the trunk
   const int W = h->cfg.W, D = h->cfg.D, F = h->cfg.F, PP = h->PP;
   const int ha_n = h->cfg.h_alpha, hr_n = h->cfg.h_rgb;
   ChainLayout L = make_layout(h, M, 1);
@@ -525,7 +526,7 @@ int chain_network_bwd(CfnHandle* h, const float* g_flow_params, int64_t B, int N
   float* dAb = dAm + (int64_t)PP * (ha_n > hr_n ? ha_n : hr_n);   // (rows) gathered bias grads
 
   // 1. through the tanh on the diagonals
-  if (head_phase) {
+  {
     int64_t total = M * PP;
     tanh_bwd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(g_flow_params, ws + L.P, h->tanh_flags, ws + L.GP,
                                                                     total, PP, 3 * F, L.gpa, L.ldGP,
@@ -557,20 +558,20 @@ int chain_network_bwd(CfnHandle* h, const float* g_flow_params, int64_t B, int N
 
   // Gradient tensors laid out back to back in slot order (cfnerf_b200.dist.FusedTrainStep's flat bucket): ONE memset
   // replaces the ~40 per-tensor ones of the split-K wgrads (each a graph node / launch of its own at 512 rays per step)
-  if (head_phase) h->zero_lo = h->zero_hi = nullptr;
-  if (head_phase) {
+  Zeroed zeroed;
+  {
     bool flat = true;
     for (size_t i = 5; i < h->slots.size(); ++i)
       flat = flat && (grads[i] == grads[4] + (h->slots[i].offset - h->slots[4].offset));
     if (flat) {
       const int64_t n = h->n_floats - h->slots[4].offset;
       CFN_CUDA(cudaMemsetAsync(grads[4], 0, (size_t)n * sizeof(float), s));
-      h->zero_lo = grads[4];
-      h->zero_hi = grads[4] + n;
+      zeroed.lo = grads[4];
+      zeroed.hi = grads[4] + n;
     }
   }
   // zero every flow-conditioning gradient: rows the path never reads keep an exact 0 (SURVEY §0 fact 5)
-  if (head_phase && !h->zero_lo)
+  if (!zeroed.lo)
     for (int base : {h->s_frgb, h->s_falpha})
       for (int j = 0; j < 8; ++j)
         CFN_CUDA(cudaMemsetAsync(grads[base + j], 0, h->slots[base + j].numel * sizeof(float), s));
@@ -580,9 +581,9 @@ int chain_network_bwd(CfnHandle* h, const float* g_flow_params, int64_t B, int N
   for (size_t i = 0; i < 64; ++i) table.p[i] = i < h->slots.size() ? grads[i] : nullptr;
 
   // 2. alpha conditioning branch
-  if (head_phase) {
+  {
     // gathered dAmA = GP[:, :3F]^T ha ; bias = colsum
-    if ((rc = wgrad(h, GPa, ldGP, 3 * F, ws + L.ha, ha_n, ha_n, M, dAm, dAb, s))) return rc;
+    if ((rc = wgrad(h, GPa, ldGP, 3 * F, ws + L.ha, ha_n, ha_n, M, dAm, dAb, zeroed, s))) return rc;
     scatter_rows_kernel<<<3 * F, 64, 0, s>>>(dAm, dAb, ha_n, h->gatherA_dev, 3 * F, table);
     CFN_LAUNCH_CHECK();
     // g_ha = GP[:, :3F] amA
@@ -592,13 +593,13 @@ int chain_network_bwd(CfnHandle* h, const float* g_flow_params, int64_t B, int N
     g.C = gha; g.c_rs = ld_gha; g.M = M; g.N = ha_n; g.K = 3 * F; g.split_k = 1;
     g.ab_bf16 = g.c_bf16 = h->chain_bf16;
     if ((rc = gemm(h, g, 1, s))) return rc;
-    if ((rc = wgrad_slot(h, h->s_halpha, gha, ld_gha, h7, ld7, M, grads[h->s_halpha], grads[h->s_halpha + 1], dWp, s))) return rc;
+    if ((rc = wgrad_slot(h, h->s_halpha, gha, ld_gha, h7, ld7, M, grads[h->s_halpha], grads[h->s_halpha + 1], dWp, zeroed, s))) return rc;
     // g_h7 (unmasked, first contribution) = g_ha W_halpha  -- or, fused, left for the K-concatenated GEMM of step 3
     if (!fuse_heads && (rc = dgrad(h, h->s_halpha, gha, ld_gha, 0, W, G1, W, M, nullptr, 0, 0, s))) return rc;
   }
   // 3. rgb conditioning branch
-  if (head_phase) {
-    if ((rc = wgrad(h, GPc, ldGP, 15 * F, ws + L.hr, hr_n, hr_n, M, dAm, dAb, s))) return rc;
+  {
+    if ((rc = wgrad(h, GPc, ldGP, 15 * F, ws + L.hr, hr_n, hr_n, M, dAm, dAb, zeroed, s))) return rc;
     scatter_rows_kernel<<<15 * F, 64, 0, s>>>(dAm, dAb, hr_n, h->gatherC_dev, 15 * F, table);
     CFN_LAUNCH_CHECK();
     GemmArgs g{};
@@ -607,13 +608,13 @@ int chain_network_bwd(CfnHandle* h, const float* g_flow_params, int64_t B, int N
     g.C = gh; g.c_rs = hr_n; g.M = M; g.N = hr_n; g.K = 15 * F; g.split_k = 1;
     g.ab_bf16 = g.c_bf16 = h->chain_bf16;
     if ((rc = gemm(h, g, 1, s))) return rc;
-    if ((rc = wgrad_slot(h, h->s_hrgb, gh, hr_n, ws + L.v, W / 2, M, grads[h->s_hrgb], grads[h->s_hrgb + 1], dWp, s))) return rc;
+    if ((rc = wgrad_slot(h, h->s_hrgb, gh, hr_n, ws + L.v, W / 2, M, grads[h->s_hrgb], grads[h->s_hrgb + 1], dWp, zeroed, s))) return rc;
     // g_v = (g_hr W_hrgb) * relu'(v)
     if ((rc = dgrad(h, h->s_hrgb, gh, hr_n, 0, W / 2, gv, W / 2, M, ws + L.v, W / 2, 0, s, mbv, L.bwv))) return rc;
-    if ((rc = wgrad_slot(h, h->s_views, gv, W / 2, ws + L.V, L.ldv, M, grads[h->s_views], grads[h->s_views + 1], dWp, s))) return rc;
+    if ((rc = wgrad_slot(h, h->s_views, gv, W / 2, ws + L.V, L.ldv, M, grads[h->s_views], grads[h->s_views + 1], dWp, zeroed, s))) return rc;
     // g_feat = g_v W_view[:, :W]   (gamma(d) columns need no gradient)
     if ((rc = dgrad(h, h->s_views, gv, W / 2, 0, W, G2, ld_g2, M, nullptr, 0, 0, s))) return rc;
-    if ((rc = wgrad_slot(h, h->s_feat, G2, ld_g2, h7, ld7, M, grads[h->s_feat], grads[h->s_feat + 1], dWp, s))) return rc;
+    if ((rc = wgrad_slot(h, h->s_feat, G2, ld_g2, h7, ld7, M, grads[h->s_feat], grads[h->s_feat + 1], dWp, zeroed, s))) return rc;
     if (fuse_heads) {
       // g_h7 = ([g_feat | g_ha] [W_feat ; W_halpha]) * relu'(h7): one GEMM over the concatenated K instead of a second,
       // accumulating one (its read-modify-write of g_h7 cost three times a plain dgrad)
@@ -634,19 +635,10 @@ int chain_network_bwd(CfnHandle* h, const float* g_flow_params, int64_t B, int N
   // 4. trunk, last layer to first
   float* gout = G1;
   float* gin = G2;
-  int i_first = D - 1;
-  if (part == 2) {
-    // resume: layers D-1 .. split_layer swapped the two gradient buffers once per dgrad (D-1-split_layer of them)
-    i_first = split_layer;
-    if ((D - 1 - split_layer) & 1) { gout = G2; gin = G1; }
-  }
-  for (int i = i_first; i >= 0; --i) {
+  for (int i = D - 1; i >= 0; --i) {
     LayerIO io = trunk_io(h, L, ws, M, i, 1);
     const int slot = h->s_pts(i, 0);
-    if (!(part == 2 && i == split_layer)) {     // (part 1 already took this layer's weight gradient)
-      if ((rc = wgrad_slot(h, slot, gout, W, io.in, io.ld_in, M, grads[slot], grads[slot + 1], dWp, s))) return rc;
-    }
-    if (part == 1 && i == split_layer) break;
+    if ((rc = wgrad_slot(h, slot, gout, W, io.in, io.ld_in, M, grads[slot], grads[slot + 1], dWp, zeroed, s))) return rc;
     if (i == 0) break;
     // gradient w.r.t. the previous layer's (post-ReLU) output, masked by its ReLU
     LayerIO prev = trunk_io(h, L, ws, M, i - 1, 1);

@@ -28,7 +28,7 @@ namespace cfn {
 
 // -DCFN_TC_ISSUE_STAMPS=1 (CFN_NVCC_EXTRA of cfnerf_b200/build.py): three clock64() stamps per ring slot in the MMA issuer
 // instead of one — the diagnostic build behind scripts/r2_k1_issue.py; the stamps cost ~10 % of the kernel.
-// -DCFN_TC_TIMELINE=1: the clock64() stamps behind scripts/k1_timeline.py / r2_k1_ring.py (CFN_TC_PROFILE=1 at run time).
+// -DCFN_TC_TIMELINE=1: the clock64() stamps behind scripts/k1_timeline.py (CFN_TC_PROFILE=1 at run time).
 // Compiled OUT by default: predicated off they still cost 1.8 % of the kernel (same-box A/B, 17.36 -> 17.04 ms) - the
 // single-warp producer / issuer loops are that sensitive to their instruction count.
 #ifndef CFN_TC_TIMELINE
@@ -45,6 +45,7 @@ constexpr int TC_SRC_GP = 8, TC_SRC_GD = 9;   // host-side source ids; the devic
 constexpr int TC_THREADS = 384;             // warps 0..7 encode/epilogue, 8 TMEM alloc, 9 (profiling), 10 TMA, 11 MMA
 constexpr int TC_W_ALLOC = 8, TC_W_WATCH = 9, TC_W_TMA = 10, TC_W_MMA = 11;   // the scheduler favours high warp ids
 constexpr int TC_MAX_STAGES = 8;
+constexpr int CG = 2;                       // cta_group::2: every tile of 256 points is shared by a CTA pair
 
 struct TcStep {
   int kind;       // 0: bias+ReLU -> A tile, 1: bias -> A tile, 2: bias (+tanh where flagged) -> flow_params in HBM
@@ -95,7 +96,6 @@ struct TcArgs {
 
 struct TcPlan {
   TcPlanDev dev;
-  int cg;                       // cta_group (1 or 2)
   void* stream_dev;             // packed weight stream (2-byte elements)
   int64_t stream_rows;
   float* table_dev;             // biases + flags
@@ -121,37 +121,27 @@ struct TcPlan {
 // ======================================================================================================
 using namespace ptx;   // mbarrier / cluster / TMA / tcgen05 wrappers shared with gemm_tc.cu (ptx_sm100.cuh)
 
-template <int CG>
 __device__ __forceinline__ void umma(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-  if (CG == 1)
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                 "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-                 :: "r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
-  else
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                 "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-                 :: "r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
+  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+               "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+               :: "r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
 }
 
 // The four K=16 instructions of one 64-column K chunk in ONE asm block: the descriptors differ only in the start
 // address field (+2 per 32 bytes of K), so the block takes the two low words and builds everything else itself.
-template <int CG>
 __device__ __forceinline__ void umma_k64(uint32_t d_tmem, uint32_t a_lo, uint32_t b_lo, uint32_t desc_hi, uint32_t idesc,
                                          uint32_t accumulate) {
-#define CFN_MMA4(GRP)                                                                                         \
-  asm volatile("{\n\t.reg .pred p, t;\n\t.reg .b64 da, db;\n\t.reg .b32 xa, xb;\n\t"                          \
-               "setp.ne.b32 p, %5, 0;\n\tsetp.eq.b32 t, %5, %5;\n\t"                                         \
-               "mov.b64 da, {%1, %3};\n\tmov.b64 db, {%2, %3};\n\t"                                          \
-               "tcgen05.mma.cta_group::" GRP ".kind::f16 [%0], da, db, %4, p;\n\t"                            \
-               "add.u32 xa, %1, 2;\n\tadd.u32 xb, %2, 2;\n\tmov.b64 da, {xa, %3};\n\tmov.b64 db, {xb, %3};\n\t" \
-               "tcgen05.mma.cta_group::" GRP ".kind::f16 [%0], da, db, %4, t;\n\t"                            \
-               "add.u32 xa, %1, 4;\n\tadd.u32 xb, %2, 4;\n\tmov.b64 da, {xa, %3};\n\tmov.b64 db, {xb, %3};\n\t" \
-               "tcgen05.mma.cta_group::" GRP ".kind::f16 [%0], da, db, %4, t;\n\t"                            \
-               "add.u32 xa, %1, 6;\n\tadd.u32 xb, %2, 6;\n\tmov.b64 da, {xa, %3};\n\tmov.b64 db, {xb, %3};\n\t" \
-               "tcgen05.mma.cta_group::" GRP ".kind::f16 [%0], da, db, %4, t;\n\t}"                           \
-               :: "r"(d_tmem), "r"(a_lo), "r"(b_lo), "r"(desc_hi), "r"(idesc), "r"(accumulate) : "memory")
-  if (CG == 1) CFN_MMA4("1"); else CFN_MMA4("2");
-#undef CFN_MMA4
+  asm volatile("{\n\t.reg .pred p, t;\n\t.reg .b64 da, db;\n\t.reg .b32 xa, xb;\n\t"
+               "setp.ne.b32 p, %5, 0;\n\tsetp.eq.b32 t, %5, %5;\n\t"
+               "mov.b64 da, {%1, %3};\n\tmov.b64 db, {%2, %3};\n\t"
+               "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %4, p;\n\t"
+               "add.u32 xa, %1, 2;\n\tadd.u32 xb, %2, 2;\n\tmov.b64 da, {xa, %3};\n\tmov.b64 db, {xb, %3};\n\t"
+               "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %4, t;\n\t"
+               "add.u32 xa, %1, 4;\n\tadd.u32 xb, %2, 4;\n\tmov.b64 da, {xa, %3};\n\tmov.b64 db, {xb, %3};\n\t"
+               "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %4, t;\n\t"
+               "add.u32 xa, %1, 6;\n\tadd.u32 xb, %2, 6;\n\tmov.b64 da, {xa, %3};\n\tmov.b64 db, {xb, %3};\n\t"
+               "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %4, t;\n\t}"
+               :: "r"(d_tmem), "r"(a_lo), "r"(b_lo), "r"(desc_hi), "r"(idesc), "r"(accumulate) : "memory");
 }
 
 // two fp32 -> packed 16-bit pair (lo = element c, hi = element c+1), optional fused ReLU
@@ -255,7 +245,7 @@ __device__ __forceinline__ void encode_row(float x, float y, float z, int L, uin
   }
 }
 
-template <int CG, bool FP16>
+template <bool FP16>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 mlp_tc_kernel(const __grid_constant__ CUtensorMap tm_big, const __grid_constant__ CUtensorMap tm_small,
               const __grid_constant__ CUtensorMap tm_bias,
@@ -274,12 +264,12 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tm_big, const __grid_constant_
   // the shuffle tells the compiler that `warp` is warp-uniform: the role branches below are then uniform branches and
   // the schedule arithmetic of the producer / issuer warps lives in the uniform datapath (no R2UR in front of every MMA)
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
-  const uint32_t rank = (CG == 2) ? cluster_ctarank() : 0u;
+  const uint32_t rank = cluster_ctarank();
   const int64_t unit0 = blockIdx.x / CG, n_grid_units = gridDim.x / CG;
 
   // barrier addresses: local (shared::cta) and as seen on the pair's leader (shared::cluster)
   auto bar_local = [&](const uint64_t* b) { return smem_u32(b); };
-  auto bar_leader = [&](const uint64_t* b) { return (CG == 2) ? mapa_rank(smem_u32(b), 0) : smem_u32(b); };
+  auto bar_leader = [&](const uint64_t* b) { return mapa_rank(smem_u32(b), 0); };
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < TC_MAX_STAGES; ++s) { mbar_init(bar_local(&bars->full[s]), CG); mbar_init(bar_local(&bars->empty[s]), 1); }
@@ -293,20 +283,18 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tm_big, const __grid_constant_
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == TC_W_ALLOC) {
-    if (CG == 1) {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(&bars->tmem_ptr)), "r"(512) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(&bars->tmem_ptr)), "r"(512) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(&bars->tmem_ptr)), "r"(512) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
   }
   tc_fence_before();
-  if (CG == 2) cluster_sync_all(); else __syncthreads();
+  cluster_sync_all();
   tc_fence_after();
   const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(&bars->tmem_ptr);
   // All CTA pairs walk the SAME weight stream; started together they hit the same L2 lines at the same instant.
   // A one-off start-up skew (persistent kernel, uniform tiles: the skew persists) spreads the reads over the stream.
+  // CFN_TC_STAGGER sets it and nothing else does, yet the prologue stays: without it the warp-role dispatch below is
+  // compiled differently and K1 ran 0.6 % slower (fp16 17.29-17.32 -> 17.40-17.50 ms per 4.19 M points, same box;
+  // B200 at 1000 W).
   if (a.stagger > 0) {
     const long long t0 = clock64();
     const long long wait = (long long)unit0 * a.stagger;
@@ -328,7 +316,7 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tm_big, const __grid_constant_
           prof.stamp();
           const bool bias_tile = (st.kinfo[blk % st.n_k] >> 24) & 1u;
           if (elect_one()) {
-            const uint32_t full_bar = bar_local(&bars->full[stage]);   // peer bit cleared inside tma_load_2d (CG == 2)
+            const uint32_t full_bar = bar_local(&bars->full[stage]);   // peer bit cleared inside tma_load_2d
             const int row_g = st.row0 + blk * st.n_part + (int)rank * rows;
             const uint32_t dst = stage_base + (uint32_t)stage * a.stage_bytes;
             if (bias_tile) {
@@ -432,13 +420,13 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tm_big, const __grid_constant_
               if (elect_one()) {
                 const uint32_t nks = (info >> 16) & 0xfu;
                 const uint32_t acc = kc > 0 ? 1u : 0u;
-                if (nks == 4u) umma_k64<CG>(d_tmem, a_lo, b_lo, hi128, idesc, acc);
+                if (nks == 4u) umma_k64(d_tmem, a_lo, b_lo, hi128, idesc, acc);
                 else if ((info >> 24) & 1u)   // bias tile: K-major SWIZZLE_32B [rows][16], a single K=16 slice
-                  umma<CG>(d_tmem, ((uint64_t)hi128 << 32) | a_lo, ((uint64_t)hi32 << 32) | b_lo, idesc, acc);
+                  umma(d_tmem, ((uint64_t)hi128 << 32) | a_lo, ((uint64_t)hi32 << 32) | b_lo, idesc, acc);
                 else
                   for (uint32_t ks = 0; ks < nks; ++ks)
-                    umma<CG>(d_tmem, ((uint64_t)hi128 << 32) | (a_lo + 2u * ks), ((uint64_t)hi128 << 32) | (b_lo + 2u * ks), idesc,
-                             (acc || ks > 0) ? 1u : 0u);
+                    umma(d_tmem, ((uint64_t)hi128 << 32) | (a_lo + 2u * ks), ((uint64_t)hi128 << 32) | (b_lo + 2u * ks), idesc,
+                         (acc || ks > 0) ? 1u : 0u);
                 umma_commit<CG>(empty_bar0 + 8u * stage);
                 if (commit_afree) {
                   // input chunk x has now been read for the last time: the epilogue may overwrite it with output chunk x
@@ -731,11 +719,8 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tm_big, const __grid_constant_
 
   // teardown: everything issued has been consumed (the epilogue waited for the last commit)
   tc_fence_before();
-  if (CG == 2) cluster_sync_all(); else __syncthreads();
-  if (warp == TC_W_ALLOC) {
-    if (CG == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem_base), "r"(512) : "memory");
-    else asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" :: "r"(tmem_base), "r"(512) : "memory");
-  }
+  cluster_sync_all();
+  if (warp == TC_W_ALLOC) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" :: "r"(tmem_base), "r"(512) : "memory");
 }
 
 // ======================================================================================================
@@ -824,9 +809,6 @@ int tc_create(CfnHandle* h) {
   CFN_CHECK_ARG(h->slots.size() <= 60, "too many parameter tensors");
   TcPlan* p = new TcPlan();
   h->tc = p;
-  p->cg = 2;
-  if (const char* e = getenv("CFN_TC_CTA_GROUP")) p->cg = (atoi(e) == 1) ? 1 : 2;
-  const int CG = p->cg;
   p->stagger = 0;
   if (const char* e = getenv("CFN_TC_STAGGER")) p->stagger = atoi(e);
   p->prof_dev = nullptr;
@@ -838,9 +820,6 @@ int tc_create(CfnHandle* h) {
   int64_t stream_row = 0;
   int table_off = 0;
 
-  // CFN_TC_SPLIT_DRAIN=0 keeps the round-1 schedule (one accumulator commit per layer) for A/B timing
-  bool split_drain = true;
-  if (const char* e = getenv("CFN_TC_SPLIT_DRAIN")) split_drain = atoi(e) != 0;
   struct KCh { int src, kstart, ksteps, col0, cols_valid, with_bias; };
   // every kind 0/1 step multiplies the ones columns (62, 63) of the gamma(d) tile by the (hi, lo) split of its fp32
   // bias, so the epilogue is a pure convert-and-store; kind 2 steps add their (tiny) bias in the epilogue
@@ -873,7 +852,7 @@ int tc_create(CfnHandle* h) {
       if (kch[i].src == TC_SRC_GP && kch[i].with_bias != 2) dev.gd_step = dev.n_steps - 1;   // last reader of gamma(p)
     }
     st.split_commit = 0;
-    if (kind != 2 && st.n_parts == 2 && !st.order_rev && (st.n_part % 128) == 0 && st.n_part / 64 <= 4 && split_drain) {
+    if (kind != 2 && st.n_parts == 2 && !st.order_rev && (st.n_part % 128) == 0 && st.n_part / 64 <= 4) {
       st.split_commit = 1;
       for (int x = 0; x < st.n_part / 64; ++x) {
         int pos = 0;                                  // not read by this step: free right after the first K chunk
@@ -945,7 +924,6 @@ int tc_create(CfnHandle* h) {
   }
   // staging the last step's record rows needs 128 x (15F+1) floats in the upper half of the activation tile
   dev.stage_out = ((size_t)128 * (15 * F + 1) * sizeof(float) <= (size_t)(AC - AC / 2) * TC_CHUNK_BYTES) ? 1 : 0;
-  if (const char* e = getenv("CFN_TC_STAGE_OUT")) dev.stage_out = dev.stage_out && atoi(e) != 0;   // A/B timing
   p->stream_rows = stream_row;
   p->table_floats = table_off;
 
@@ -960,7 +938,6 @@ int tc_create(CfnHandle* h) {
   const size_t smem_max = (size_t)prop.sharedMemPerBlockOptin;
   int stages = (int)((smem_max - fixed) / p->stage_bytes);
   if (stages > TC_MAX_STAGES) stages = TC_MAX_STAGES;
-  if (const char* e = getenv("CFN_TC_STAGES")) { int v = atoi(e); if (v >= 2 && v < stages) stages = v; }   // experiments only
   if (stages < 2) return fail("not enough shared memory for two weight stages");
   p->stages = stages;
   p->smem_bytes = fixed + (size_t)stages * p->stage_bytes;
@@ -999,9 +976,7 @@ int tc_create(CfnHandle* h) {
   auto set_attr = [&](const void* fnp) {
     return cudaFuncSetAttribute(fnp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem_bytes) == cudaSuccess;
   };
-  bool ok = true;
-  if (CG == 1) ok = fp16 ? set_attr((const void*)mlp_tc_kernel<1, true>) : set_attr((const void*)mlp_tc_kernel<1, false>);
-  else ok = fp16 ? set_attr((const void*)mlp_tc_kernel<2, true>) : set_attr((const void*)mlp_tc_kernel<2, false>);
+  const bool ok = fp16 ? set_attr((const void*)mlp_tc_kernel<true>) : set_attr((const void*)mlp_tc_kernel<false>);
   if (!ok) return fail("cudaFuncSetAttribute(max dynamic shared memory)");
   return CFN_OK;
 }
@@ -1068,7 +1043,6 @@ int tc_debug_profile(CfnHandle* h, unsigned long long* out_host, int n) {
 int tc_network_fwd(CfnHandle* h, const float* rays, const float* z_vals, const float* pts, const float* viewdirs,
                    int64_t B, int N, float* flow_params, void*, size_t, cudaStream_t s) {
   TcPlan* p = h->tc;
-  const int CG = p->cg;
   TcArgs a;
   a.rays = rays; a.z_vals = z_vals; a.pts = pts; a.viewdirs = viewdirs;
   a.M = B * N; a.N = N; a.L_pos = h->cfg.L_pos; a.L_dir = h->cfg.L_dir;
@@ -1078,7 +1052,6 @@ int tc_network_fwd(CfnHandle* h, const float* rays, const float* z_vals, const f
   a.prof = p->prof_dev;
   a.stagger = p->stagger;
   int64_t units_grid = p->num_sms / CG;
-  if (const char* e = getenv("CFN_TC_MAX_SMS")) { int v = atoi(e); if (v >= CG && v / CG < units_grid) units_grid = v / CG; }   // experiments only
   if (units_grid > a.n_units) units_grid = a.n_units;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3((unsigned)(units_grid * CG));
@@ -1090,11 +1063,8 @@ int tc_network_fwd(CfnHandle* h, const float* rays, const float* z_vals, const f
   attr[0].val.clusterDim.x = CG; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
   const bool fp16 = h->cfg.precision == CFN_PREC_FP16;
-  cudaError_t e;
-  if (CG == 1) e = fp16 ? cudaLaunchKernelEx(&cfg, mlp_tc_kernel<1, true>, p->tm_big, p->tm_small, p->tm_bias, p->dev, a)
-                        : cudaLaunchKernelEx(&cfg, mlp_tc_kernel<1, false>, p->tm_big, p->tm_small, p->tm_bias, p->dev, a);
-  else e = fp16 ? cudaLaunchKernelEx(&cfg, mlp_tc_kernel<2, true>, p->tm_big, p->tm_small, p->tm_bias, p->dev, a)
-                : cudaLaunchKernelEx(&cfg, mlp_tc_kernel<2, false>, p->tm_big, p->tm_small, p->tm_bias, p->dev, a);
+  const cudaError_t e = fp16 ? cudaLaunchKernelEx(&cfg, mlp_tc_kernel<true>, p->tm_big, p->tm_small, p->tm_bias, p->dev, a)
+                             : cudaLaunchKernelEx(&cfg, mlp_tc_kernel<false>, p->tm_big, p->tm_small, p->tm_bias, p->dev, a);
   if (e != cudaSuccess) { set_error("mlp_tc_kernel launch failed: %s", cudaGetErrorString(e)); return CFN_ECUDA; }
   return CFN_OK;
 }

@@ -7,8 +7,6 @@ weights and scatters/gathers activations on every network call, run_nerf_uncerta
 """
 from __future__ import annotations
 
-import os
-
 import torch
 import torch.distributed as dist
 
@@ -119,7 +117,7 @@ class FusedTrainStep:
     def __init__(self, network_fn, lr: float = 5e-4, betas=(0.9, 0.999), eps: float = 1e-8, beta1: float = 0.01,
                  precision: str | None = None, N_samples: int = 128, white_bkgd: bool = False, lindisp: bool = False,
                  depth_lambda: float = 0.0, netchunk: int | None = None, lrate_decay: float = 0.0,
-                 use_graph: bool = False, deterministic: bool = False, overlap_allreduce: bool = False):
+                 use_graph: bool = False, deterministic: bool = False):
         from . import api
         from .engine import _unwrap, engine_for
         self.module = _unwrap(network_fn)
@@ -131,18 +129,6 @@ class FusedTrainStep:
         self.netchunk = api.DEFAULT_NETCHUNK if netchunk is None else int(netchunk)
         self.decay_steps = float(lrate_decay) * 1000.0            # args.lrate_decay is in thousands of steps (main:1074)
         self.use_graph = bool(use_graph)
-        # Opt-in for data-parallel runs: the backward is issued in two parts (cfn_network_bwd_part) and the gradients that
-        # are final after the first one (everything from pts_linears.<D/2> on: 60 % of the bucket) are all-reduced on a side
-        # stream while the lower trunk layers are still being differentiated; the rest follows on the main stream.
-        # OFF by default: measured on 2 B200s (NVLink) the single all-reduce of the 10 MB bucket costs ~40 us of a step
-        # and the second NCCL call + graph launch of the overlapped form cost more than they hide (512 rays / GPU:
-        # 1.628 -> 1.672 ms; 4096 rays / GPU: 9.98 -> 10.12 ms; profiles/r02_bench_2gpu_{nooverlap,overlap}.json).
-        self.split_layer = max(1, int(self.eng.cfg.D) // 2)
-        self.overlap_allreduce = bool(overlap_allreduce) and int(self.eng.cfg.D) >= 2
-        if os.environ.get("CFN_OVERLAP_ALLREDUCE") in ("0", "1"):      # A/B timing of the overlap
-            self.overlap_allreduce = os.environ["CFN_OVERLAP_ALLREDUCE"] == "1" and int(self.eng.cfg.D) >= 2
-        self.two_part_backward = False     # tests: issue the backward in its two parts even without a process group
-        self._side = None
         if deterministic:       # two-pass split-K weight gradients: bitwise identical steps for identical inputs
             self.eng.set_deterministic(True)
         ps = self.eng.params
@@ -164,7 +150,6 @@ class FusedTrainStep:
         import ctypes as C
         arr = lambda ts: (C.c_void_p * len(ts))(*[t.data_ptr() for t in ts])  # noqa: E731
         self._arrs = (arr(ps), arr(self.grads), arr(self._m), arr(self._v), (C.c_int64 * len(ps))(*[p.numel() for p in ps]))
-        self._split_off = sum(p.numel() for p in ps[:4 + 2 * self.split_layer])   # first float of pts_linears.<split>
         self.adam_state = torch.zeros(4, **f32)    # [step, lr, 1 - b1^t, sqrt(1 - b2^t)] — advanced on the device
         self.step_count = 0
         self._shapes = {}
@@ -199,18 +184,11 @@ class FusedTrainStep:
         return st
 
     # ---- the chain --------------------------------------------------------------------------------------------
-    def _forward_backward(self, st, part: int = 0):
-        """part 0: the whole chain; part 1: forward + backward down to the split layer; part 2: the rest of the backward."""
+    def _forward_backward(self, st):
         from ._lib import check
         from .engine import _ptr, _stream
         eng, N, K = self.eng, self.N, self.eng.K
         B, rays = st["B"], st["rays"]
-        if part == 2:
-            g_fp, ws, g_glob = st["_carry"]
-            eng.network_bwd(g_fp, B, N, ws, grads=self.grads, part=2, split_layer=self.split_layer)
-            check(eng.lib.cfn_globals_grad_f32(eng.h, _ptr(g_glob), g_glob.shape[0], float(self.beta1),
-                                               _ptr(self.flat_grad), _stream()), "cfn_globals_grad_f32")
-            return
         from . import api
         t_vals = api.reference_t_schedule(N, self.dev)
         z = eng.zvals(rays, t_vals, st["t_rand"], self.lindisp)
@@ -227,29 +205,12 @@ class FusedTrainStep:
                                               st["g_rgb"], st["g_depth"] if Bd else None, st["g_ld"],
                                               trans=out["trans"], eps_group_rays=st["group_rays"],
                                               seg_sums=out["seg_sums"])
-        st["out"] = out
-        if part == 1:
-            eng.network_bwd(g_fp, B, N, ws, grads=self.grads, part=1, split_layer=self.split_layer)
-            st["_carry"] = (g_fp, ws, g_glob)       # what part 2 continues from (static tensors under graph capture)
-            return
         eng.network_bwd(g_fp, B, N, ws, grads=self.grads)
         # parameters 0..3 (alpha_mean, alpha_std, rgb_mean, rgb_std) sit first in the flat gradient buffer
         check(eng.lib.cfn_globals_grad_f32(eng.h, _ptr(g_glob), g_glob.shape[0], float(self.beta1), _ptr(self.flat_grad),
                                            _stream()),
               "cfn_globals_grad_f32")
-
-    def _reduce_overlapped(self, run_part1, run_part2):
-        """part 1 -> [all-reduce of the finished bucket on the side stream || part 2] -> all-reduce of the rest."""
-        main = torch.cuda.current_stream(self.dev)
-        if self._side is None:
-            self._side = torch.cuda.Stream(self.dev)
-        run_part1()
-        self._side.wait_stream(main)
-        with torch.cuda.stream(self._side):
-            dist.all_reduce(self.flat_grad[self._split_off:], op=dist.ReduceOp.SUM)
-        run_part2()
-        dist.all_reduce(self.flat_grad[:self._split_off], op=dist.ReduceOp.SUM)
-        main.wait_stream(self._side)
+        st["out"] = out
 
     def _update(self, world: int):
         from ._lib import check
@@ -289,17 +250,10 @@ class FusedTrainStep:
             else:
                 st["eps_a"].copy_(_f32c(eps_alpha, dev).reshape(G, K))
                 st["eps_c"].copy_(_f32c(eps_rgb, dev).reshape(G, K, 3))
-            overlap = w > 1 and self.overlap_allreduce and self.flat_grad.is_cuda
             if not self.use_graph:
-                if overlap:
-                    self._reduce_overlapped(lambda: self._forward_backward(st, 1), lambda: self._forward_backward(st, 2))
-                elif self.two_part_backward:
-                    self._forward_backward(st, 1)
-                    self._forward_backward(st, 2)
-                else:
-                    self._forward_backward(st)
-                    if w > 1:
-                        dist.all_reduce(self.flat_grad, op=dist.ReduceOp.SUM)
+                self._forward_backward(st)
+                if w > 1:
+                    dist.all_reduce(self.flat_grad, op=dist.ReduceOp.SUM)
                 self._update(w)
             elif st["graph_a"] is None:
                 # first step of this shape: run it eagerly (warm-up: function attributes, allocator), then capture the same
@@ -313,16 +267,8 @@ class FusedTrainStep:
                 ga, gb = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
                 state_backup = [t.clone() for t in (self.flat_param, self.flat_grad, self.exp_avg, self.exp_avg_sq,
                                                     self.adam_state)]
-                if overlap:
-                    ga2 = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(ga):
-                        self._forward_backward(st, 1)
-                    with torch.cuda.graph(ga2, pool=ga.pool()):
-                        self._forward_backward(st, 2)
-                    st["graph_a2"] = ga2
-                else:
-                    with torch.cuda.graph(ga):
-                        self._forward_backward(st)
+                with torch.cuda.graph(ga):
+                    self._forward_backward(st)
                 with torch.cuda.graph(gb, pool=ga.pool()):
                     self._update(w)
                 for t, bck in zip((self.flat_param, self.flat_grad, self.exp_avg, self.exp_avg_sq, self.adam_state),
@@ -333,12 +279,9 @@ class FusedTrainStep:
             else:
                 if "out_captured" in st:
                     st["out"] = st.pop("out_captured")      # static tensors the replayed graph writes
-                if st.get("graph_a2") is not None:
-                    self._reduce_overlapped(st["graph_a"].replay, st["graph_a2"].replay)
-                else:
-                    st["graph_a"].replay()
-                    if w > 1:
-                        dist.all_reduce(self.flat_grad, op=dist.ReduceOp.SUM)
+                st["graph_a"].replay()
+                if w > 1:
+                    dist.all_reduce(self.flat_grad, op=dist.ReduceOp.SUM)
                 st["graph_b"].replay()
             self.step_count += 1
             bump_weights_epoch()                          # other engines of this module re-pack on their next use ...

@@ -180,21 +180,15 @@ class Engine:
               "cfn_flow_composite_bwd_dev")
         return g_fp, g_glob
 
-    def network_bwd(self, g_flow_params, B: int, N: int, ws, grads=None, part: int = 0, split_layer: int = 0):
+    def network_bwd(self, g_flow_params, B: int, N: int, ws, grads=None):
         """-> list of gradient tensors in parameter order (entries 0..3 are None: globals come from the flow stage).
-        `grads`: optional preallocated fp32 tensors to write into (entries 0..3 ignored).
-        `part` 1 / 2: the two halves of cfn_network_bwd_part (part 1 ends with the weight gradient of trunk layer
-        `split_layer`; every gradient from `pts_linears.<split_layer>` on is final after it)."""
+        `grads`: optional preallocated fp32 tensors to write into (entries 0..3 ignored)."""
         if grads is None:
             grads = [None] * 4 + [torch.empty_like(p, dtype=torch.float32, memory_format=torch.contiguous_format)
                                   for p in self.params[4:]]
         arr = (C.c_void_p * len(grads))(*[(g.data_ptr() if (g is not None and i >= 4) else 0) for i, g in enumerate(grads)])
-        if part == 0:
-            check(self.lib.cfn_network_bwd(self.h, _ptr(g_flow_params), B, N, _ptr(ws), ws.numel(), arr, len(grads),
-                                           _stream()), "cfn_network_bwd")
-        else:
-            check(self.lib.cfn_network_bwd_part(self.h, _ptr(g_flow_params), B, N, _ptr(ws), ws.numel(), arr, len(grads),
-                                                int(part), int(split_layer), _stream()), "cfn_network_bwd_part")
+        check(self.lib.cfn_network_bwd(self.h, _ptr(g_flow_params), B, N, _ptr(ws), ws.numel(), arr, len(grads),
+                                       _stream()), "cfn_network_bwd")
         return grads
 
 

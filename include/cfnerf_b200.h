@@ -123,15 +123,6 @@ int cfn_network_fwd(CfnHandle* h, const float* rays, const float* z_vals, const 
 int cfn_network_bwd(CfnHandle* h, const float* g_flow_params, int64_t B, int N, void* workspace,
                     size_t workspace_bytes, float* const* grads, int n_params, void* stream);
 
-/* The same backward in two calls, for data-parallel training (loss.backward() + the gradient all-reduce of a DDP-style
- * trainer around main:1065-1067): part 1 runs from the flow records down to and including the weight gradient of trunk
- * layer split_layer (1 .. netdepth-1) — after it grads[i] is final for every parameter from pts_linears.<split_layer> on
- * (in cfn_param_name order), so the caller can start all-reducing that bucket on another stream; part 2 (same arguments)
- * finishes the trunk below it.  part 1 followed by part 2 writes exactly what cfn_network_bwd writes. */
-int cfn_network_bwd_part(CfnHandle* h, const float* g_flow_params, int64_t B, int N, void* workspace,
-                         size_t workspace_bytes, float* const* grads, int n_params, int part, int split_layer,
-                         void* stream);
-
 /* ---- A6-A8 (+A11 partials): K-sample flows + alpha compositing --------------------------------- */
 /* eps_alpha (G,K), eps_rgb (G,K,3): base latent draws (models.py:198-206 / 233-251).  eps_group_rays = 0: G = 1, one
  * set shared by all rays (test mode; a training call of at most netchunk points).  eps_group_rays = R > 0: ray b uses

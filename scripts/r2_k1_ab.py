@@ -1,5 +1,4 @@
-"""K1 A/B timing on one GPU: 8 chunks of 32768 rays x 128 samples through Engine.network (CUDA events), fp16 and bf16.
-Env toggles are read at handle creation (CFN_TC_SPLIT_DRAIN=0 restores the round-1 schedule)."""
+"""K1 A/B timing on one GPU: 8 chunks of 32768 rays x 128 samples through Engine.network (CUDA events), fp16 and bf16."""
 import json
 import os
 import sys
@@ -38,4 +37,4 @@ for prec in ("fp16", "bf16"):
     # correctness against the fp32 check mode on a slice
     ref = cf.engine_for(net, dev, "fp32").network(256, N, rays=rays[:256], z_vals=z[:256])
     res[prec]["max_err_vs_fp32"] = float((fp[:256 * N] - ref).abs().max())
-print(json.dumps({"lib": os.environ.get("CFN_AB_LIB", "tree"), "split_drain": os.environ.get("CFN_TC_SPLIT_DRAIN", "1"), **res}))
+print(json.dumps({"lib": os.environ.get("CFN_AB_LIB", "tree"), **res}))

@@ -550,33 +550,6 @@ def test_global_batch_gradient_equals_mean_of_shard_gradients(cf, dev, precision
     assert abs(float(lf["loss"]) - sum(losses) / shards) <= 1e-4 * max(1.0, abs(float(lf["loss"])))
 
 
-@pytest.mark.parametrize("precision", ["fp32", "bf16"])
-def test_two_part_backward_equals_the_whole_backward(cf, dev, precision):
-    """cfn_network_bwd_part (part 1 down to the weight gradient of trunk layer D/2, part 2 the rest) is what lets the
-    data-parallel trainer all-reduce the finished half of its gradient bucket under the rest of the backward: the two
-    calls must write exactly what cfn_network_bwd writes (deterministic mode: bit for bit)."""
-    from cfnerf_b200 import dist as D
-    cfg = O.CfnConfig()
-    p = O.make_params(cfg, 5, "lively")
-    sa, sr = O.make_latents(cfg, 5)
-    B = 96
-    rays = O.synthetic_rays(B, 3).to(dev)
-    g = torch.Generator().manual_seed(11)
-    target = torch.rand(B, 3, generator=g).to(dev)
-    t_rand = torch.rand(B, 128, generator=g).to(dev)
-    ea, er = torch.randn(cfg.K, 1, generator=g).to(dev), torch.randn(cfg.K, 3, generator=g).to(dev)
-    grads = []
-    for two in (False, True):
-        net = make_net(cf, cfg, p, sa, sr, dev)
-        tr = D.FusedTrainStep(net, lr=0.0, precision=precision, deterministic=True)
-        tr.two_part_backward = two
-        tr.step(rays, target, t_rand=t_rand, eps_alpha=ea, eps_rgb=er)
-        grads.append(tr.flat_grad.clone())
-        assert 0 < tr._split_off < tr.flat_grad.numel()
-    assert float(grads[0].abs().max()) > 0
-    assert torch.equal(grads[0], grads[1])
-
-
 @pytest.mark.parametrize("precision,K", [("fp32", 32), ("bf16", 32), ("fp32", 40)])
 def test_small_batch_training_forward_equals_the_one_warp_per_ray_kernel(cf, dev, precision, K):
     """Batches of at most 1536 rays take the four-warps-per-ray training forward (each warp walks a quarter of the samples
