@@ -34,14 +34,11 @@ SYMBOLS = {
     "cfn_flow_composite_fwd": (_i32, [_vp, _f32p, _f32p, _f32p, _i32, _f32p, _f32p, _i64, _i64, _i32, _i32, _f32p, _f32p,
                                       _f32p, _f32p, _f32p, _f32p, _f32p, _f32p, _f32p, _i32, _vp]),
     "cfn_flow_composite_bwd": (_i32, [_vp, _f32p, _f32p, _f32p, _i32, _f32p, _f32p, _i64, _i64, _i32, _i32, _f32p, _f32p,
-                                      C.c_float, C.c_float, _f32p, _i32, _f32p, _i32, _f32p, _f32p, _vp]),
-    "cfn_flow_composite_bwd_dev": (_i32, [_vp, _f32p, _f32p, _f32p, _i32, _f32p, _f32p, _i64, _i64, _i32, _i32, _f32p,
-                                          _f32p, _f32p, _f32p, _i32, _f32p, _i32, _f32p, _f32p, _vp]),
+                                      _f32p, _f32p, _f32p, _i32, _f32p, _f32p, _vp]),
     "cfn_raw2outputs_f32": (_i32, [_f32p, _f32p, _f32p, _i32, _i32, _f32p, _f32p, _f32p, _f32p, _i64, _i32, _i32, _vp]),
     "cfn_sample_pdf_f32": (_i32, [_f32p, _f32p, _f32p, _f32p, _vp, _i64, _i32, _i32, _vp]),
     "cfn_merge_sorted_f32": (_i32, [_f32p, _f32p, _f32p, _i64, _i32, _i32, _vp]),
     "cfn_mean_over_k_f32": (_i32, [_f32p, _f32p, _i64, _i32, _vp]),
-    "cfn_kde_nll_f32": (_i32, [_f32p, _f32p, _i64, _i32, C.c_float, _f32p, _f32p, _vp]),
     "cfn_trainer_loss_f32": (_i32, [_f32p, _f32p, _f32p, _f32p, _i64, _i64, _i32, C.c_float, C.c_float, _f32p, _f32p, _f32p,
                                     _vp]),
     "cfn_adam_step_f32": (_i32, [_i32, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_i64),

@@ -190,6 +190,28 @@ def latent_groups(B: int, N: int, netchunk: int):
     return 0, 1
 
 
+def _latent_draws(module, K: int, device, train: bool, G: int, eps_alpha, eps_rgb, batch: str):
+    """The base latent draws of a batch that makes G network calls -> (eps_a, eps_c): (K), (K,3) when G = 1, else
+    (G,K), (G,K,3).  Without eps_alpha: in train mode one fresh (alpha, rgb) pair per network call, drawn in the
+    reference's order (models.py:234, 246); in test mode the constructor-time draws.  The caller's eps_alpha / eps_rgb
+    may be (K,1) / (K,3) (one call) or (G,K,1) / (G,K,3) (one pair per call).  `batch` describes the batch in errors."""
+    if eps_alpha is None:
+        if train:
+            pairs = [(torch.empty([K, 1], device=device).normal_(),                            # models.py:234
+                      torch.empty([K, 3], device=device).normal_()) for _ in range(G)]        # models.py:246
+            eps_alpha, eps_rgb = torch.stack([a for a, _ in pairs], 0), torch.stack([c for _, c in pairs], 0)
+        else:
+            eps_alpha, eps_rgb = test_latents(module, device)
+    if eps_rgb.dim() == 3:      # (G,K,3): the caller fixed the draws of every network call
+        if eps_rgb.shape[0] != G:
+            raise ValueError(f"{eps_rgb.shape[0]} latent draws given but the batch makes {G} network calls ({batch})")
+        eps_a, eps_c = _f32c(eps_alpha.reshape(G, -1), device), _f32c(eps_rgb, device)
+        return (eps_a[0].contiguous(), eps_c[0].contiguous()) if G == 1 else (eps_a, eps_c)
+    if G > 1:
+        raise ValueError(f"the batch makes {G} network calls: pass eps_alpha (G,K,1) and eps_rgb (G,K,3)")
+    return _f32c(eps_alpha.reshape(-1), device), _f32c(eps_rgb.reshape(-1, 3), device)
+
+
 def _entropy_base_terms(module, eps_a, eps_c):
     """base log-densities of models.py:268/283 (no 2*pi term), written like the reference so autograd gives the same
     gradient for the global std parameters.  eps_a (K) / eps_c (K,3) -> two scalars; with a leading group axis
@@ -251,20 +273,8 @@ def run_network(inputs, viewdirs, fn, is_val, is_test, embed_fn=None, embeddirs_
     train = not is_test
     # train mode: one latent draw per batchify call of `netchunk` points (main:47-64, models.py:233-251)
     group_rays, G = latent_groups(B, N, int(netchunk)) if train else (0, 1)
-    if eps_alpha is None:
-        if train:
-            pairs = [(torch.empty([eng.K, 1], device=dev).normal_(),                          # models.py:234
-                      torch.empty([eng.K, 3], device=dev).normal_()) for _ in range(G)]      # models.py:246
-            eps_alpha = torch.stack([a for a, _ in pairs], 0) if G > 1 else pairs[0][0]
-            eps_rgb = torch.stack([c for _, c in pairs], 0) if G > 1 else pairs[0][1]
-        else:
-            eps_alpha, eps_rgb = test_latents(module, dev)
-    if G > 1:
-        if eps_rgb.dim() != 3 or eps_rgb.shape[0] != G:
-            raise ValueError(f"the batch makes {G} network calls: pass eps_alpha (G,K,1) and eps_rgb (G,K,3)")
-        eps_a, eps_c = _f32c(eps_alpha.reshape(G, -1), dev), _f32c(eps_rgb, dev)
-    else:
-        eps_a, eps_c = _f32c(eps_alpha.reshape(-1), dev), _f32c(eps_rgb.reshape(-1, 3), dev)
+    eps_a, eps_c = _latent_draws(module, eng.K, dev, train, G, eps_alpha, eps_rgb,
+                                 f"{B} rays x {N} samples, netchunk {netchunk}")
     with torch.cuda.device(dev), torch.no_grad():
         fp = eng.network(B, N, pts=pts, viewdirs=vd)
         # raw comes out of the flow stage; compositing outputs are discarded here (z/dirs are dummies)
@@ -334,25 +344,8 @@ def render_rays(ray_batch, network_fn, network_query_fn=None, N_samples=128, is_
         group_rays, G = (0, 1)
         if is_train and not hier:
             group_rays, G = latent_groups(B, N_samples, DEFAULT_NETCHUNK if netchunk is None else int(netchunk))
-        if eps_alpha is None:
-            if is_train:
-                pairs = [(torch.empty([eng.K, 1], device=dev).normal_(),                      # models.py:234
-                          torch.empty([eng.K, 3], device=dev).normal_()) for _ in range(G)]  # models.py:246
-                eps_alpha = torch.stack([a for a, _ in pairs], 0) if G > 1 else pairs[0][0]
-                eps_rgb = torch.stack([c for _, c in pairs], 0) if G > 1 else pairs[0][1]
-            else:
-                eps_alpha, eps_rgb = test_latents(module, dev)
-        if eps_rgb.dim() == 3:      # (G,K,3): the caller fixed the draws of every network call
-            if eps_rgb.shape[0] != G and not (G == 1 and eps_rgb.shape[0] == 1):
-                raise ValueError(f"{eps_rgb.shape[0]} latent draws given but the batch makes {G} network calls "
-                                 f"({B} rays x {N_samples} samples, netchunk {netchunk or DEFAULT_NETCHUNK})")
-            eps_a, eps_c = _f32c(eps_alpha.reshape(eps_rgb.shape[0], -1), dev), _f32c(eps_rgb, dev)
-            if G == 1:
-                eps_a, eps_c = eps_a[0].contiguous(), eps_c[0].contiguous()
-        else:
-            if G > 1:
-                raise ValueError(f"the batch makes {G} network calls: pass eps_alpha (G,K,1) and eps_rgb (G,K,3)")
-            eps_a, eps_c = _f32c(eps_alpha.reshape(-1), dev), _f32c(eps_rgb, dev)
+        eps_a, eps_c = _latent_draws(module, eng.K, dev, is_train, G, eps_alpha, eps_rgb,
+                                     f"{B} rays x {N_samples} samples, netchunk {netchunk or DEFAULT_NETCHUNK}")
         if is_train and raw_noise_std > 0.:
             # the reference draws noise here and never adds it (main:432-442); same count keeps the RNG stream aligned
             torch.randn(B, N_samples, eng.K, device=dev)
@@ -503,41 +496,16 @@ def install(ref_module, precision: str | None = None, train_precision: str | Non
 # ------------------------------------------------------------------------------------------------------
 # A11: the caller's K-reduction and KDE-NLL loss (main:1027-1050), kept in torch for round 1 (SURVEY F1)
 # ------------------------------------------------------------------------------------------------------
-class _KdeNllFn(torch.autograd.Function):
-    """cfn_kde_nll_f32: loss_nll and mse in one kernel, the gradient seed w.r.t. rgb_map computed in the same pass."""
-
-    @staticmethod
-    def forward(ctx, rgb_map, target):
-        lib = _lib.load()
-        dev = rgb_map.device
-        x, t = _f32c(rgb_map.detach(), dev), _f32c(target, dev)
-        B, _, K = x.shape
-        partial = torch.empty(B, 2, dtype=torch.float32, device=dev)
-        g = torch.empty_like(x)
-        with torch.cuda.device(dev):
-            check(lib.cfn_kde_nll_f32(_ptr(x), _ptr(t), B, K, 1.0 / (3.0 * B), _ptr(partial), _ptr(g), _stream()),
-                  "cfn_kde_nll_f32")
-        ctx.save_for_backward(g)
-        tot = partial.sum(0) / (3.0 * B)
-        nll, mse = tot[0].clone(), tot[1].clone()
-        ctx.mark_non_differentiable(mse)        # the mark applies to the very tensor object that is returned
-        return nll, mse
-
-    @staticmethod
-    def backward(ctx, g_nll, g_mse):
-        (g,) = ctx.saved_tensors
-        return g * g_nll, None
-
-
 class _TrainerLossFn(torch.autograd.Function):
     """cfn_trainer_loss_f32: KDE-NLL + mse over the colour rays and the depth squared error over the depth rays in one
-    kernel, both gradient seeds computed in the same pass."""
+    kernel, both gradient seeds computed in the same pass.  depth_map may be None when there are no depth rays."""
 
     @staticmethod
     def forward(ctx, rgb_map, depth_map, target, target_depth):
         lib = _lib.load()
         dev = rgb_map.device
-        x, d, t = _f32c(rgb_map.detach(), dev), _f32c(depth_map.detach(), dev), _f32c(target, dev)
+        x, t = _f32c(rgb_map.detach(), dev), _f32c(target, dev)
+        d = _f32c(depth_map.detach(), dev) if depth_map is not None else None
         B, _, K = x.shape
         B_rgb = t.shape[0]
         B_depth = B - B_rgb
@@ -545,7 +513,7 @@ class _TrainerLossFn(torch.autograd.Function):
         if B_depth and td.shape[0] != B_depth:
             raise ValueError(f"{B} rays rendered, {B_rgb} colour targets, {td.shape[0]} depth targets")
         partial = torch.empty(B, 3, dtype=torch.float32, device=dev)
-        g_rgb, g_depth = torch.empty_like(x), torch.empty_like(d)
+        g_rgb, g_depth = torch.empty_like(x), (torch.empty_like(d) if d is not None else None)
         with torch.cuda.device(dev):
             check(lib.cfn_trainer_loss_f32(_ptr(x), _ptr(d), _ptr(t), _ptr(td), B_rgb, B_depth, K, 1.0 / (3.0 * B_rgb),
                                            (1.0 / B_depth) if B_depth else 0.0, _ptr(partial), _ptr(g_rgb), _ptr(g_depth),
@@ -560,7 +528,7 @@ class _TrainerLossFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_nll, g_mse, g_dl):
         g_rgb, g_depth = ctx.saved_tensors
-        return g_rgb * g_nll, g_depth * g_dl, None, None
+        return g_rgb * g_nll, (g_depth * g_dl if g_depth is not None else None), None, None
 
 
 def trainer_loss(out, target_s, K, beta1=0.01, target_depth=None, depth_lambda=0.0):
@@ -585,12 +553,12 @@ def trainer_loss(out, target_s, K, beta1=0.01, target_depth=None, depth_lambda=0
 
 
 def kde_nll_loss(rgb_map, target, loss_entropy, K, beta1=0.01, fused=None):
-    """main:1027-1050.  On CUDA tensors the K-reduction, the KDE-NLL and its gradient run in one kernel (F1); the
-    torch expression below is the CPU form used by the host-side tests."""
+    """main:1027-1050.  On CUDA tensors the K-reduction, the KDE-NLL and its gradient run in one kernel (F1, the
+    trainer loss kernel without depth rays); the torch expression below is the CPU form used by the host-side tests."""
     if fused is None:
         fused = rgb_map.is_cuda
     if fused:
-        nll, mse = _KdeNllFn.apply(rgb_map, target)
+        nll, mse, _ = _TrainerLossFn.apply(rgb_map, None, target, None)
         psnr = -10. * torch.log(mse) / math.log(10.)
         loss = nll + beta1 * loss_entropy.mean() if beta1 else nll
         return {"loss": loss, "loss_nll": nll, "mse": mse, "psnr": psnr}

@@ -17,7 +17,7 @@ void set_error(const char* fmt, ...) {
 using namespace cfn;
 
 extern "C" const char* cfn_last_error(void) { return g_err; }
-extern "C" int cfn_version(void) { return 101; }
+extern "C" int cfn_version(void) { return 102; }
 
 static void add_slot(CfnHandle* h, const std::string& name, int rows, int cols) {
   ParamSlot s;
@@ -320,14 +320,14 @@ extern "C" int cfn_flow_composite_fwd(CfnHandle* h, const float* flow_params, co
                                    weights, logdet_sums, kstats, trans, seg_sums, n_segments, (cudaStream_t)stream);
 }
 
-static int flow_composite_bwd_impl(CfnHandle* h, const float* flow_params, const float* z_vals, const float* rays_d,
-                                  int rays_d_stride, const float* eps_alpha, const float* eps_rgb, int64_t eps_group_rays,
-                                  int64_t B, int N, int white_bkgd, const float* g_rgb_map, const float* g_depth_map,
-                                  float g_logdet_alpha, float g_logdet_rgb, const float* g_logdet_dev, float* trans,
-                                  int trans_valid, const float* seg_sums, int n_segments, float* g_flow_params,
-                                  float* g_globals_partial, void* stream) {
-  CFN_CHECK_ARG(h && flow_params && z_vals && rays_d && eps_alpha && eps_rgb && g_rgb_map && g_flow_params &&
-                    g_globals_partial && trans,
+extern "C" int cfn_flow_composite_bwd(CfnHandle* h, const float* flow_params, const float* z_vals,
+                                      const float* rays_d, int rays_d_stride, const float* eps_alpha,
+                                      const float* eps_rgb, int64_t eps_group_rays, int64_t B, int N, int white_bkgd,
+                                      const float* g_rgb_map, const float* g_depth_map, const float* g_logdet,
+                                      const float* trans, const float* seg_sums, int n_segments, float* g_flow_params,
+                                      float* g_globals_partial, void* stream) {
+  CFN_CHECK_ARG(h && flow_params && z_vals && rays_d && eps_alpha && eps_rgb && g_rgb_map && g_logdet && trans &&
+                    g_flow_params && g_globals_partial,
                 "cfn_flow_composite_bwd: null argument");
   CFN_CHECK_ARG(eps_group_rays >= 0, "cfn_flow_composite_bwd: negative eps_group_rays");
   if (!h->packed) {
@@ -336,31 +336,8 @@ static int flow_composite_bwd_impl(CfnHandle* h, const float* flow_params, const
   }
   return launch_flow_composite_bwd(h->cfg.precision != CFN_PREC_FP32 ? 1 : 0, h->cfg.F, h->cfg.K, h->globals, flow_params,
                                    z_vals, rays_d, rays_d_stride, eps_alpha, eps_rgb, eps_group_rays, B, N, white_bkgd,
-                                   g_rgb_map, g_depth_map, g_logdet_alpha, g_logdet_rgb, g_logdet_dev, trans, trans_valid,
-                                   seg_sums, n_segments, g_flow_params, g_globals_partial, (cudaStream_t)stream);
-}
-
-extern "C" int cfn_flow_composite_bwd(CfnHandle* h, const float* flow_params, const float* z_vals,
-                                      const float* rays_d, int rays_d_stride, const float* eps_alpha,
-                                      const float* eps_rgb, int64_t eps_group_rays, int64_t B, int N, int white_bkgd,
-                                      const float* g_rgb_map, const float* g_depth_map, float g_logdet_alpha,
-                                      float g_logdet_rgb, float* trans, int trans_valid, const float* seg_sums,
-                                      int n_segments, float* g_flow_params, float* g_globals_partial, void* stream) {
-  return flow_composite_bwd_impl(h, flow_params, z_vals, rays_d, rays_d_stride, eps_alpha, eps_rgb, eps_group_rays, B, N,
-                                 white_bkgd, g_rgb_map, g_depth_map, g_logdet_alpha, g_logdet_rgb, nullptr, trans,
-                                 trans_valid, seg_sums, n_segments, g_flow_params, g_globals_partial, stream);
-}
-
-extern "C" int cfn_flow_composite_bwd_dev(CfnHandle* h, const float* flow_params, const float* z_vals,
-                                          const float* rays_d, int rays_d_stride, const float* eps_alpha,
-                                          const float* eps_rgb, int64_t eps_group_rays, int64_t B, int N, int white_bkgd,
-                                          const float* g_rgb_map, const float* g_depth_map, const float* g_logdet_dev,
-                                          float* trans, int trans_valid, const float* seg_sums, int n_segments,
-                                          float* g_flow_params, float* g_globals_partial, void* stream) {
-  CFN_CHECK_ARG(g_logdet_dev != nullptr, "cfn_flow_composite_bwd_dev: g_logdet_dev is null");
-  return flow_composite_bwd_impl(h, flow_params, z_vals, rays_d, rays_d_stride, eps_alpha, eps_rgb, eps_group_rays, B, N,
-                                 white_bkgd, g_rgb_map, g_depth_map, 0.f, 0.f, g_logdet_dev, trans, trans_valid, seg_sums,
-                                 n_segments, g_flow_params, g_globals_partial, stream);
+                                   g_rgb_map, g_depth_map, g_logdet, trans, seg_sums, n_segments, g_flow_params,
+                                   g_globals_partial, (cudaStream_t)stream);
 }
 
 extern "C" int cfn_raw2outputs_f32(const float* raw, const float* z_vals, const float* rays_d, int rays_d_stride,
@@ -432,19 +409,13 @@ extern "C" int cfn_gemm_bf16(const void* A, int64_t a_rs, int64_t a_cs, const vo
   return launch_tgemm(g, 0, (cudaStream_t)stream);
 }
 
-extern "C" int cfn_kde_nll_f32(const float* rgb_map, const float* target, int64_t B, int K, float grad_scale, float* partial,
-                               float* g_rgb_map, void* stream) {
-  CFN_CHECK_ARG(B >= 0 && (B == 0 || (rgb_map && target && partial)), "cfn_kde_nll_f32: null argument");
-  return launch_kde_nll(rgb_map, target, B, K, grad_scale, partial, g_rgb_map, (cudaStream_t)stream);
-}
-
 extern "C" int cfn_trainer_loss_f32(const float* rgb_map, const float* depth_map, const float* target_rgb,
                                     const float* target_depth, int64_t B_rgb, int64_t B_depth, int K, float nll_scale,
                                     float depth_scale, float* partial, float* g_rgb_map, float* g_depth_map, void* stream) {
   CFN_CHECK_ARG(B_rgb >= 0 && B_depth >= 0, "cfn_trainer_loss_f32: negative batch");
-  CFN_CHECK_ARG(B_rgb + B_depth == 0 || (rgb_map && depth_map && partial), "cfn_trainer_loss_f32: null argument");
+  CFN_CHECK_ARG(B_rgb + B_depth == 0 || (rgb_map && partial), "cfn_trainer_loss_f32: null argument");
   CFN_CHECK_ARG(B_rgb == 0 || target_rgb, "cfn_trainer_loss_f32: target_rgb is null");
-  CFN_CHECK_ARG(B_depth == 0 || target_depth, "cfn_trainer_loss_f32: target_depth is null");
+  CFN_CHECK_ARG(B_depth == 0 || (depth_map && target_depth), "cfn_trainer_loss_f32: depth_map / target_depth is null");
   return launch_trainer_loss(rgb_map, depth_map, target_rgb, target_depth, B_rgb, B_depth, K, nll_scale, depth_scale, partial,
                              g_rgb_map, g_depth_map, (cudaStream_t)stream);
 }
@@ -480,25 +451,7 @@ extern "C" int cfn_globals_grad_f32(const CfnHandle* h, const float* g_globals_p
 extern "C" int cfn_set_deterministic(CfnHandle* h, int on) {
   CFN_CHECK_ARG(h != nullptr, "cfn_set_deterministic: null handle");
   if (on && !h->det_scratch) {
-    // the largest (splits x (out x in + out)) over every weight gradient the backward chain issues; the split count is
-    // bounded by one K slice per CTA (tensor-core engine) or 8 per SM (CUDA-core engine), whichever engine runs
-    int64_t need = 0;
-    auto account = [&](int64_t out_f, int64_t in_f) {
-      const int cg = out_f <= 128 ? 1 : 2;
-      const int64_t bn = in_f >= 256 ? 256 : ((in_f + 15) / 16) * 16;
-      const int64_t tiles_tc = ((out_f + 128 * cg - 1) / (128 * cg)) * ((in_f + bn - 1) / bn);
-      const int64_t tiles_cc = ((out_f + 127) / 128) * ((in_f + 127) / 128);
-      int64_t split = (148 / cg) / tiles_tc;
-      const int64_t split_cc = (148 * 8 + tiles_cc - 1) / tiles_cc;
-      if (split_cc > split) split = split_cc;
-      if (split < 2) split = 2;
-      const int64_t n = split * (out_f * in_f + out_f);
-      if (n > need) need = n;
-    };
-    for (size_t i = 0; i < h->slots.size(); ++i)
-      if (h->wv[i].ld) account(h->slots[i].rows, h->wv[i].ld);
-    account(3 * h->cfg.F, (h->cfg.h_alpha + 7) & ~7);
-    account(15 * h->cfg.F, (h->cfg.h_rgb + 7) & ~7);
+    const int64_t need = chain_det_scratch_floats(h);
     CFN_CUDA(cudaMalloc(&h->det_scratch, (size_t)need * sizeof(float)));
     h->det_floats = need;
   }

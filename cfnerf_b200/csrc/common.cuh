@@ -93,8 +93,6 @@ int launch_raw2outputs(const float* raw, const float* z_vals, const float* rays_
 int launch_sample_pdf(const float* bins, const float* weights, const float* u, float* samples, int32_t* below,
                       int64_t B, int M, int Nf, cudaStream_t s);
 int launch_merge_sorted(const float* a, const float* b, float* out, int64_t B, int Na, int Nb, cudaStream_t s);
-int launch_kde_nll(const float* rgb_map, const float* target, int64_t B, int K, float grad_scale, float* partial, float* g,
-                   cudaStream_t s);
 int launch_trainer_loss(const float* rgb_map, const float* depth_map, const float* target_rgb, const float* target_depth,
                         int64_t B_rgb, int64_t B_depth, int K, float nll_scale, float depth_scale, float* partial, float* g_rgb,
                         float* g_depth, cudaStream_t s);
@@ -115,9 +113,8 @@ int launch_flow_composite_fwd(int fast_math, int F, int K, const float* globals,
 int launch_flow_composite_bwd(int fast_math, int F, int K, const float* globals, const float* flow_params, const float* z_vals,
                               const float* rays_d, int rays_d_stride, const float* eps_alpha, const float* eps_rgb,
                               int64_t eps_group_rays, int64_t B, int N, int white_bkgd, const float* g_rgb_map,
-                              const float* g_depth_map, float g_ld_alpha, float g_ld_rgb, const float* g_ld_dev,
-                              float* trans, int trans_valid, const float* seg_sums, int n_seg, float* g_flow_params,
-                              float* g_globals, cudaStream_t s);
+                              const float* g_depth_map, const float* g_ld, const float* trans, const float* seg_sums,
+                              int n_seg, float* g_flow_params, float* g_globals, cudaStream_t s);
 
 // C[m,n] = epi( sum_k A(m,k) * B(k,n) + bias[n] ) with arbitrary element strides (fp32 CUDA-core GEMM).
 enum Epilogue { EPI_NONE = 0, EPI_RELU = 1, EPI_TANH_MASK = 2, EPI_RELU_MASK_MUL = 3 };

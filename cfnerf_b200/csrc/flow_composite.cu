@@ -502,8 +502,7 @@ int launch_flow_composite_fwd(int fast_math, int F, int K, const float* globals,
 // =====================================================================================================
 // Backward (K4).  One warp per ray, lane = latent sample k, ONE pass back to front:
 //   * the transmittance T_n in front of every sample comes from HBM (B,N,K): the training forward writes it for free
-//     (K2 `trans` output), or `trans_prepass_kernel` (alpha stack only) fills it when the caller has none.  Keeping it in
-//     shared memory (round 1: N x 32 floats per warp) capped the kernel at 8 warps per SM, and at ~1200 dependent
+//     (K2 `trans` output).  Keeping it in shared memory (round 1: N x 32 floats per warp) capped the kernel at 8 warps per SM, and at ~1200 dependent
 //     instructions per point the kernel is latency bound: occupancy is what it needs;
 //   * per point both stacks are recomputed with their intermediates in registers, the compositing adjoint carries the
 //     suffix sum S (Appendix A.2), the flow adjoints run step by step in reverse (Appendix A.1);
@@ -517,42 +516,6 @@ int launch_flow_composite_fwd(int fast_math, int F, int K, const float* globals,
 // =====================================================================================================
 constexpr int kBwdPB = 4;     // points per staged block
 constexpr int kBwdGLD = 36;   // row stride of the reduction scratch: 32 lanes + 4 (rows stay 16-byte aligned, no conflicts)
-
-template <int FT, bool FAST>
-__global__ void __launch_bounds__(256)
-trans_prepass_kernel(int K, const float* __restrict__ globals, const float* __restrict__ flow_params,
-                     const float* __restrict__ z_vals, const float* __restrict__ rays_d, int rays_d_stride,
-                     const float* __restrict__ eps_alpha, int64_t eps_group_rays, int64_t B, int N,
-                     float* __restrict__ trans) {
-  constexpr int F = FT, PP = 18 * FT;
-  const int lane = threadIdx.x & 31;
-  const int64_t b = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  if (b >= B) return;
-  const int64_t egrp = eps_group_rays > 0 ? b / eps_group_rays : 0;
-  eps_alpha += egrp * K;
-  const float* d = rays_d + b * rays_d_stride;
-  const float norm = sqrtf(d[0] * d[0] + d[1] * d[1] + d[2] * d[2]);
-  const float a_mean = globals[0], a_std = globals[1];
-  const float* prow = flow_params + (b * N) * PP;
-  const float* zrow = z_vals + b * N;
-  for (int k = lane; k < K; k += 32) {
-    const float za0 = eps_alpha[k] * a_std + a_mean;
-    float T = 1.0f;
-    float zn = __ldg(zrow);
-    for (int n = 0; n < N; ++n) {
-      const float* P = prow + (int64_t)n * PP;   // warp-uniform address: one broadcast transaction
-      const float znext = (n < N - 1) ? __ldg(zrow + n + 1) : 0.f;
-      const float dist = ((n < N - 1) ? (znext - zn) : 10.0f) * norm;
-      zn = znext;
-      float za = za0;
-#pragma unroll
-      for (int f = 0; f < F; ++f) za += __ldg(P + f) * tanh_<FAST>(__ldg(P + F + f) * za + __ldg(P + 2 * F + f));
-      const float alpha = 1.0f - exp_<FAST>(-softplus_<FAST>(za) * dist);
-      trans[(b * N + n) * K + k] = T;
-      T = T * ((1.0f - alpha) + 1e-10f);
-    }
-  }
-}
 
 // sum v[0..NV) over the 32 lanes, 16 rows per round; row r of round g0 lands in out[g0 + r]
 template <int NV>
@@ -586,8 +549,8 @@ flow_composite_bwd_kernel(int K, const float* __restrict__ globals, const float*
                           const float* __restrict__ z_vals, const float* __restrict__ rays_d, int rays_d_stride,
                           const float* __restrict__ eps_alpha, const float* __restrict__ eps_rgb, int64_t eps_group_rays,
                           int64_t B, int N, int white_bkgd, const float* __restrict__ g_rgb_map,
-                          const float* __restrict__ g_depth_map, float gl_a_host, float gl_c_host,
-                          const float* __restrict__ g_ld_dev, const float* __restrict__ trans,
+                          const float* __restrict__ g_depth_map, const float* __restrict__ g_ld,
+                          const float* __restrict__ trans,
                           const float* __restrict__ seg_sums, int n_seg,
                           float* __restrict__ g_flow_params, float* __restrict__ g_globals_partial) {
   constexpr int F = FT;
@@ -611,10 +574,10 @@ flow_composite_bwd_kernel(int K, const float* __restrict__ globals, const float*
   if (b >= B) return;
   const int seg_len = N / n_seg;
   const int n_lo = seg * seg_len, n_hi = n_lo + seg_len;
-  // gradient seeds of the two log-det sums of THIS ray: by value (host scalars), or read from the device (B,2) so that
-  // the host never waits for the loss graph and rays of different network calls / loss terms can carry different seeds
-  const float gl_a = g_ld_dev ? g_ld_dev[b * 2 + 0] : gl_a_host;
-  const float gl_c = g_ld_dev ? g_ld_dev[b * 2 + 1] : gl_c_host;
+  // gradient seeds of the two log-det sums of THIS ray, read from the device (B,2) so that the host never waits for the
+  // loss graph and rays of different network calls / loss terms can carry different seeds
+  const float gl_a = g_ld[b * 2 + 0];
+  const float gl_c = g_ld[b * 2 + 1];
   const int64_t egrp = eps_group_rays > 0 ? b / eps_group_rays : 0;
   eps_alpha += egrp * K;
   eps_rgb += egrp * K * 3;
@@ -833,31 +796,23 @@ flow_composite_bwd_kernel(int K, const float* __restrict__ globals, const float*
 int launch_flow_composite_bwd(int fast_math, int F, int K, const float* globals, const float* flow_params, const float* z_vals,
                               const float* rays_d, int rays_d_stride, const float* eps_alpha, const float* eps_rgb,
                               int64_t eps_group_rays, int64_t B, int N, int white_bkgd, const float* g_rgb_map,
-                              const float* g_depth_map, float g_ld_alpha, float g_ld_rgb, const float* g_ld_dev,
-                              float* trans, int trans_valid, const float* seg_sums, int n_seg, float* g_flow_params,
-                              float* g_globals_partial, cudaStream_t s) {
+                              const float* g_depth_map, const float* g_ld, const float* trans, const float* seg_sums,
+                              int n_seg, float* g_flow_params, float* g_globals_partial, cudaStream_t s) {
   if (B == 0) return CFN_OK;
   if (!seg_sums || n_seg < 1) n_seg = 1;
   CFN_CHECK_ARG(N % n_seg == 0 && (N / n_seg) >= 1, "flow_composite_bwd: N=%d is not a multiple of n_segments=%d", N, n_seg);
   CFN_CHECK_ARG(F >= 1 && F <= kMaxF, "flow_composite_bwd: n_flows=%d unsupported (1..%d)", F, kMaxF);
   CFN_CHECK_ARG(N >= 2 && N <= 4096 && K >= 1, "flow_composite_bwd: unsupported N=%d (2..4096) K=%d", N, K);
-  CFN_CHECK_ARG(trans != nullptr, "flow_composite_bwd: the transmittance buffer (B,N,K) is required");
   const int PP = 18 * F;
   size_t smem = (size_t)4 * (((2 * N + 3) & ~3) + 2 * kBwdPB * PP + 2 * 16 * kBwdGLD) * sizeof(float);
   unsigned grid = (unsigned)((B * n_seg + 3) / 4);
-  unsigned grid_pre = (unsigned)((B * 32 + 255) / 256);
 #define CFN_BWD_CASE(FF)                                                                                             \
   case FF: {                                                                                                         \
-    if (!trans_valid) {                                                                                              \
-      auto pre = fast_math ? trans_prepass_kernel<FF, true> : trans_prepass_kernel<FF, false>;                       \
-      pre<<<grid_pre, 256, 0, s>>>(K, globals, flow_params, z_vals, rays_d, rays_d_stride, eps_alpha, eps_group_rays, \
-                                   B, N, trans);                                                                     \
-    }                                                                                                                \
     auto kern = fast_math ? flow_composite_bwd_kernel<FF, true> : flow_composite_bwd_kernel<FF, false>;              \
     if (smem > 48 * 1024) CFN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
     kern<<<grid, 128, smem, s>>>(K, globals, flow_params, z_vals, rays_d, rays_d_stride, eps_alpha, eps_rgb,         \
-                                 eps_group_rays, B, N, white_bkgd, g_rgb_map, g_depth_map, g_ld_alpha, g_ld_rgb,     \
-                                 g_ld_dev, trans, seg_sums, n_seg, g_flow_params, g_globals_partial);                \
+                                 eps_group_rays, B, N, white_bkgd, g_rgb_map, g_depth_map, g_ld, trans, seg_sums,    \
+                                 n_seg, g_flow_params, g_globals_partial);                                           \
   } break;
   switch (F) {
     CFN_BWD_CASE(1) CFN_BWD_CASE(2) CFN_BWD_CASE(3) CFN_BWD_CASE(4) CFN_BWD_CASE(5) CFN_BWD_CASE(6) CFN_BWD_CASE(7)

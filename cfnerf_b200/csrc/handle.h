@@ -78,6 +78,7 @@ int chain_network_fwd(CfnHandle* h, const float* rays, const float* z_vals, cons
                      int64_t B, int N, float* flow_params, float* ws, int save, cudaStream_t s);
 int chain_network_bwd(const CfnHandle* h, const float* g_flow_params, int64_t B, int N, float* ws, float* const* grads,
                       cudaStream_t s);
+int64_t chain_det_scratch_floats(const CfnHandle* h);   // deterministic split-K scratch of chain_network_bwd
 int pack_fp32(CfnHandle* h, const float* const* params, cudaStream_t s);
 
 // tensor-core path (mlp_tc.cu)

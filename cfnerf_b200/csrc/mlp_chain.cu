@@ -7,6 +7,8 @@
 // later GEMM's operand (activations, gradients, weights) is stored ROUNDED to tf32, because the tensor core truncates.
 #include <cuda_bf16.h>
 
+#include <algorithm>
+
 #include "handle.h"
 
 namespace cfn {
@@ -416,6 +418,41 @@ struct Zeroed {
   bool has(const float* q) const { return lo && q >= lo && q < hi; }
 };
 
+// K splits of the weight gradient dW(out_f x in_f) over M points, on the tensor cores (tc) or the CUDA cores; M < 0 gives
+// the cap over every M (what the deterministic scratch is sized for)
+static int64_t wgrad_split(bool tc, int64_t out_f, int64_t in_f, int64_t M) {
+  int64_t split;
+  if (tc) {
+    // one K slice per CTA (pair): (m tiles x n tiles x splits) ~ number of SMs (pairs)
+    const int cg = out_f <= 128 ? 1 : 2;
+    const int64_t bn = in_f >= 256 ? 256 : ((in_f + 15) / 16) * 16;
+    const int64_t tiles = ((out_f + 128 * cg - 1) / (128 * cg)) * ((in_f + bn - 1) / bn);
+    split = (148 / cg) / tiles;
+    if (M >= 0 && split > (M + 255) / 256) split = (M + 255) / 256;
+  } else {
+    const int64_t tiles = ((out_f + 127) / 128) * ((in_f + 127) / 128);
+    split = (148 * 8 + tiles - 1) / tiles;
+    if (M >= 0 && split > (M + 1023) / 1024) split = (M + 1023) / 1024;
+  }
+  return split < 2 ? 2 : split;             // split_k > 1 selects the atomic accumulate path
+}
+
+// floats of deterministic scratch (cfn_set_deterministic): the largest split x (out x in + out) over every weight gradient
+// the backward chain issues, at the larger of the two engines' caps (a tensor-core handle falls back to the CUDA cores
+// for a shape tgemm_supported rejects)
+int64_t chain_det_scratch_floats(const CfnHandle* h) {
+  int64_t need = 0;
+  auto account = [&](int64_t out_f, int64_t in_f) {
+    const int64_t split = std::max(wgrad_split(true, out_f, in_f, -1), wgrad_split(false, out_f, in_f, -1));
+    need = std::max(need, split * (out_f * in_f + out_f));
+  };
+  for (size_t i = 0; i < h->slots.size(); ++i)
+    if (h->wv[i].ld) account(h->slots[i].rows, h->wv[i].ld);
+  account(3 * h->cfg.F, (h->cfg.h_alpha + 7) & ~7);    // amortisation matrices (padded K)
+  account(15 * h->cfg.F, (h->cfg.h_rgb + 7) & ~7);
+  return need;
+}
+
 // dW(out x in) = G(M x out)^T X(M x in), split over the point dimension, atomically accumulated into zeroed dW
 // db (optional): the bias gradient = column sums of G, fused into the tensor-core GEMM when possible
 static int wgrad(const CfnHandle* h, const float* G, int64_t ldg, int out_f, const float* X, int64_t ldx, int in_f, int64_t M,
@@ -428,23 +465,7 @@ static int wgrad(const CfnHandle* h, const float* G, int64_t ldg, int out_f, con
   g.M = out_f; g.N = in_f; g.K = M;
   g.ab_bf16 = h->chain_bf16; g.c_bf16 = 0;   // weight gradients are fp32
   g.split_k = 2;                             // (so that tgemm_supported sees the split-K flavour)
-  int64_t split;
-  if (h->gemm_tc && tgemm_supported(g)) {
-    // one K slice per CTA (pair): (m tiles x n tiles x splits) ~ number of SMs (pairs)
-    const int cg = out_f <= 128 ? 1 : 2;
-    const int bn = in_f >= 256 ? 256 : ((in_f + 15) / 16) * 16;
-    const int tiles = ((out_f + 128 * cg - 1) / (128 * cg)) * ((in_f + bn - 1) / bn);
-    split = (148 / cg) / tiles;
-    const int64_t cap = (M + 255) / 256;
-    if (split > cap) split = cap;
-  } else {
-    const int tiles = ((out_f + 127) / 128) * ((in_f + 127) / 128);
-    split = (M + 1023) / 1024;
-    const int64_t cap = (148 * 8 + tiles - 1) / tiles;
-    if (split > cap) split = cap;
-  }
-  if (split < 2) split = 2;                 // split_k > 1 selects the atomic accumulate path
-  g.split_k = (int)split;
+  g.split_k = (int)wgrad_split(h->gemm_tc && tgemm_supported(g), out_f, in_f, M);
   if (h->deterministic) { g.partials = h->det_scratch; g.partials_floats = h->det_floats; }
   if (db) {
     if (h->gemm_tc && tgemm_can_rowsum(g)) {

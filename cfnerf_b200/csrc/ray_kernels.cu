@@ -299,7 +299,6 @@ __global__ void mean_over_k_kernel(const float* __restrict__ w, float* __restric
 // gradient seed in one pass.  One warp per ray, lanes stride over the K latent samples.
 //   mean_k, unbiased std * K/(K-1) (main:1034), bandwidth h = std * (0.8/K)^(-1/7) + 1e-5 (detached, main:1036),
 //   p_k = exp(-(x_k - t)^2 / (2 h^2)) * (2 pi)^(-1.5) / h, nll = -log(mean_k p_k + 1e-5).
-// partial (B,2) = [sum_c nll_c, sum_c (mean_c - t_c)^2]; g (B,3,K) = grad_scale * d(sum_c nll_c)/d x.
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
@@ -339,30 +338,10 @@ __device__ __forceinline__ void kde_nll_ray(const float* __restrict__ x3, const 
   }
 }
 
-__global__ void kde_nll_kernel(const float* __restrict__ rgb_map, const float* __restrict__ target, int64_t B, int K,
-                               float bw_factor, float grad_scale, float* __restrict__ partial, float* __restrict__ g) {
-  const int64_t b = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  if (b >= B) return;
-  float nll_sum, mse_sum;
-  kde_nll_ray(rgb_map + b * 3 * K, target + b * 3, K, bw_factor, grad_scale, g ? g + b * 3 * K : nullptr, lane, nll_sum, mse_sum);
-  if (lane == 0) { partial[b * 2 + 0] = nll_sum; partial[b * 2 + 1] = mse_sum; }
-}
-
-int launch_kde_nll(const float* rgb_map, const float* target, int64_t B, int K, float grad_scale, float* partial, float* g,
-                   cudaStream_t s) {
-  if (B == 0) return CFN_OK;
-  CFN_CHECK_ARG(K >= 2, "kde_nll: K_samples must be >= 2 (unbiased std)");
-  const float bw = (float)pow(0.8 / (double)K, -1.0 / 7.0);
-  int64_t threads = B * 32;
-  kde_nll_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, s>>>(rgb_map, target, B, K, bw, grad_scale, partial, g);
-  CFN_LAUNCH_CHECK();
-  return CFN_OK;
-}
-
 // ------------------------------------------------------------------------------------------------
 // F1, the whole trainer loss of the shipped recipe (colmap_depth, run_nerf_uncertainty_NF.py:1018-1055) in one launch
-// over the concatenated batch [B_rgb colour rays | B_depth depth rays] (main:1009-1011):
+// over the concatenated batch [B_rgb colour rays | B_depth depth rays] (main:1009-1011); with B_depth = 0 it is the
+// plain KDE-NLL loss (api.kde_nll_loss):
 //   colour rays: K-mean + KDE-NLL as above (the gradient seed w.r.t. rgb_map; their depth gets no gradient);
 //   depth rays : depth = mean_K depth_map (main:1020), squared error against the COLMAP depth (img2mse, main:1053);
 //                d/d depth_map[b,k] = depth_scale * 2 * err / K; their colours get no gradient (rgbs[:N_batch], main:1021).

@@ -104,7 +104,7 @@ class FusedTrainStep:
     """The trainer body (main:1014-1067: render in train mode -> K-mean + KDE-NLL + beta1 * entropy [+ depth_lambda *
     depth MSE on the depth rays] -> backward -> Adam with the reference's lr decay) as a straight chain of C-ABI calls,
     without an autograd graph: cfn_zvals -> cfn_network_fwd(save) -> cfn_flow_composite_fwd (also writes the
-    transmittances the backward reads) -> cfn_trainer_loss (loss + gradient seeds) -> cfn_flow_composite_bwd_dev ->
+    transmittances the backward reads) -> cfn_trainer_loss (loss + gradient seeds) -> cfn_flow_composite_bwd ->
     cfn_network_bwd -> cfn_globals_grad -> [one all-reduce of the flat gradient] -> cfn_adam_step_dev -> cfn_pack_weights.
 
     Same kernels and numbers as `train_step`.  Parameters, gradients and Adam moments each live in ONE flat fp32 buffer
@@ -223,6 +223,12 @@ class FusedTrainStep:
               "cfn_adam_step_dev_f32")
         eng.pack(force=True)        # the next forward reads the re-packed operand copies
 
+    def _eager_step(self, st, world: int):
+        self._forward_backward(st)
+        if world > 1:
+            dist.all_reduce(self.flat_grad, op=dist.ReduceOp.SUM)
+        self._update(world)
+
     @torch.no_grad()
     def step(self, ray_batch, target, t_rand=None, eps_alpha=None, eps_rgb=None, want_loss: bool = True,
              depth_rays=None, target_depth=None):
@@ -251,17 +257,11 @@ class FusedTrainStep:
                 st["eps_a"].copy_(_f32c(eps_alpha, dev).reshape(G, K))
                 st["eps_c"].copy_(_f32c(eps_rgb, dev).reshape(G, K, 3))
             if not self.use_graph:
-                self._forward_backward(st)
-                if w > 1:
-                    dist.all_reduce(self.flat_grad, op=dist.ReduceOp.SUM)
-                self._update(w)
+                self._eager_step(st, w)
             elif st["graph_a"] is None:
                 # first step of this shape: run it eagerly (warm-up: function attributes, allocator), then capture the same
                 # calls for every later step.  The all-reduce stays outside the graphs (NCCL on the current stream).
-                self._forward_backward(st)
-                if w > 1:
-                    dist.all_reduce(self.flat_grad, op=dist.ReduceOp.SUM)
-                self._update(w)
+                self._eager_step(st, w)
                 torch.cuda.synchronize()
                 eager_out = st["out"]                # this step's results; the capture below re-binds st["out"]
                 ga, gb = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()

@@ -162,22 +162,19 @@ class Engine:
                     seg_sums=sg)
 
     def flow_composite_bwd(self, flow_params, z_vals, rays_d, rays_d_stride, eps_alpha, eps_rgb, white_bkgd,
-                           g_rgb, g_depth, g_ld, trans=None, eps_group_rays: int = 0, seg_sums=None):
+                           g_rgb, g_depth, g_ld, *, trans, eps_group_rays: int = 0, seg_sums=None):
         """g_ld: device tensor (B,2) = d loss / d (per-ray sums of the alpha / rgb log-dets); stays on the device (no
-        host sync).  trans / seg_sums: what the training forward wrote (trans None: recomputed into scratch).
+        host sync).  trans / seg_sums: what the training forward (flow_composite(..., want_trans=True)) wrote.
         -> g_flow_params (B*N,18F), g_globals_partial (B*S,8) (sum the rows)."""
         B, N = z_vals.shape
         S = seg_sums.shape[1] if seg_sums is not None else 1
         g_fp = torch.empty_like(flow_params)
         g_glob = torch.empty(B * S, 8, dtype=torch.float32, device=self.device)
-        valid = trans is not None
-        if trans is None:
-            trans = torch.empty(B, N, self.K, dtype=torch.float32, device=self.device)
-        check(self.lib.cfn_flow_composite_bwd_dev(self.h, _ptr(flow_params), _ptr(z_vals), _ptr(rays_d), rays_d_stride,
-                                                  _ptr(eps_alpha), _ptr(eps_rgb), int(eps_group_rays), B, N,
-                                                  int(white_bkgd), _ptr(g_rgb), _ptr(g_depth), _ptr(g_ld), _ptr(trans),
-                                                  int(valid), _ptr(seg_sums), S, _ptr(g_fp), _ptr(g_glob), _stream()),
-              "cfn_flow_composite_bwd_dev")
+        check(self.lib.cfn_flow_composite_bwd(self.h, _ptr(flow_params), _ptr(z_vals), _ptr(rays_d), rays_d_stride,
+                                              _ptr(eps_alpha), _ptr(eps_rgb), int(eps_group_rays), B, N, int(white_bkgd),
+                                              _ptr(g_rgb), _ptr(g_depth), _ptr(g_ld), _ptr(trans), _ptr(seg_sums), S,
+                                              _ptr(g_fp), _ptr(g_glob), _stream()),
+              "cfn_flow_composite_bwd")
         return g_fp, g_glob
 
     def network_bwd(self, g_flow_params, B: int, N: int, ws, grads=None):

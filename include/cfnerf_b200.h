@@ -134,7 +134,7 @@ int cfn_network_bwd(CfnHandle* h, const float* g_flow_params, int64_t B, int N, 
  * (models.py:263,278) for the entropy loss (requesting them selects the training flavour); optional kstats (B,8):
  * mean_k rgb (3), "uncertainty" std (unbiased std * K/(K-1), main:1034/1130) (3), mean_k depth, mean_k disp; optional
  * trans (B,N,K) (training flavour only): the transmittance in front of every sample, which cfn_flow_composite_bwd
- * reads instead of recomputing it; optional seg_sums (B, n_segments, 5, K) (training flavour only; N must be a multiple
+ * reads; optional seg_sums (B, n_segments, 5, K) (training flavour only; N must be a multiple
  * of n_segments): per equal sample range of every ray the sums of w*rgb (3), w*z and w — they let the backward walk the
  * n_segments ranges of a ray in independent warps.  Any optional pointer may be NULL. */
 int cfn_flow_composite_fwd(CfnHandle* h, const float* flow_params, const float* z_vals, const float* rays_d,
@@ -144,9 +144,11 @@ int cfn_flow_composite_fwd(CfnHandle* h, const float* flow_params, const float* 
                            int n_segments, void* stream);
 
 /* Backward (SURVEY.md Appendix A).  g_rgb_map (B,3,K) and g_depth_map (B,K) (NULL = zero) are upstream
- * gradients; g_logdet_alpha / g_logdet_rgb are d loss / d(sum of log-dets) (scalars, e.g. -beta1/(B*N*K)).
- * trans (B,N,K) is REQUIRED device memory: with trans_valid != 0 it holds what cfn_flow_composite_fwd wrote for the
- * same inputs; with trans_valid == 0 it is scratch that this call fills first (an alpha-stack-only pre-pass).
+ * gradients.  g_logdet (B,2), REQUIRED, holds PER-RAY gradient seeds d loss / d(sum of log-dets) in DEVICE memory:
+ * [b][0] = alpha, [b][1] = rgb (e.g. -beta1/(B*N*K)).  The host does not have to wait for the loss graph before it
+ * issues the backward (no device-to-host sync per step), and rays of different network calls / loss terms can carry
+ * different seeds (the depth rays of the shipped recipe take no part in the entropy term, main:1018-1023, 1045).
+ * trans (B,N,K), REQUIRED: what cfn_flow_composite_fwd wrote for the same inputs.
  * seg_sums / n_segments: what cfn_flow_composite_fwd wrote for the same inputs (NULL / 1: one warp walks the whole ray;
  * n_segments > 1 gives small batches n_segments times the parallelism — the reference trains on 512 rays per step).
  * Writes g_flow_params (B*N,18F) and g_globals_partial (B*n_segments,8): per ray and range the
@@ -155,18 +157,8 @@ int cfn_flow_composite_fwd(CfnHandle* h, const float* flow_params, const float* 
 int cfn_flow_composite_bwd(CfnHandle* h, const float* flow_params, const float* z_vals, const float* rays_d,
                            int rays_d_stride, const float* eps_alpha, const float* eps_rgb, int64_t eps_group_rays,
                            int64_t B, int N, int white_bkgd, const float* g_rgb_map, const float* g_depth_map,
-                           float g_logdet_alpha, float g_logdet_rgb, float* trans, int trans_valid,
-                           const float* seg_sums, int n_segments, float* g_flow_params, float* g_globals_partial,
-                           void* stream);
-/* Same, with PER-RAY log-det gradient seeds read from DEVICE memory: g_logdet_dev (B,2), [b][0] = alpha, [b][1] = rgb.
- * The host does not have to wait for the loss graph before it issues the backward (no device-to-host sync per step),
- * and rays of different network calls / loss terms can carry different seeds (the depth rays of the shipped recipe
- * take no part in the entropy term, main:1018-1023, 1045). */
-int cfn_flow_composite_bwd_dev(CfnHandle* h, const float* flow_params, const float* z_vals, const float* rays_d,
-                               int rays_d_stride, const float* eps_alpha, const float* eps_rgb, int64_t eps_group_rays,
-                               int64_t B, int N, int white_bkgd, const float* g_rgb_map, const float* g_depth_map,
-                               const float* g_logdet_dev, float* trans, int trans_valid, const float* seg_sums,
-                               int n_segments, float* g_flow_params, float* g_globals_partial, void* stream);
+                           const float* g_logdet, const float* trans, const float* seg_sums, int n_segments,
+                           float* g_flow_params, float* g_globals_partial, void* stream);
 
 /* ---- A8 stand-alone: raw2outputs (run_nerf_uncertainty_NF.py:411-454) ------------------------ */
 int cfn_raw2outputs_f32(const float* raw, const float* z_vals, const float* rays_d, int rays_d_stride,
@@ -183,20 +175,16 @@ int cfn_merge_sorted_f32(const float* a, const float* b, float* out, int64_t B, 
 /* mean over K of weights (B,N,K) -> (B,N)  (the shared fine grid decision, SURVEY.md A9) */
 int cfn_mean_over_k_f32(const float* w, float* out, int64_t rows, int K, void* stream);
 
-/* ---- F1: K-reduction + KDE negative log-likelihood of the trainer (run_nerf_uncertainty_NF.py:1027-1042) ------ */
-/* rgb_map (B,3,K), target (B,3) -> partial (B,2) = per-ray [sum_c nll_c, sum_c (mean_k rgb - target)^2] and, when
- * g_rgb_map != NULL, g_rgb_map (B,3,K) = grad_scale * d(sum_c nll_c)/d rgb_map (bandwidth detached as in main:1036).
- * The trainer's loss_nll is sum(partial[:,0]) / (3B); pass grad_scale = 1/(3B) to get its gradient directly. */
-int cfn_kde_nll_f32(const float* rgb_map, const float* target, int64_t B, int K, float grad_scale, float* partial,
-                    float* g_rgb_map, void* stream);
-
-/* The whole loss of the shipped recipe (--colmap_depth, --depth_lambda; run_nerf_uncertainty_NF.py:1018-1055) over the
- * concatenated batch [B_rgb colour rays | B_depth depth rays] (main:1009-1011) in one launch.  rgb_map (B,3,K),
- * depth_map (B,K) with B = B_rgb + B_depth; target_rgb (B_rgb,3); target_depth (B_depth) (may be NULL when B_depth = 0).
+/* ---- F1: K-reduction + KDE negative log-likelihood of the trainer (run_nerf_uncertainty_NF.py:1018-1055) ------ */
+/* The whole loss of the shipped recipe (--colmap_depth, --depth_lambda) over the concatenated batch [B_rgb colour rays |
+ * B_depth depth rays] (main:1009-1011) in one launch.  rgb_map (B,3,K), depth_map (B,K) with B = B_rgb + B_depth;
+ * target_rgb (B_rgb,3); target_depth (B_depth) (depth_map and target_depth may be NULL when B_depth = 0).
  * partial (B,3) = per-ray [sum_c nll_c, sum_c (mean_k rgb - target)^2, (mean_k depth - target_depth)^2] (colour rays fill
- * columns 0-1, depth rays column 2).  g_rgb_map (B,3,K) = nll_scale * d(sum_c nll_c)/d rgb_map on colour rays, 0 on
- * depth rays (rgbs[:N_batch], main:1021); g_depth_map (B,K) = depth_scale * d(err^2)/d depth_map on depth rays, 0 on
- * colour rays.  Pass nll_scale = 1/(3 B_rgb) and depth_scale = depth_lambda / B_depth to seed the backward directly. */
+ * columns 0-1, depth rays column 2).  g_rgb_map (B,3,K) = nll_scale * d(sum_c nll_c)/d rgb_map on colour rays (bandwidth
+ * detached as in main:1036), 0 on depth rays (rgbs[:N_batch], main:1021); g_depth_map (B,K) = depth_scale *
+ * d(err^2)/d depth_map on depth rays, 0 on colour rays; either may be NULL when not wanted.  The trainer's loss_nll is
+ * sum(partial[:,0]) / (3 B_rgb): pass nll_scale = 1/(3 B_rgb) and depth_scale = depth_lambda / B_depth to seed the
+ * backward directly. */
 int cfn_trainer_loss_f32(const float* rgb_map, const float* depth_map, const float* target_rgb, const float* target_depth,
                          int64_t B_rgb, int64_t B_depth, int K, float nll_scale, float depth_scale, float* partial,
                          float* g_rgb_map, float* g_depth_map, void* stream);

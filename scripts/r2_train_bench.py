@@ -47,7 +47,6 @@ for B in (512, 4096):
     g_ld = torch.full((B, 2), -0.01 / (B * N * K), device=dev)
     res[f"k2_train_fwd_ms_{B}"] = timeit(lambda: eng.flow_composite(fp, z, rays[:, 3:6], 11, ea, er, False, train=True, want_trans=True))
     res[f"k4_bwd_ms_{B}"] = timeit(lambda: eng.flow_composite_bwd(fp, z, rays[:, 3:6], 11, ea, er, False, g_rgb, None, g_ld, trans=out["trans"], seg_sums=out["seg_sums"]))
-    res[f"k4_bwd_with_prepass_ms_{B}"] = timeit(lambda: eng.flow_composite_bwd(fp, z, rays[:, 3:6], 11, ea, er, False, g_rgb, None, g_ld))
     print(json.dumps({k: v for k, v in res.items() if k.endswith(str(B))}), flush=True)
 
 g = torch.Generator().manual_seed(2)
