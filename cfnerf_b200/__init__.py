@@ -6,8 +6,10 @@ Importing the package does not load the CUDA library; the first call does, and f
 from .api import (configure, gemm, gemm_bf16, install, kde_nll_loss, mean_over_k, merge_sorted, raw2outputs, rays_from_pose, reference_t_schedule,
                   render_image, render_rays, render_rays_host, run_network, sample_pdf, test_latents, trainer_loss)
 from .engine import Engine, engine_for
+from .evaluate import evaluate_view, evaluate_views, sparsification
 from .network import NeRFFlowsParams
 
 __all__ = ["render_rays", "run_network", "raw2outputs", "sample_pdf", "merge_sorted", "mean_over_k", "install", "configure",
-           "kde_nll_loss", "trainer_loss", "rays_from_pose", "gemm", "gemm_bf16", "render_image", "render_rays_host", "Engine", "engine_for", "NeRFFlowsParams", "reference_t_schedule", "test_latents"]
+           "kde_nll_loss", "trainer_loss", "rays_from_pose", "gemm", "gemm_bf16", "render_image", "render_rays_host", "Engine", "engine_for", "NeRFFlowsParams", "reference_t_schedule", "test_latents",
+           "evaluate_view", "evaluate_views", "sparsification"]
 __version__ = "0.1.0"

@@ -41,7 +41,11 @@ SYMBOLS = {
     "cfn_mean_over_k_f32": (_i32, [_f32p, _f32p, _i64, _i32, _vp]),
     "cfn_trainer_loss_f32": (_i32, [_f32p, _f32p, _f32p, _f32p, _i64, _i64, _i32, C.c_float, C.c_float, _f32p, _f32p, _f32p,
                                     _vp]),
-    "cfn_adam_step_f32": (_i32, [_i32, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_i64),
+    "cfn_eval_records_f32": (_i32, [_f32p, _f32p, _f32p, _f32p, _f32p, _i64, _i32, _f32p, _f32p, _f32p, _f32p, _f32p, _f32p,
+                                    _f32p, _vp]),
+    "cfn_sparsification_workspace_bytes": (_i32, [_i64, _i64, _i32, C.POINTER(_sz)]),
+    "cfn_sparsification_f32": (_i32, [_f32p, _f32p, _f32p, _i64, _i64, _i32, _vp, _sz, _f32p, _f32p, _vp]),
+    "cfn_adam_step_f32":(_i32, [_i32, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_i64),
                           C.c_float, C.c_float, C.c_float, C.c_float, _i32, C.c_float, _vp]),
     "cfn_adam_step_dev_f32": (_i32, [_i32, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_i64),
                               _f32p, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, _vp]),

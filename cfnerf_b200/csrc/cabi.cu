@@ -17,7 +17,7 @@ void set_error(const char* fmt, ...) {
 using namespace cfn;
 
 extern "C" const char* cfn_last_error(void) { return g_err; }
-extern "C" int cfn_version(void) { return 102; }
+extern "C" int cfn_version(void) { return 103; }
 
 static void add_slot(CfnHandle* h, const std::string& name, int rows, int cols) {
   ParamSlot s;
@@ -418,6 +418,47 @@ extern "C" int cfn_trainer_loss_f32(const float* rgb_map, const float* depth_map
   CFN_CHECK_ARG(B_depth == 0 || (depth_map && target_depth), "cfn_trainer_loss_f32: depth_map / target_depth is null");
   return launch_trainer_loss(rgb_map, depth_map, target_rgb, target_depth, B_rgb, B_depth, K, nll_scale, depth_scale, partial,
                              g_rgb_map, g_depth_map, (cudaStream_t)stream);
+}
+
+extern "C" int cfn_eval_records_f32(const float* kstats, const float* partial, const float* target_rgb,
+                                    const float* depth_map, const float* target_depth, int64_t B, int K, float* uncertainty,
+                                    float* sq_err, float* abs_err, float* nll, float* depth_uncertainty,
+                                    float* depth_sq_err, float* depth_abs_err, void* stream) {
+  CFN_CHECK_ARG(B >= 0 && K >= 2, "cfn_eval_records_f32: need B >= 0 and K >= 2 (unbiased variance)");
+  CFN_CHECK_ARG(B == 0 || (kstats && partial && target_rgb && uncertainty && sq_err && abs_err && nll),
+                "cfn_eval_records_f32: null argument");
+  CFN_CHECK_ARG(!depth_map || (target_depth && depth_uncertainty && depth_sq_err && depth_abs_err),
+                "cfn_eval_records_f32: depth_map needs target_depth and the three depth outputs");
+  return launch_eval_records(kstats, partial, target_rgb, depth_map, target_depth, B, K, uncertainty, sq_err, abs_err, nll,
+                             depth_uncertainty, depth_sq_err, depth_abs_err, (cudaStream_t)stream);
+}
+
+// checked without touching CUDA, so a host without a GPU can test them
+static int check_sparsification_shape(const char* fn, int64_t n_views, int64_t n_pixels, int n_fractions) {
+  CFN_CHECK_ARG(n_views >= 1 && n_pixels >= 1, "%s: need n_views >= 1 and n_pixels >= 1 (got %lld, %lld)", fn,
+                (long long)n_views, (long long)n_pixels);
+  CFN_CHECK_ARG(n_views <= 65535, "%s: n_views %lld > 65535", fn, (long long)n_views);
+  CFN_CHECK_ARG(n_fractions >= 2, "%s: n_fractions %d < 2", fn, n_fractions);
+  CFN_CHECK_ARG(n_pixels < ((int64_t)1 << 31) && n_views * n_pixels < ((int64_t)1 << 31),
+                "%s: n_views * n_pixels must be < 2^31 (32-bit pixel index)", fn);
+  return CFN_OK;
+}
+
+extern "C" int cfn_sparsification_workspace_bytes(int64_t n_views, int64_t n_pixels, int n_fractions, size_t* out) {
+  CFN_CHECK_ARG(out != nullptr, "cfn_sparsification_workspace_bytes: null argument");
+  const int rc = check_sparsification_shape("cfn_sparsification_workspace_bytes", n_views, n_pixels, n_fractions);
+  if (rc != CFN_OK) return rc;
+  return sparsify_workspace_bytes(n_views, n_pixels, n_fractions, out);
+}
+
+extern "C" int cfn_sparsification_f32(const float* uncertainty, const float* sq_err, const float* abs_err, int64_t n_views,
+                                      int64_t n_pixels, int n_fractions, void* workspace, size_t workspace_bytes,
+                                      float* curves, float* ause, void* stream) {
+  const int rc = check_sparsification_shape("cfn_sparsification_f32", n_views, n_pixels, n_fractions);
+  if (rc != CFN_OK) return rc;
+  CFN_CHECK_ARG(uncertainty && sq_err && abs_err && workspace && curves && ause, "cfn_sparsification_f32: null argument");
+  return launch_sparsify(uncertainty, sq_err, abs_err, n_views, n_pixels, n_fractions, workspace, workspace_bytes, curves,
+                         ause, (cudaStream_t)stream);
 }
 
 extern "C" int cfn_adam_step_f32(int n_tensors, float* const* params, const float* const* grads, float* const* exp_avg,

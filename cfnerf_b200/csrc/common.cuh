@@ -104,6 +104,12 @@ int launch_adam_dev(int n_tensors, float* const* params, const float* const* gra
                     float decay_steps, float beta1, float beta2, float eps, float grad_scale, cudaStream_t s);
 int launch_globals_grad(const float* partial, int64_t B, const float* globals8, float ent_coef, float* out, cudaStream_t s);
 int launch_mean_over_k(const float* w, float* out, int64_t rows, int K, cudaStream_t s);
+int launch_eval_records(const float* kstats, const float* partial, const float* target_rgb, const float* depth_map,
+                        const float* target_depth, int64_t B, int K, float* u, float* sq_err, float* abs_err, float* nll,
+                        float* depth_u, float* depth_sq_err, float* depth_abs_err, cudaStream_t s);
+int sparsify_workspace_bytes(int64_t V, int64_t P, int S, size_t* out);
+int launch_sparsify(const float* u, const float* e, const float* a, int64_t V, int64_t P, int S, void* workspace,
+                    size_t workspace_bytes, float* curves, float* ause, cudaStream_t s);
 
 int launch_flow_composite_fwd(int fast_math, int F, int K, const float* globals, const float* flow_params, const float* z_vals,
                               const float* rays_d, int rays_d_stride, const float* eps_alpha, const float* eps_rgb,

@@ -189,6 +189,28 @@ int cfn_trainer_loss_f32(const float* rgb_map, const float* depth_map, const flo
                          int64_t B_rgb, int64_t B_depth, int K, float nll_scale, float depth_scale, float* partial,
                          float* g_rgb_map, float* g_depth_map, void* stream);
 
+/* ---- F5: evaluation of the predictive uncertainty (PSNR, KDE-NLL, AUSE; INTEGRATION.md §2) ----------------------- */
+/* Per-pixel records of B rays from what K2 (kstats (B,8)) and cfn_trainer_loss_f32 (partial (B,3), B_rgb = B) wrote for
+ * the same maps, target_rgb (B,3):  uncertainty = (s_0^2 + s_1^2 + s_2^2) / 3 with s the "uncertainty" std of kstats;
+ * sq_err = partial[:,1] / 3; abs_err = mean_c |mean_k rgb - target|; nll = partial[:,0] / 3 (the KDE-NLL averaged over
+ * the channels).  depth_map (B,K) may be NULL; when given, target_depth (B) is required and depth_uncertainty = unbiased
+ * variance over k, depth_sq_err / depth_abs_err = squared / absolute error of mean_k depth.  K >= 2. */
+int cfn_eval_records_f32(const float* kstats, const float* partial, const float* target_rgb, const float* depth_map,
+                         const float* target_depth, int64_t B, int K, float* uncertainty, float* sq_err, float* abs_err,
+                         float* nll, float* depth_uncertainty, float* depth_sq_err, float* depth_abs_err, void* stream);
+
+/* Sparsification curves and AUSE of n_views views of n_pixels pixels each (1 <= n_views <= 65535, n_views * n_pixels
+ * < 2^31, n_fractions = S >= 2).  uncertainty, sq_err and abs_err are (V,P) and must be finite and >= 0 (device
+ * pointers: not checked).  For i < S, m_i = P - floor(i P / S) pixels are kept, the least uncertain first (stable: ties
+ * keep the lower pixel index).  curves (V,4,S): [RMSE by uncertainty, RMSE oracle (by sq_err), MAE by uncertainty, MAE
+ * oracle (by abs_err)], each divided by its value at i = 0 (0 when that is 0); ause (V,2) [RMSE, MAE] =
+ * sum_{i<S-1} (d_i + d_{i+1}) / (2S), d = curve - oracle.  Bitwise deterministic.  workspace: at least
+ * cfn_sparsification_workspace_bytes (which asks CUB for its temporary storage) bytes of device memory, else CFN_ENOMEM. */
+int cfn_sparsification_workspace_bytes(int64_t n_views, int64_t n_pixels, int n_fractions, size_t* out);
+int cfn_sparsification_f32(const float* uncertainty, const float* sq_err, const float* abs_err, int64_t n_views,
+                           int64_t n_pixels, int n_fractions, void* workspace, size_t workspace_bytes, float* curves,
+                           float* ause, void* stream);
+
 /* ---- F3: fused optimiser step (torch.optim.Adam, run_nerf_uncertainty_NF.py:339, 1065-1077) ------------------- */
 /* One launch over all n_tensors parameter tensors.  The four pointer arrays and numels live in HOST memory and hold
  * DEVICE pointers / element counts; `step` is the 1-based step count (bias correction), `lr` the already decayed
