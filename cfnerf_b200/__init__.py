@@ -7,9 +7,10 @@ from .api import (configure, gemm, gemm_bf16, install, kde_nll_loss, mean_over_k
                   render_image, render_rays, render_rays_host, run_network, sample_pdf, test_latents, trainer_loss)
 from .engine import Engine, engine_for
 from .evaluate import evaluate_view, evaluate_views, sparsification
+from .field import field_grid, query_field
 from .network import NeRFFlowsParams
 
 __all__ = ["render_rays", "run_network", "raw2outputs", "sample_pdf", "merge_sorted", "mean_over_k", "install", "configure",
            "kde_nll_loss", "trainer_loss", "rays_from_pose", "gemm", "gemm_bf16", "render_image", "render_rays_host", "Engine", "engine_for", "NeRFFlowsParams", "reference_t_schedule", "test_latents",
-           "evaluate_view", "evaluate_views", "sparsification"]
+           "evaluate_view", "evaluate_views", "sparsification", "query_field", "field_grid"]
 __version__ = "0.1.0"

@@ -45,6 +45,7 @@ SYMBOLS = {
                                     _f32p, _vp]),
     "cfn_sparsification_workspace_bytes": (_i32, [_i64, _i64, _i32, C.POINTER(_sz)]),
     "cfn_sparsification_f32": (_i32, [_f32p, _f32p, _f32p, _i64, _i64, _i32, _vp, _sz, _f32p, _f32p, _vp]),
+    "cfn_field_stats_f32": (_i32, [_vp, _f32p, _f32p, _f32p, _i64, _f32p, _vp]),
     "cfn_adam_step_f32":(_i32, [_i32, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_i64),
                           C.c_float, C.c_float, C.c_float, C.c_float, _i32, C.c_float, _vp]),
     "cfn_adam_step_dev_f32": (_i32, [_i32, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_i64),

@@ -461,6 +461,22 @@ extern "C" int cfn_sparsification_f32(const float* uncertainty, const float* sq_
                          ause, (cudaStream_t)stream);
 }
 
+extern "C" int cfn_field_stats_f32(const CfnHandle* h, const float* flow_params, const float* eps_alpha,
+                                   const float* eps_rgb, int64_t M, float* out, void* stream) {
+  CFN_CHECK_ARG(h != nullptr, "cfn_field_stats_f32: null handle");
+  CFN_CHECK_ARG(M >= 0, "cfn_field_stats_f32: negative point count %lld", (long long)M);
+  CFN_CHECK_ARG(M == 0 || (flow_params && eps_alpha && eps_rgb && out), "cfn_field_stats_f32: null argument");
+  if (!h->packed) {
+    set_error("cfn_field_stats_f32: call cfn_pack_weights first");
+    return CFN_ESTATE;
+  }
+  if (M == 0) return CFN_OK;
+  // the accurate functions in the fp32 check mode, one-MUFU transcendentals behind the tensor-core modes (as K2)
+  const int fast = (h->cfg.precision != CFN_PREC_FP32) ? 1 : 0;
+  return launch_field_stats(fast, h->cfg.F, h->cfg.K, h->globals, flow_params, eps_alpha, eps_rgb, M, out,
+                            (cudaStream_t)stream);
+}
+
 extern "C" int cfn_adam_step_f32(int n_tensors, float* const* params, const float* const* grads, float* const* exp_avg,
                                  float* const* exp_avg_sq, const int64_t* numels, float lr, float beta1, float beta2,
                                  float eps, int step, float grad_scale, void* stream) {

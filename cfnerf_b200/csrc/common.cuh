@@ -110,6 +110,8 @@ int launch_eval_records(const float* kstats, const float* partial, const float* 
 int sparsify_workspace_bytes(int64_t V, int64_t P, int S, size_t* out);
 int launch_sparsify(const float* u, const float* e, const float* a, int64_t V, int64_t P, int S, void* workspace,
                     size_t workspace_bytes, float* curves, float* ause, cudaStream_t s);
+int launch_field_stats(int fast_math, int F, int K, const float* globals, const float* flow_params, const float* eps_alpha,
+                       const float* eps_rgb, int64_t M, float* out, cudaStream_t s);
 
 int launch_flow_composite_fwd(int fast_math, int F, int K, const float* globals, const float* flow_params, const float* z_vals,
                               const float* rays_d, int rays_d_stride, const float* eps_alpha, const float* eps_rgb,

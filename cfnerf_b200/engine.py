@@ -161,7 +161,19 @@ class Engine:
         return dict(rgb_map=rgb, disp_map=disp, depth_map=depth, raw=raw, weights=w, logdet_sums=ld, kstats=ks, trans=tr,
                     seg_sums=sg)
 
-    def flow_composite_bwd(self, flow_params, z_vals, rays_d, rays_d_stride, eps_alpha, eps_rgb, white_bkgd,
+    def field_stats(self, flow_params, eps_alpha, eps_rgb, out=None):
+        """flow_params (M,18F) from network(B=M, N=1, pts=, viewdirs=), base draws eps_alpha (K) / eps_rgb (K,3) ->
+        (M,8) [sigma mean, sigma std, rgb mean (3), rgb std (3)] over the K draws (cfn_field_stats_f32; definitions in
+        cfnerf_b200/field.py).  `out`: optional contiguous (M,8) fp32 device tensor to write into."""
+        self.pack()
+        M = flow_params.shape[0]
+        if out is None:
+            out = torch.empty(M, 8, dtype=torch.float32, device=self.device)
+        check(self.lib.cfn_field_stats_f32(self.h, _ptr(flow_params), _ptr(eps_alpha), _ptr(eps_rgb), M, _ptr(out),
+                                           _stream()), "cfn_field_stats_f32")
+        return out
+
+    def flow_composite_bwd(self,flow_params, z_vals, rays_d, rays_d_stride, eps_alpha, eps_rgb, white_bkgd,
                            g_rgb, g_depth, g_ld, *, trans, eps_group_rays: int = 0, seg_sums=None):
         """g_ld: device tensor (B,2) = d loss / d (per-ray sums of the alpha / rgb log-dets); stays on the device (no
         host sync).  trans / seg_sums: what the training forward (flow_composite(..., want_trans=True)) wrote.

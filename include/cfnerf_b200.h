@@ -211,6 +211,18 @@ int cfn_sparsification_f32(const float* uncertainty, const float* sq_err, const 
                            int64_t n_pixels, int n_fractions, void* workspace, size_t workspace_bytes, float* curves,
                            float* ause, void* stream);
 
+/* ---- F6: field-space statistics over the K latent draws (INTEGRATION.md §2) ------------------------------------- */
+/* For M query points whose flow records flow_params (M, 18F) cfn_network_fwd wrote (explicit points: B = M, N = 1),
+ * run both flow stacks for the K base draws eps_alpha (K) / eps_rgb (K,3) and reduce over k on the device:
+ * out (M,8) = [mean sigma, std sigma, mean rgb (3), std rgb (3)] with sigma_k = softplus(raw alpha) (main:424),
+ * rgb_k = sigmoid(raw rgb) (main:431), std = sqrt(sum_k (x_k - mean)^2 / (K-1)) and 0 when K = 1 (the plain sample
+ * std, not the "uncertainty" std of kstats, which carries an extra K/(K-1)).  Welford accumulation in fp32 over
+ * k = 0..K-1: bitwise repeatable and independent of the other points of the call.  The transcendentals follow the
+ * handle's precision as in cfn_flow_composite_fwd.  Arguments are checked before any CUDA call; M == 0 launches nothing.
+ * Added without a cfn_version() change: callers detect the feature by the presence of this symbol. */
+int cfn_field_stats_f32(const CfnHandle* h, const float* flow_params, const float* eps_alpha, const float* eps_rgb,
+                        int64_t M, float* out, void* stream);
+
 /* ---- F3: fused optimiser step (torch.optim.Adam, run_nerf_uncertainty_NF.py:339, 1065-1077) ------------------- */
 /* One launch over all n_tensors parameter tensors.  The four pointer arrays and numels live in HOST memory and hold
  * DEVICE pointers / element counts; `step` is the 1-based step count (bias correction), `lr` the already decayed
