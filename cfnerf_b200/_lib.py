@@ -30,6 +30,8 @@ SYMBOLS = {
                                _f32p, _vp]),
     "cfn_workspace_bytes": (_i32, [_vp, _i64, _i32, C.POINTER(_sz)]),
     "cfn_network_fwd": (_i32, [_vp, _f32p, _f32p, _f32p, _f32p, _i64, _i32, _f32p, _vp, _sz, _i32, _vp]),
+    "cfn_network_fwd_composite": (_i32, [_vp, _f32p, _f32p, _i64, _i32, _f32p, _vp, _sz, _f32p, _i32, _f32p, _f32p, _i32,
+                                         _f32p, _f32p, _f32p, _f32p, _vp]),
     "cfn_network_bwd": (_i32, [_vp, _f32p, _i64, _i32, _vp, _sz, C.POINTER(_vp), _i32, _vp]),
     "cfn_flow_composite_fwd": (_i32, [_vp, _f32p, _f32p, _f32p, _i32, _f32p, _f32p, _i64, _i64, _i32, _i32, _f32p, _f32p,
                                       _f32p, _f32p, _f32p, _f32p, _f32p, _f32p, _f32p, _i32, _vp]),

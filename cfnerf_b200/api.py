@@ -190,6 +190,20 @@ def latent_groups(B: int, N: int, netchunk: int):
     return 0, 1
 
 
+# Latent draws per ray up to which the fused network + compositing kernel is faster than K1 -> K2 (see
+# fused_composite): its two compositing warps per CTA have two tile-times per tile of rays, which covers K = 32 (one
+# latent group per ray) with room to spare but not K = 128, where they would set the pace of the kernel.
+FUSED_MAX_K = 32
+
+
+def fused_composite(eng, N: int, need_weights: bool, group_rays: int) -> bool:
+    """Test-mode render passes that run network + compositing as one kernel (Engine.network(..., composite=)):
+    tensor-core precision, no weights / raw output, whole rays per 128-point tile, the compiled F = 4 flavour, one
+    latent-draw set for every ray and K <= FUSED_MAX_K.  Everything else keeps the two launches."""
+    return (eng.precision in ("fp16", "bf16") and not need_weights and 128 % N == 0 and eng.F == 4 and group_rays == 0
+            and eng.K <= FUSED_MAX_K)
+
+
 def _latent_draws(module, K: int, device, train: bool, G: int, eps_alpha, eps_rgb, batch: str):
     """The base latent draws of a batch that makes G network calls -> (eps_a, eps_c): (K), (K,3) when G = 1, else
     (G,K), (G,K,3).  Without eps_alpha: in train mode one fresh (alpha, rgb) pair per network call, drawn in the
@@ -360,6 +374,10 @@ def render_rays(ray_batch, network_fn, network_query_fn=None, N_samples=128, is_
                 return dict(rgb_map=rgb, disp_map=disp, depth_map=depth, raw=raw, weights=w if need_w else None,
                             loss_entropy=ent)
             with torch.no_grad():
+                if fused_composite(e, N, need_w, group_rays):
+                    return e.network(B, N, rays=rays, z_vals=z, composite=dict(
+                        rays_d=rays[:, 3:6], rays_d_stride=11, eps_alpha=eps_a, eps_rgb=eps_c, white_bkgd=bool(white_bkgd),
+                        want_kstats=want_kstats))
                 fp = e.network(B, N, rays=rays, z_vals=z)
                 return e.flow_composite(fp, z, rays[:, 3:6], 11, eps_a, eps_c, bool(white_bkgd),
                                         want_raw=False, want_weights=need_w, want_kstats=want_kstats)

@@ -283,6 +283,38 @@ extern "C" int cfn_network_fwd(CfnHandle* h, const float* rays, const float* z_v
   return CFN_OK;
 }
 
+extern "C" int cfn_network_fwd_composite(CfnHandle* h, const float* rays, const float* z_vals, int64_t B, int N,
+                                         float* flow_params, void* workspace, size_t workspace_bytes, const float* rays_d,
+                                         int rays_d_stride, const float* eps_alpha, const float* eps_rgb, int white_bkgd,
+                                         float* rgb_map, float* disp_map, float* depth_map, float* kstats, void* stream) {
+  CFN_CHECK_ARG(h && B >= 0 && N >= 1, "cfn_network_fwd_composite: bad argument");
+  CFN_CHECK_ARG(B == 0 || (rays && z_vals && flow_params && rays_d && eps_alpha && eps_rgb && rgb_map && disp_map && depth_map),
+                "cfn_network_fwd_composite: null argument");
+  CFN_CHECK_ARG(h->tc, "cfn_network_fwd_composite: needs a tensor-core precision (bf16 / fp16)");
+  CFN_CHECK_ARG(128 % N == 0, "cfn_network_fwd_composite: N = %d must divide 128 (whole rays per tile)", N);
+  CFN_CHECK_ARG(h->cfg.F == 4, "cfn_network_fwd_composite: n_flows = %d unsupported (4)", h->cfg.F);
+  if (!h->packed) {
+    set_error("cfn_network_fwd_composite: call cfn_pack_weights first");
+    return CFN_ESTATE;
+  }
+  if (B == 0) return CFN_OK;
+  size_t need = 0;
+  cfn_workspace_bytes(h, B * N, 0, &need);
+  if (workspace_bytes < need || (!workspace && need)) {
+    set_error("cfn_network_fwd_composite: workspace %zu bytes < required %zu", workspace_bytes, need);
+    return CFN_ENOMEM;
+  }
+  cudaStream_t s = (cudaStream_t)stream;
+  if (h->tc_dirty) {
+    int rc = tc_pack(h, s);
+    if (rc != CFN_OK) return rc;
+    h->tc_dirty = 0;
+  }
+  const TcComposite c{h->globals, rays_d, rays_d_stride, eps_alpha, eps_rgb, h->cfg.K, white_bkgd, rgb_map, disp_map,
+                      depth_map, kstats};
+  return tc_network_fwd(h, rays, z_vals, nullptr, nullptr, B, N, flow_params, workspace, workspace_bytes, s, &c);
+}
+
 extern "C" int cfn_network_bwd(CfnHandle* h, const float* g_flow_params, int64_t B, int N, void* workspace,
                                size_t workspace_bytes, float* const* grads, int n_params, void* stream) {
   CFN_CHECK_ARG(h && g_flow_params && grads && workspace, "cfn_network_bwd: null argument");

@@ -87,6 +87,16 @@ void tc_destroy(CfnHandle* h);
 int tc_pack(CfnHandle* h, cudaStream_t s);
 size_t tc_workspace_bytes(const CfnHandle* h, int64_t n_points);
 int tc_debug_profile(CfnHandle* h, unsigned long long* out_host, int n);
+// K2's render arguments for the fused network + compositing kernel (tc_network_fwd with comp != nullptr)
+struct TcComposite {
+  const float* globals;
+  const float* rays_d; int rays_d_stride;
+  const float* eps_alpha; const float* eps_rgb;   // one (K) / (K,3) draw set for every ray
+  int K; int white_bkgd;
+  float* rgb_map; float* disp_map; float* depth_map;
+  float* kstats;                                  // optional
+};
 int tc_network_fwd(CfnHandle* h, const float* rays, const float* z_vals, const float* pts, const float* viewdirs,
-                   int64_t B, int N, float* flow_params, void* ws, size_t ws_bytes, cudaStream_t s);
+                   int64_t B, int N, float* flow_params, void* ws, size_t ws_bytes, cudaStream_t s,
+                   const TcComposite* comp = nullptr);
 }  // namespace cfn

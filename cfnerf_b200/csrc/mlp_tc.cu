@@ -21,6 +21,7 @@
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
+#include "flow_step.cuh"
 #include "handle.h"
 #include "ptx_sm100.cuh"
 
@@ -44,6 +45,10 @@ constexpr int TC_SRC_GP = 8, TC_SRC_GD = 9;   // host-side source ids; the devic
                                               // gamma(p) and gamma(d) time-share one 16 KB tile (see TcPlanDev::gd_step)
 constexpr int TC_THREADS = 384;             // warps 0..7 encode/epilogue, 8 TMEM alloc, 9 (profiling), 10 TMA, 11 MMA
 constexpr int TC_W_ALLOC = 8, TC_W_WATCH = 9, TC_W_TMA = 10, TC_W_MMA = 11;   // the scheduler favours high warp ids
+// COMPOSITE (K1 + K2's render flavour in one kernel): warps 8 and 9, idle once TMEM is allocated (the watcher only runs
+// in profiling builds), composite the rays of finished tiles ("flow warps"): tile i of a CTA goes to warp 8 + i % 2.
+constexpr int TC_FLOW_WARPS = 2;
+constexpr int TC_FLOW_BARS = 2 * TC_FLOW_WARPS;   // rec_ready[2] + rec_free[2], after the bias staging area
 constexpr int TC_MAX_STAGES = 8;
 constexpr int CG = 2;                       // cta_group::2: every tile of 256 points is shared by a CTA pair
 
@@ -245,11 +250,63 @@ __device__ __forceinline__ void encode_row(float x, float y, float z, int L, uin
   }
 }
 
-template <bool FP16>
+__device__ __forceinline__ void mbar_arrive_local(uint32_t bar) {   // default .release.cta
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(bar) : "memory");
+}
+
+// Composite one ray in the fused kernel: K2's render flavour (flow_composite_fwd_kernel<9, false, true, 4>: FAST, F = 4)
+// with the same operations in the same order, so the maps are bitwise equal to K1 -> K2.  The records are read with
+// coherent (L1-cached, never .nc) warp-uniform 16-byte loads: this kernel wrote them moments ago.
+__device__ __forceinline__ void composite_ray_fused(const TcArgs& a, const TcComposite& c, int64_t b, int lane) {
+  constexpr int F = 4, PP = 18 * F;
+  const int N = a.N, K = c.K;
+  const float* zr = a.z_vals + b * N;
+  const float* d = c.rays_d + b * c.rays_d_stride;
+  const float dx = d[0], dy = d[1], dz = d[2];
+  const float norm = sqrtf(dx * dx + dy * dy + dz * dz);
+  const float a_mean = c.globals[0], a_std = c.globals[1];
+  const float c_mean0 = c.globals[2], c_mean1 = c.globals[3], c_mean2 = c.globals[4];
+  const float c_std0 = c.globals[5], c_std1 = c.globals[6], c_std2 = c.globals[7];
+  const float* prow = a.flow_params + b * N * PP;
+  float st_sum[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
+  const int KG = (K + 31) / 32;
+  for (int kg = 0; kg < KG; ++kg) {
+    const int k = kg * 32 + lane;
+    const bool active = k < K;
+    const float ea = active ? c.eps_alpha[k] : 0.f;
+    const float e0 = active ? c.eps_rgb[k * 3 + 0] : 0.f, e1 = active ? c.eps_rgb[k * 3 + 1] : 0.f,
+                e2 = active ? c.eps_rgb[k * 3 + 2] : 0.f;
+    const float za0 = ea * a_std + a_mean;
+    const float zc00 = e0 * c_std0 + c_mean0, zc01 = e1 * c_std1 + c_mean1, zc02 = e2 * c_std2 + c_mean2;
+    RayAcc ray;
+    for (int n = 0; n < N; ++n) {
+      const float* P = prow + n * PP;
+      // pull the record four samples ahead into L1: its 288 bytes touch at most three 128-byte lines, and four probes
+      // 92 bytes apart hit every one of them
+      if (lane < 4 && n + 4 < N) asm volatile("prefetch.global.L1 [%0];" :: "l"(P + 4 * PP + lane * 23));
+      float rec[PP];
+#pragma unroll
+      for (int j = 0; j < PP / 4; ++j) {
+        const float4 q4 = __ldca(reinterpret_cast<const float4*>(P) + j);
+        rec[4 * j] = q4.x; rec[4 * j + 1] = q4.y; rec[4 * j + 2] = q4.z; rec[4 * j + 3] = q4.w;
+      }
+      const float z = __ldg(zr + n);
+      const float dist = ((n < N - 1) ? (__ldg(zr + n + 1) - z) : 10.0f) * norm;
+      const float za = flow_alpha<true>(rec, F, za0);
+      float z0 = zc00, z1 = zc01, z2 = zc02;
+      flow_rgb<true>(rec, F, z0, z1, z2);
+      composite_sample<true>(ray, za, z0, z1, z2, z, dist);
+    }
+    finish_ray(ray, c.white_bkgd, active, b, K, k, c.rgb_map, c.disp_map, c.depth_map, st_sum);
+  }
+  if (c.kstats) write_kstats(b, K, lane, c.rgb_map, st_sum, c.kstats);
+}
+
+template <bool FP16, bool COMPOSITE>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 mlp_tc_kernel(const __grid_constant__ CUtensorMap tm_big, const __grid_constant__ CUtensorMap tm_small,
               const __grid_constant__ CUtensorMap tm_bias,
-              const __grid_constant__ TcPlanDev plan, const TcArgs a) {
+              const __grid_constant__ TcPlanDev plan, const TcArgs a, const TcComposite comp) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   // 1024-byte alignment is required by SWIZZLE_128B; the dynamic segment is the only shared allocation
   const uint32_t smem_base = smem_u32(smem_raw);
@@ -260,6 +317,9 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tm_big, const __grid_constant_
   const uint32_t gp_base = act_base + act_chunks * TC_CHUNK_BYTES;
   const uint32_t stage_base = gp_base + TC_CHUNK_BYTES;
   TcBarriers* bars = reinterpret_cast<TcBarriers*>(smem_gen + (stage_base - smem_base) + (size_t)a.stages * a.stage_bytes);
+  // COMPOSITE: rec_ready[j] (tile i's records are in memory, j = i % 2) and rec_free[j] (flow warp j has taken tile i),
+  // after the bias staging area so that the plain kernel's layout is untouched
+  uint64_t* fbars = reinterpret_cast<uint64_t*>(reinterpret_cast<uint8_t*>(bars) + sizeof(TcBarriers) + 512 * sizeof(float));
 
   // the shuffle tells the compiler that `warp` is warp-uniform: the role branches below are then uniform branches and
   // the schedule arithmetic of the producer / issuer warps lives in the uniform datapath (no R2UR in front of every MMA)
@@ -280,6 +340,8 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tm_big, const __grid_constant_
     mbar_init(bar_local(&bars->out_done), 8 * CG);
     mbar_init(bar_local(&bars->in_ready), 4 * CG);
     mbar_init(bar_local(&bars->gd_ready), 4 * CG);
+    if (COMPOSITE)
+      for (int j = 0; j < TC_FLOW_BARS; ++j) mbar_init(bar_local(fbars + j), 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == TC_W_ALLOC) {
@@ -454,6 +516,19 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tm_big, const __grid_constant_
         }
       }
     }
+  } else if (COMPOSITE && (warp == TC_W_ALLOC || warp == TC_W_WATCH)) {
+    // ================================= flow warps (COMPOSITE) =================================
+    // Each has two tile-times for the 128 / N whole rays of its tile, on the MUFU and issue slots the tensor-core chain
+    // leaves idle.
+    const int fw = warp - TC_W_ALLOC;
+    const uint32_t ready_bar = bar_local(fbars + fw), free_bar = bar_local(fbars + TC_FLOW_WARPS + fw);
+    for (int64_t i = fw; unit0 + i * n_grid_units < a.n_units; i += TC_FLOW_WARPS) {
+      mbar_wait(ready_bar, (uint32_t)(i / TC_FLOW_WARPS) & 1u);   // acquire: the records of tile i
+      __syncwarp();
+      if (lane == 0) mbar_arrive_local(free_bar);
+      const int64_t m0 = ((unit0 + i * n_grid_units) * CG + rank) * 128;
+      for (int64_t b = m0 / a.N; b < (m0 + 128) / a.N && b * a.N < a.M; ++b) composite_ray_fused(a, comp, b, lane);
+    }
   } else if (warp == TC_W_WATCH) {
     // profiling only: time at which each stage's TMA data has landed (independent of the MMA thread's progress)
     if (a.prof && blockIdx.x == 0 && rank == 0) {
@@ -476,6 +551,7 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tm_big, const __grid_constant_
     const int row = q * 32 + lane;                         // TMEM lane == row of the tile owned by this thread
     const uint32_t tmem_row = tmem_base + ((uint32_t)(q * 32) << 16);
     uint32_t acc_cnt = 0, split_cnt = 0;
+    uint32_t n_tiles = 0;   // COMPOSITE: tiles of this CTA handed to the flow warps
     Prof prof{(a.prof && blockIdx.x == 0 && warp == 0 && lane == 0) ? a.prof : nullptr, 0};
     Prof prof2{nullptr, 0};   // (role 3 of the profile buffer is used by the TMA-landing watcher in warp 3)
     float* sbias = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(bars) + sizeof(TcBarriers));   // 512 floats
@@ -706,6 +782,14 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tm_big, const __grid_constant_
           }
         }
         if (st.kind == 2) epi_sync();                 // everyone is done with this step's bias (and the staged outputs)
+        if (COMPOSITE && g == plan.n_steps - 1 && tid_e == 0) {
+          // every record of the tile is stored: the bar.sync above orders the 256 threads' stores before this release.
+          // rec_free keeps this arrival from running two phases ahead of flow warp j (mbarrier parity aliasing)
+          const uint32_t j = n_tiles % TC_FLOW_WARPS, use = n_tiles / TC_FLOW_WARPS;
+          if (use > 0) mbar_wait(bar_local(fbars + TC_FLOW_WARPS + j), (use - 1u) & 1u);
+          mbar_arrive_local(bar_local(fbars + j));
+          ++n_tiles;
+        }
         {
           const int gn = (g + 1 < plan.n_steps) ? g + 1 : 0;
           if (gn != 0 || unit + n_grid_units < a.n_units) load_bias(gn);
@@ -934,7 +1018,8 @@ int tc_create(CfnHandle* h) {
   if (prop.major != 10) { set_error("tensor-core path needs sm_100 (found sm_%d%d)", prop.major, prop.minor); return CFN_EINVAL; }
   p->num_sms = prop.multiProcessorCount;
   p->stage_bytes = (256 / CG) * 128;
-  const size_t fixed = (size_t)(AC + 1) * TC_CHUNK_BYTES + sizeof(TcBarriers) + 2048;   // + bias staging (512 floats)
+  // + bias staging (512 floats) + the fused kernel's flow barriers (they fit in the last stage's slack for every W)
+  const size_t fixed = (size_t)(AC + 1) * TC_CHUNK_BYTES + sizeof(TcBarriers) + 2048 + TC_FLOW_BARS * sizeof(uint64_t);
   const size_t smem_max = (size_t)prop.sharedMemPerBlockOptin;
   int stages = (int)((smem_max - fixed) / p->stage_bytes);
   if (stages > TC_MAX_STAGES) stages = TC_MAX_STAGES;
@@ -976,7 +1061,8 @@ int tc_create(CfnHandle* h) {
   auto set_attr = [&](const void* fnp) {
     return cudaFuncSetAttribute(fnp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem_bytes) == cudaSuccess;
   };
-  const bool ok = fp16 ? set_attr((const void*)mlp_tc_kernel<true>) : set_attr((const void*)mlp_tc_kernel<false>);
+  const bool ok = fp16 ? set_attr((const void*)mlp_tc_kernel<true, false>) && set_attr((const void*)mlp_tc_kernel<true, true>)
+                        : set_attr((const void*)mlp_tc_kernel<false, false>) && set_attr((const void*)mlp_tc_kernel<false, true>);
   if (!ok) return fail("cudaFuncSetAttribute(max dynamic shared memory)");
   return CFN_OK;
 }
@@ -1041,7 +1127,7 @@ int tc_debug_profile(CfnHandle* h, unsigned long long* out_host, int n) {
 }
 
 int tc_network_fwd(CfnHandle* h, const float* rays, const float* z_vals, const float* pts, const float* viewdirs,
-                   int64_t B, int N, float* flow_params, void*, size_t, cudaStream_t s) {
+                   int64_t B, int N, float* flow_params, void*, size_t, cudaStream_t s, const TcComposite* comp) {
   TcPlan* p = h->tc;
   TcArgs a;
   a.rays = rays; a.z_vals = z_vals; a.pts = pts; a.viewdirs = viewdirs;
@@ -1063,8 +1149,10 @@ int tc_network_fwd(CfnHandle* h, const float* rays, const float* z_vals, const f
   attr[0].val.clusterDim.x = CG; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
   const bool fp16 = h->cfg.precision == CFN_PREC_FP16;
-  const cudaError_t e = fp16 ? cudaLaunchKernelEx(&cfg, mlp_tc_kernel<true>, p->tm_big, p->tm_small, p->tm_bias, p->dev, a)
-                             : cudaLaunchKernelEx(&cfg, mlp_tc_kernel<false>, p->tm_big, p->tm_small, p->tm_bias, p->dev, a);
+  const TcComposite c = comp ? *comp : TcComposite{};
+  auto kern = fp16 ? (comp ? mlp_tc_kernel<true, true> : mlp_tc_kernel<true, false>)
+                   : (comp ? mlp_tc_kernel<false, true> : mlp_tc_kernel<false, false>);
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, p->tm_big, p->tm_small, p->tm_bias, p->dev, a, c);
   if (e != cudaSuccess) { set_error("mlp_tc_kernel launch failed: %s", cudaGetErrorString(e)); return CFN_ECUDA; }
   return CFN_OK;
 }

@@ -125,11 +125,26 @@ class Engine:
               "cfn_zvals_f32")
         return z
 
-    def network(self, B: int, N: int, rays=None, z_vals=None, pts=None, viewdirs=None, save: bool = False):
-        """-> flow_params (B*N, 18F) [, workspace when save]"""
+    def network(self, B: int, N: int, rays=None, z_vals=None, pts=None, viewdirs=None, save: bool = False,
+                composite=None):
+        """-> flow_params (B*N, 18F) [, workspace when save].
+        composite=dict(rays_d=, rays_d_stride=, eps_alpha=, eps_rgb=, white_bkgd=, want_kstats=): the network and the
+        render flavour of flow_composite in one kernel (cfn_network_fwd_composite; needs rays and z_vals) -> the dict
+        flow_composite returns, bitwise equal to network() followed by flow_composite()."""
         self.pack()
         out = torch.empty(B * N, self.PP, dtype=torch.float32, device=self.device)
         ws = self.workspace(B * N, save)
+        if composite is not None:
+            K, f32 = self.K, dict(dtype=torch.float32, device=self.device)
+            rgb, disp, depth = torch.empty(B, 3, K, **f32), torch.empty(B, K, **f32), torch.empty(B, K, **f32)
+            ks = torch.empty(B, 8, **f32) if composite.get("want_kstats") else None
+            c = composite
+            check(self.lib.cfn_network_fwd_composite(self.h, _ptr(rays), _ptr(z_vals), B, N, _ptr(out), _ptr(ws), ws.numel(),
+                                                     _ptr(c["rays_d"]), int(c["rays_d_stride"]), _ptr(c["eps_alpha"]),
+                                                     _ptr(c["eps_rgb"]), int(bool(c["white_bkgd"])), _ptr(rgb), _ptr(disp),
+                                                     _ptr(depth), _ptr(ks), _stream()), "cfn_network_fwd_composite")
+            return dict(rgb_map=rgb, disp_map=disp, depth_map=depth, raw=None, weights=None, logdet_sums=None, kstats=ks,
+                        trans=None, seg_sums=None)
         check(self.lib.cfn_network_fwd(self.h, _ptr(rays), _ptr(z_vals), _ptr(pts), _ptr(viewdirs), B, N, _ptr(out),
                                        _ptr(ws), ws.numel(), int(save), _stream()), "cfn_network_fwd")
         return (out, ws) if save else out

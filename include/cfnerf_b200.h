@@ -116,6 +116,16 @@ int cfn_network_fwd(CfnHandle* h, const float* rays, const float* z_vals, const 
                     int64_t B, int N, float* flow_params, void* workspace, size_t workspace_bytes,
                     int save_for_backward, void* stream);
 
+/* Render fast path (CFN_PREC_BF16 / CFN_PREC_FP16, n_flows = 4, N dividing 128, one latent-draw set for every ray):
+ * cfn_network_fwd from (rays, z_vals) followed by the render flavour of cfn_flow_composite_fwd (no raw / weights /
+ * log-dets), in ONE kernel whose spare warps composite each tile's rays while the network runs on the next tile.
+ * flow_params (B*N,18F) is still written (and read back by the compositing warps).  Outputs are bitwise equal to
+ * the two calls: rgb_map (B,3,K), disp_map (B,K), depth_map (B,K), kstats (B,8) optional. */
+int cfn_network_fwd_composite(CfnHandle* h, const float* rays, const float* z_vals, int64_t B, int N, float* flow_params,
+                              void* workspace, size_t workspace_bytes, const float* rays_d, int rays_d_stride,
+                              const float* eps_alpha, const float* eps_rgb, int white_bkgd, float* rgb_map,
+                              float* disp_map, float* depth_map, float* kstats, void* stream);
+
 /* Backward of cfn_network_fwd (training path).  g_flow_params (B*N,18F) is d loss / d flow_params;
  * workspace must be the one a save_for_backward forward of the same points filled.  grads[i] (device,
  * fp32, same shapes/order as the parameters; entries may be NULL to skip) are OVERWRITTEN for i >= 4
