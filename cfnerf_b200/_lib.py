@@ -48,6 +48,12 @@ SYMBOLS = {
     "cfn_sparsification_workspace_bytes": (_i32, [_i64, _i64, _i32, C.POINTER(_sz)]),
     "cfn_sparsification_f32": (_i32, [_f32p, _f32p, _f32p, _i64, _i64, _i32, _vp, _sz, _f32p, _f32p, _vp]),
     "cfn_field_stats_f32": (_i32, [_vp, _f32p, _f32p, _f32p, _i64, _f32p, _vp]),
+    "cfn_flow_composite_bwd_rays": (_i32, [_vp, _f32p, _f32p, _f32p, _i32, _f32p, _f32p, _i64, _i64, _i32, _i32, _f32p,
+                                           _f32p, _f32p, _f32p, _f32p, _i32, _f32p, _f32p, _f32p, _f32p, _vp]),
+    "cfn_input_grad_width": (_i32, [_vp]),
+    "cfn_network_bwd_inputs": (_i32, [_vp, _f32p, _i64, _i32, _vp, _sz, C.POINTER(_vp), _i32, _f32p, _vp]),
+    "cfn_ray_grad_f32": (_i32, [_vp, _f32p, _f32p, _f32p, _f32p, _i32, _f32p, _f32p, _f32p, _i64, _i32, _f32p, _vp]),
+    "cfn_rays_from_pose_bwd_f32": (_i32, [_i32, _i32, C.c_double, _f32p, _i32, C.c_double, _f32p, _f32p, _f32p, _vp]),
     "cfn_adam_step_f32":(_i32, [_i32, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_i64),
                           C.c_float, C.c_float, C.c_float, C.c_float, _i32, C.c_float, _vp]),
     "cfn_adam_step_dev_f32": (_i32, [_i32, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_i64),

@@ -141,15 +141,18 @@ def mean_over_k(w):
 class _RenderTrainFn(torch.autograd.Function):
     """forward: cfn_network_fwd(save) + cfn_flow_composite_fwd(train); backward: cfn_flow_composite_bwd +
     cfn_network_bwd.  The parameters are inputs so that autograd writes into the reference module's own .grad.
-    eps_a (G,K) / eps_c (G,K,3): one latent draw per group of `group_rays` rays (0: G = 1)."""
+    eps_a (G,K) / eps_c (G,K,3): one latent draw per group of `group_rays` rays (0: G = 1).
+    sched = (t_vals, t_rand or None, lindisp): what made z_vals from the rays.  When the rays need a gradient the
+    backward runs the ray flavour instead (cfn_flow_composite_bwd_rays + cfn_network_bwd_inputs + cfn_ray_grad_f32),
+    without any weight gradient when no parameter needs one."""
 
     @staticmethod
-    def forward(ctx, eng: Engine, rays, z_vals, eps_a, eps_c, white_bkgd, want_weights, group_rays, *params):
+    def forward(ctx, eng: Engine, rays, z_vals, eps_a, eps_c, white_bkgd, want_weights, group_rays, sched, *params):
         B, N = z_vals.shape
         fp, ws = eng.network(B, N, rays=rays, z_vals=z_vals, save=True)
         out = eng.flow_composite(fp, z_vals, rays[:, 3:6], 11, eps_a, eps_c, white_bkgd, want_raw=True,
                                  want_weights=want_weights, train=True, eps_group_rays=group_rays, want_trans=True)
-        ctx.eng, ctx.white_bkgd, ctx.group_rays = eng, white_bkgd, group_rays
+        ctx.eng, ctx.white_bkgd, ctx.group_rays, ctx.sched = eng, white_bkgd, group_rays, sched
         sg = out["seg_sums"] if out["seg_sums"] is not None else torch.empty(0, device=rays.device)
         ctx.save_for_backward(rays, z_vals, eps_a, eps_c, fp, ws, out["trans"], sg)
         w = out["weights"] if want_weights else torch.empty(0, device=rays.device)
@@ -167,16 +170,28 @@ class _RenderTrainFn(torch.autograd.Function):
         g_depth = _f32c(g_depth, dev) if g_depth is not None else None
         # the per-ray log-det gradient seeds stay on the device: reading them back would stall the host once per step
         gl = _f32c(g_ld.detach(), dev) if g_ld is not None else torch.zeros(B, 2, device=dev)
+        g_rays = None
         with torch.cuda.device(dev):
-            g_fp, g_glob = eng.flow_composite_bwd(fp, z_vals, rays[:, 3:6], 11, eps_a, eps_c, ctx.white_bkgd, g_rgb,
-                                                  g_depth, gl, trans=trans, eps_group_rays=ctx.group_rays,
-                                                  seg_sums=sg if sg.numel() else None)
-            grads = eng.network_bwd(g_fp, B, N, ws)
+            if not ctx.needs_input_grad[1]:
+                g_fp, g_glob = eng.flow_composite_bwd(fp, z_vals, rays[:, 3:6], 11, eps_a, eps_c, ctx.white_bkgd, g_rgb,
+                                                      g_depth, gl, trans=trans, eps_group_rays=ctx.group_rays,
+                                                      seg_sums=sg if sg.numel() else None)
+                grads = eng.network_bwd(g_fp, B, N, ws)
+            else:
+                g_fp, g_glob, g_zd, g_dl = eng.flow_composite_bwd(
+                    fp, z_vals, rays[:, 3:6], 11, eps_a, eps_c, ctx.white_bkgd, g_rgb, g_depth, gl, trans=trans,
+                    eps_group_rays=ctx.group_rays, seg_sums=sg if sg.numel() else None, ray_terms=True)
+                need_w = any(ctx.needs_input_grad[9:])
+                grads, g_enc = eng.network_bwd_inputs(g_fp, B, N, ws, weights=need_w)
+                t_vals, t_rand, lindisp = ctx.sched
+                g_rays = eng.ray_grad(rays, z_vals, t_vals, t_rand, lindisp, g_enc, g_zd, g_dl)
+                if not need_w:
+                    return (None, g_rays) + (None,) * (7 + len(eng.params))
         gg = g_glob.sum(0)
         grads[0], grads[1] = gg[0:1], gg[1:2]
         grads[2], grads[3] = gg[2:5], gg[5:8]
         grads = [g.reshape(p.shape) for g, p in zip(grads, eng.params)]
-        return (None, None, None, None, None, None, None, None, *grads)
+        return (None, g_rays, None, None, None, None, None, None, None, *grads)
 
 
 def latent_groups(B: int, N: int, netchunk: int):
@@ -321,8 +336,17 @@ def render_rays(ray_batch, network_fn, network_query_fn=None, N_samples=128, is_
     be passed as (K,1) / (K,3) (one call) or (G,K,1) / (G,K,3) (one pair per call)."""
     module = _unwrap(network_fn)
     dev = ray_batch.device
+    hier = N_importance > 0 and network_fine is not None
+    # F7: the rays need a gradient -> the training kernels run in test mode too (the reference's render_rays is one
+    # autograd graph from ray_batch in both modes); single-network passes only
+    ray_grad = ray_batch.requires_grad and torch.is_grad_enabled()
+    if ray_grad and hier:
+        raise ValueError("ray gradients cover single-network passes: the coarse+fine pass (N_importance > 0 with "
+                         "network_fine) is not differentiable in ray_batch")
+    if ray_grad and want_kstats:
+        raise ValueError("want_kstats is not available together with ray gradients (ray_batch.requires_grad)")
     prec = precision or DEFAULT_PRECISION
-    if is_train:
+    if is_train or ray_grad:
         prec = precision or DEFAULT_TRAIN_PRECISION
     eng = engine_for(network_fn, dev, prec)
     if K_samples and K_samples != eng.K:
@@ -331,7 +355,6 @@ def render_rays(ray_batch, network_fn, network_query_fn=None, N_samples=128, is_
     if rays.shape[-1] != 11:
         raise ValueError("ray_batch must be (B,11) = [o d near far viewdir] (use_viewdirs, main:504-507)")
     B = rays.shape[0]
-    hier = N_importance > 0 and network_fine is not None
     if B == 0 and not is_train:
         # an empty ray batch (a ragged last shard): empty maps of the right shapes, no launches
         K, f32 = eng.K, dict(dtype=torch.float32, device=dev)
@@ -354,6 +377,7 @@ def render_rays(ray_batch, network_fn, network_query_fn=None, N_samples=128, is_
         if t_rand is not None:
             t_rand = _f32c(t_rand, dev)
         z_vals = eng.zvals(rays, t_vals, t_rand if perturb > 0. or t_rand is not None else None, lindisp)
+        sched = (t_vals, t_rand, bool(lindisp))
         # latent draws: one pair per network call of the reference (train mode), the constructor-time draws in test mode
         group_rays, G = (0, 1)
         if is_train and not hier:
@@ -367,9 +391,11 @@ def render_rays(ray_batch, network_fn, network_query_fn=None, N_samples=128, is_
         def one_pass(net, z, train, need_w):
             e = engine_for(net, dev, prec)
             N = z.shape[1]
-            if train:
+            if train or ray_grad:
                 rgb, disp, depth, raw, ld, w = _RenderTrainFn.apply(e, rays, z, eps_a, eps_c, bool(white_bkgd),
-                                                                    need_w, group_rays, *e.params)
+                                                                    need_w, group_rays, sched, *e.params)
+                if not train:       # test mode with ray gradients: the maps (and weights), as the reference returns
+                    return dict(rgb_map=rgb, disp_map=disp, depth_map=depth, weights=w if need_w else None)
                 ent = _entropy_rows(_unwrap(net), eps_a, eps_c, ld, B, N, e.K, group_rays)    # models.py:286-291
                 return dict(rgb_map=rgb, disp_map=disp, depth_map=depth, raw=raw, weights=w if need_w else None,
                             loss_entropy=ent)
@@ -417,13 +443,47 @@ def render_rays(ray_batch, network_fn, network_query_fn=None, N_samples=128, is_
     return ret
 
 
+class _RaysFromPoseFn(torch.autograd.Function):
+    """rays_from_pose with a gradient for c2w: backward = cfn_rays_from_pose_bwd_f32 (c2w read on the device)."""
+
+    @staticmethod
+    def forward(ctx, c2w, H, W, focal, near, far, ndc, device):
+        ctx.save_for_backward(c2w)
+        ctx.args = (H, W, focal, ndc, device)
+        return _rays_from_pose(H, W, focal, c2w.detach(), near, far, ndc, device)
+
+    @staticmethod
+    def backward(ctx, g_rays):
+        (c2w,) = ctx.saved_tensors
+        H, W, focal, ndc, dev = ctx.args
+        lib = _lib.load()
+        c = _f32c(c2w.detach()[:3, :4], dev)
+        g = torch.empty(3, 4, dtype=torch.float32, device=dev)
+        partials = torch.empty(3072, dtype=torch.float32, device=dev)       # CFN_POSE_BWD_PARTIALS
+        with torch.cuda.device(dev):
+            check(lib.cfn_rays_from_pose_bwd_f32(int(H), int(W), float(focal), _ptr(c), int(bool(ndc)), 1.0,
+                                                 _ptr(_f32c(g_rays, dev)), _ptr(partials), _ptr(g), _stream()),
+                  "cfn_rays_from_pose_bwd_f32")
+        gc = torch.zeros(c2w.shape, dtype=c2w.dtype, device=c2w.device)
+        gc[:3, :4] = g.to(device=c2w.device, dtype=c2w.dtype)
+        return gc, None, None, None, None, None, None, None
+
+
 def rays_from_pose(H, W, focal, c2w, near=0., far=1., ndc=False, device=None):
     """The ray batch `render(H, W, focal, c2w=pose, use_viewdirs=True)` assembles (main:129-158) — (H*W,11) on the
-    device, generated by one kernel from the 3x4 pose instead of six (H,W,3) torch intermediates."""
-    lib = _lib.load()
-    c = torch.as_tensor(c2w, dtype=torch.float32).detach().cpu()[:3, :4].contiguous()
+    device, generated by one kernel from the 3x4 pose instead of six (H,W,3) torch intermediates.  When c2w is a tensor
+    that requires a gradient (and grad mode is on) the rays carry a grad_fn whose backward is the adjoint kernel, so
+    render_rays / render_image become differentiable in the pose."""
     dev = torch.device(device) if device is not None else (c2w.device if isinstance(c2w, torch.Tensor) and c2w.is_cuda
                                                            else torch.device("cuda", torch.cuda.current_device()))
+    if isinstance(c2w, torch.Tensor) and c2w.requires_grad and torch.is_grad_enabled():
+        return _RaysFromPoseFn.apply(c2w, H, W, focal, near, far, ndc, dev)
+    return _rays_from_pose(H, W, focal, c2w, near, far, ndc, dev)
+
+
+def _rays_from_pose(H, W, focal, c2w, near, far, ndc, dev):
+    lib = _lib.load()
+    c = torch.as_tensor(c2w, dtype=torch.float32).detach().cpu()[:3, :4].contiguous()
     rays = torch.empty(H * W, 11, dtype=torch.float32, device=dev)
     arr = (C.c_float * 12)(*c.reshape(-1).tolist())
     with torch.cuda.device(dev):

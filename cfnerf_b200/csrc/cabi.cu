@@ -509,6 +509,60 @@ extern "C" int cfn_field_stats_f32(const CfnHandle* h, const float* flow_params,
                             (cudaStream_t)stream);
 }
 
+extern "C" int cfn_flow_composite_bwd_rays(CfnHandle* h, const float* flow_params, const float* z_vals,
+                                           const float* rays_d, int rays_d_stride, const float* eps_alpha,
+                                           const float* eps_rgb, int64_t eps_group_rays, int64_t B, int N, int white_bkgd,
+                                           const float* g_rgb_map, const float* g_depth_map, const float* g_logdet,
+                                           const float* trans, const float* seg_sums, int n_segments, float* g_flow_params,
+                                           float* g_globals_partial, float* g_zdirect, float* g_delta, void* stream) {
+  CFN_CHECK_ARG(B >= 0 && N >= 2 && eps_group_rays >= 0, "cfn_flow_composite_bwd_rays: bad shape (B %lld, N %d)", (long long)B, N);
+  CFN_CHECK_ARG(h && flow_params && z_vals && rays_d && eps_alpha && eps_rgb && g_rgb_map && g_logdet && trans &&
+                    g_flow_params && g_globals_partial && g_zdirect && g_delta,
+                "cfn_flow_composite_bwd_rays: null argument");
+  if (!h->packed) {
+    set_error("cfn_flow_composite_bwd_rays: call cfn_pack_weights first");
+    return CFN_ESTATE;
+  }
+  return launch_flow_composite_bwd(h->cfg.precision != CFN_PREC_FP32 ? 1 : 0, h->cfg.F, h->cfg.K, h->globals, flow_params,
+                                   z_vals, rays_d, rays_d_stride, eps_alpha, eps_rgb, eps_group_rays, B, N, white_bkgd,
+                                   g_rgb_map, g_depth_map, g_logdet, trans, seg_sums, n_segments, g_flow_params,
+                                   g_globals_partial, (cudaStream_t)stream, g_zdirect, g_delta);
+}
+
+extern "C" int cfn_input_grad_width(const CfnHandle* h) { return h ? chain_input_grad_width(h) : 0; }
+
+extern "C" int cfn_network_bwd_inputs(CfnHandle* h, const float* g_flow_params, int64_t B, int N, void* workspace,
+                                      size_t workspace_bytes, float* const* grads, int n_params, float* g_enc, void* stream) {
+  CFN_CHECK_ARG(B >= 0 && N >= 1, "cfn_network_bwd_inputs: bad shape (B %lld, N %d)", (long long)B, N);
+  CFN_CHECK_ARG(h && g_flow_params && workspace && g_enc, "cfn_network_bwd_inputs: null argument");
+  CFN_CHECK_ARG(!grads || n_params == (int)h->slots.size(), "cfn_network_bwd_inputs: expected %d tensors", (int)h->slots.size());
+  size_t need = 0;
+  cfn_workspace_bytes(h, B * N, 1, &need);
+  if (workspace_bytes < need) {
+    set_error("cfn_network_bwd_inputs: workspace %zu bytes < required %zu", workspace_bytes, need);
+    return CFN_ENOMEM;
+  }
+  if (B == 0) return CFN_OK;
+  return chain_network_bwd(h, g_flow_params, B, N, (float*)workspace, grads, (cudaStream_t)stream, g_enc);
+}
+
+extern "C" int cfn_ray_grad_f32(const CfnHandle* h, const float* rays, const float* z_vals, const float* t_vals,
+                                const float* t_rand, int lindisp, const float* g_enc, const float* g_zdirect,
+                                const float* g_delta, int64_t B, int N, float* g_rays, void* stream) {
+  CFN_CHECK_ARG(B >= 0 && N >= 1, "cfn_ray_grad_f32: bad shape (B %lld, N %d)", (long long)B, N);
+  CFN_CHECK_ARG(h != nullptr, "cfn_ray_grad_f32: null handle");
+  CFN_CHECK_ARG(B == 0 || (rays && z_vals && t_vals && g_enc && g_zdirect && g_delta && g_rays), "cfn_ray_grad_f32: null argument");
+  return launch_ray_grad(rays, z_vals, t_vals, t_rand, lindisp, g_enc, chain_input_grad_width(h), h->gp, h->skip >= 0 ? 1 : 0,
+                         h->cfg.L_pos, h->cfg.L_dir, g_zdirect, g_delta, B, N, g_rays, (cudaStream_t)stream);
+}
+
+extern "C" int cfn_rays_from_pose_bwd_f32(int H, int W, double focal, const float* c2w, int ndc, double ndc_near,
+                                          const float* g_rays, float* partials, float* g_c2w, void* stream) {
+  CFN_CHECK_ARG(H > 0 && W > 0 && focal > 0 && (int64_t)H * W < (1ll << 31), "cfn_rays_from_pose_bwd_f32: bad image size");
+  CFN_CHECK_ARG(c2w && g_rays && partials && g_c2w, "cfn_rays_from_pose_bwd_f32: null argument");
+  return launch_rays_from_pose_bwd(H, W, focal, c2w, ndc, ndc_near, g_rays, partials, g_c2w, (cudaStream_t)stream);
+}
+
 extern "C" int cfn_adam_step_f32(int n_tensors, float* const* params, const float* const* grads, float* const* exp_avg,
                                  float* const* exp_avg_sq, const int64_t* numels, float lr, float beta1, float beta2,
                                  float eps, int step, float grad_scale, void* stream) {

@@ -113,6 +113,12 @@ int launch_sparsify(const float* u, const float* e, const float* a, int64_t V, i
 int launch_field_stats(int fast_math, int F, int K, const float* globals, const float* flow_params, const float* eps_alpha,
                        const float* eps_rgb, int64_t M, float* out, cudaStream_t s);
 
+int launch_ray_grad(const float* rays, const float* z_vals, const float* t_vals, const float* t_rand, int lindisp,
+                    const float* g_enc, int ld_enc, int gp, int has_skip, int L_pos, int L_dir, const float* g_zdirect,
+                    const float* g_delta, int64_t B, int N, float* g_rays, cudaStream_t s);
+int launch_rays_from_pose_bwd(int H, int W, double focal, const float* c2w, int ndc, double ndc_near, const float* g_rays,
+                              float* partials, float* g_c2w, cudaStream_t s);
+
 int launch_flow_composite_fwd(int fast_math, int F, int K, const float* globals, const float* flow_params, const float* z_vals,
                               const float* rays_d, int rays_d_stride, const float* eps_alpha, const float* eps_rgb,
                               int64_t eps_group_rays, int64_t B, int N, int white_bkgd, float* rgb_map, float* disp_map,
@@ -122,7 +128,8 @@ int launch_flow_composite_bwd(int fast_math, int F, int K, const float* globals,
                               const float* rays_d, int rays_d_stride, const float* eps_alpha, const float* eps_rgb,
                               int64_t eps_group_rays, int64_t B, int N, int white_bkgd, const float* g_rgb_map,
                               const float* g_depth_map, const float* g_ld, const float* trans, const float* seg_sums,
-                              int n_seg, float* g_flow_params, float* g_globals, cudaStream_t s);
+                              int n_seg, float* g_flow_params, float* g_globals, cudaStream_t s,
+                              float* g_zdirect = nullptr, float* g_delta = nullptr);   // both or neither: ray flavour
 
 // C[m,n] = epi( sum_k A(m,k) * B(k,n) + bias[n] ) with arbitrary element strides (fp32 CUDA-core GEMM).
 enum Epilogue { EPI_NONE = 0, EPI_RELU = 1, EPI_TANH_MASK = 2, EPI_RELU_MASK_MUL = 3 };

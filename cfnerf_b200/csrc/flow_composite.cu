@@ -543,7 +543,12 @@ __device__ __forceinline__ void reduce_rows_over_lanes(const float (&v)[NV], flo
   }
 }
 
-template <int FT, bool FAST>
+// RAYGRAD (ray-gradient flavour, cfn_flow_composite_bwd_rays): also writes, per (ray, sample), the two sums over k that
+// the ray-input gradient needs (cfn_ray_grad_f32): g_zdirect = sum_k gD_k w_k (the depth map's direct z term) and
+// g_delta = sum_k dL/d delta_k = sum_k g_alpha_k (1 - alpha_k) softplus(raw sigma_k).  Both are reduced over the 32 lanes
+// by a fixed xor butterfly and summed over the latent groups in order; each warp writes only its own samples.  The
+// RAYGRAD = false instantiations are the plain K4 kernels.
+template <int FT, bool FAST, bool RAYGRAD = false>
 __global__ void __launch_bounds__(128, 4)
 flow_composite_bwd_kernel(int K, const float* __restrict__ globals, const float* __restrict__ flow_params,
                           const float* __restrict__ z_vals, const float* __restrict__ rays_d, int rays_d_stride,
@@ -552,7 +557,8 @@ flow_composite_bwd_kernel(int K, const float* __restrict__ globals, const float*
                           const float* __restrict__ g_depth_map, const float* __restrict__ g_ld,
                           const float* __restrict__ trans,
                           const float* __restrict__ seg_sums, int n_seg,
-                          float* __restrict__ g_flow_params, float* __restrict__ g_globals_partial) {
+                          float* __restrict__ g_flow_params, float* __restrict__ g_globals_partial,
+                          float* __restrict__ g_zdirect = nullptr, float* __restrict__ g_delta = nullptr) {
   constexpr int F = FT;
   constexpr int PP = 18 * F;
   constexpr int PB = kBwdPB;
@@ -697,6 +703,20 @@ flow_composite_bwd_kernel(int K, const float* __restrict__ globals, const float*
           S += v * w;
           // d alpha / d raw_sigma = (1-alpha) * delta * sigmoid(raw_sigma);  entropy activation term (models.py:263)
           float g_za = g_alpha * (1.0f - alpha) * sd[n] * sig_za + gl_a * (1.0f - sig_za);
+          if constexpr (RAYGRAD) {
+            // d alpha / d delta = (1 - alpha) * softplus(raw_sigma); inactive lanes contribute exact zeros
+            float rz = active ? gD * w : 0.f;
+            float rd = active ? g_alpha * (1.0f - alpha) * softplus_<FAST>(za) : 0.f;
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+              rz += __shfl_xor_sync(0xffffffffu, rz, o);
+              rd += __shfl_xor_sync(0xffffffffu, rd, o);
+            }
+            if (lane == 0) {
+              if (kg == 0) { g_zdirect[b * N + n] = rz; g_delta[b * N + n] = rd; }
+              else { g_zdirect[b * N + n] += rz; g_delta[b * N + n] += rd; }
+            }
+          }
           float gz[3];
 #pragma unroll
           for (int cc = 0; cc < 3; ++cc)
@@ -797,7 +817,8 @@ int launch_flow_composite_bwd(int fast_math, int F, int K, const float* globals,
                               const float* rays_d, int rays_d_stride, const float* eps_alpha, const float* eps_rgb,
                               int64_t eps_group_rays, int64_t B, int N, int white_bkgd, const float* g_rgb_map,
                               const float* g_depth_map, const float* g_ld, const float* trans, const float* seg_sums,
-                              int n_seg, float* g_flow_params, float* g_globals_partial, cudaStream_t s) {
+                              int n_seg, float* g_flow_params, float* g_globals_partial, cudaStream_t s,
+                              float* g_zdirect, float* g_delta) {
   if (B == 0) return CFN_OK;
   if (!seg_sums || n_seg < 1) n_seg = 1;
   CFN_CHECK_ARG(N % n_seg == 0 && (N / n_seg) >= 1, "flow_composite_bwd: N=%d is not a multiple of n_segments=%d", N, n_seg);
@@ -808,11 +829,12 @@ int launch_flow_composite_bwd(int fast_math, int F, int K, const float* globals,
   unsigned grid = (unsigned)((B * n_seg + 3) / 4);
 #define CFN_BWD_CASE(FF)                                                                                             \
   case FF: {                                                                                                         \
-    auto kern = fast_math ? flow_composite_bwd_kernel<FF, true> : flow_composite_bwd_kernel<FF, false>;              \
+    auto kern = g_zdirect ? (fast_math ? flow_composite_bwd_kernel<FF, true, true> : flow_composite_bwd_kernel<FF, false, true>) \
+                          : (fast_math ? flow_composite_bwd_kernel<FF, true> : flow_composite_bwd_kernel<FF, false>);  \
     if (smem > 48 * 1024) CFN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
     kern<<<grid, 128, smem, s>>>(K, globals, flow_params, z_vals, rays_d, rays_d_stride, eps_alpha, eps_rgb,         \
                                  eps_group_rays, B, N, white_bkgd, g_rgb_map, g_depth_map, g_ld, trans, seg_sums,    \
-                                 n_seg, g_flow_params, g_globals_partial);                                           \
+                                 n_seg, g_flow_params, g_globals_partial, g_zdirect, g_delta);                       \
   } break;
   switch (F) {
     CFN_BWD_CASE(1) CFN_BWD_CASE(2) CFN_BWD_CASE(3) CFN_BWD_CASE(4) CFN_BWD_CASE(5) CFN_BWD_CASE(6) CFN_BWD_CASE(7)

@@ -588,7 +588,7 @@ bool tgemm_supported(const GemmArgs& g) {
     // bf16 storage: exactly the flavours of the training chain
     if (g.accumulate) return false;
     if (!a_mn_ && !b_mn_) return (plain && g.c_bf16) || (g.epilogue == EPI_RELU && g.c_bf16 && !atomic) || (g.epilogue == EPI_TANH_MASK && !g.c_bf16 && !atomic);
-    if (!a_mn_ && b_mn_) return g.c_bf16 && (plain || (mask && g.aux_bits != nullptr));
+    if (!a_mn_ && b_mn_) return plain || (g.c_bf16 && mask && g.aux_bits != nullptr);   // fp32 C: the input dgrads
     if (a_mn_ && b_mn_) return atomic && !g.c_bf16;
     return false;
   }
@@ -701,6 +701,7 @@ int launch_tgemm(const GemmArgs& g, int round_out, cudaStream_t s) {
     if (!a_mn && !b_mn && epi == TG_RELU && g.c_bf16) TG_BF(false, false, TG_RELU, true);
     if (!a_mn && !b_mn && epi == TG_TANH && !g.c_bf16) TG_BF(false, false, TG_TANH, false);
     if (!a_mn && b_mn && epi == TG_PLAIN && g.c_bf16) TG_BF(false, true, TG_PLAIN, true);
+    if (!a_mn && b_mn && epi == TG_PLAIN && !g.c_bf16) TG_BF(false, true, TG_PLAIN, false);
     if (!a_mn && b_mn && epi == TG_MASK && g.c_bf16) TG_BF(false, true, TG_MASK, true);
     if (a_mn && b_mn && epi == TG_ATOMIC && !g.c_bf16) TG_BF(true, true, TG_ATOMIC, false);
   } else if (!a_mn && !b_mn) {

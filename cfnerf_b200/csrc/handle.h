@@ -77,7 +77,8 @@ size_t chain_workspace_floats(const CfnHandle* h, int64_t n_points, int save);
 int chain_network_fwd(CfnHandle* h, const float* rays, const float* z_vals, const float* pts, const float* viewdirs,
                      int64_t B, int N, float* flow_params, float* ws, int save, cudaStream_t s);
 int chain_network_bwd(const CfnHandle* h, const float* g_flow_params, int64_t B, int N, float* ws, float* const* grads,
-                      cudaStream_t s);
+                      cudaStream_t s, float* g_enc = nullptr);
+int chain_input_grad_width(const CfnHandle* h);   // columns of chain_network_bwd's g_enc rows: 2 gp + gd
 int64_t chain_det_scratch_floats(const CfnHandle* h);   // deterministic split-K scratch of chain_network_bwd
 int pack_fp32(CfnHandle* h, const float* const* params, cudaStream_t s);
 

@@ -500,10 +500,11 @@ static int wgrad_slot(const CfnHandle* h, int slot, const float* G, int64_t ldg,
   return CFN_OK;
 }
 
-// Gin(M x n_cols) = [accumulate +] Gout(M x out) W[:, col0:col0+n_cols], optional ReLU mask
+// Gin(M x n_cols) = [accumulate +] Gout(M x out) W[:, col0:col0+n_cols], optional ReLU mask.  out_f32: Gin is fp32
+// and is not rounded to the tf32 grid whatever the chain's storage (it is no later GEMM's operand: the input gradients)
 static int dgrad(const CfnHandle* h, int slot, const float* Gout, int64_t ldgo, int col0, int n_cols, float* Gin,
                  int64_t ldgi, int64_t M, const float* mask, int64_t ld_mask, int accumulate, cudaStream_t s,
-                 const uint32_t* mask_bits = nullptr, int bits_ld = 0) {
+                 const uint32_t* mask_bits = nullptr, int bits_ld = 0, bool out_f32 = false) {
   const ParamSlot& w = h->slots[slot];
   const WView& v = h->wv[slot];
   GemmArgs g{};
@@ -513,10 +514,11 @@ static int dgrad(const CfnHandle* h, int slot, const float* Gout, int64_t ldgo, 
   g.aux = mask; g.aux_rs = ld_mask;
   g.aux_bits = mask ? mask_bits : nullptr; g.bits_ld = bits_ld;
   g.ab_bf16 = g.c_bf16 = h->chain_bf16;
+  if (out_f32) g.c_bf16 = 0;
   g.M = M; g.N = n_cols; g.K = w.rows;
   g.epilogue = mask ? EPI_RELU_MASK_MUL : EPI_NONE;
   g.accumulate = accumulate; g.split_k = 1;
-  return gemm(h, g, 1, s);
+  return gemm(h, g, out_f32 ? 0 : 1, s);
 }
 
 // gradient tensors by parameter slot, passed BY VALUE as a kernel parameter: copying the table to the device from pageable
@@ -534,15 +536,24 @@ __global__ void scatter_rows_kernel(const float* __restrict__ dAm, const float* 
   if (gb && threadIdx.x == 0) gb[row] = dAb[r];
 }
 
+int chain_input_grad_width(const CfnHandle* h) { return 2 * h->gp + h->gd; }
+
+// grads == nullptr: no weight gradient at all (no wgrad, no scatter, no memset: a frozen network).  g_enc (M x
+// chain_input_grad_width, fp32): when given, also the gradients of the encoded inputs, [g_gamma(p) through layer 0 |
+// g_gamma(p) through the skip layer (zeros without one) | g_gamma(d) through the view layer], each block padded to gp /
+// gp / gd columns (the pad columns meet zero weights and come out 0).
 int chain_network_bwd(const CfnHandle* h, const float* g_flow_params, int64_t B, int N, float* ws, float* const* grads,
-                      cudaStream_t s) {
+                      cudaStream_t s, float* g_enc) {
   const int64_t M = B * N;
   const int W = h->cfg.W, D = h->cfg.D, F = h->cfg.F, PP = h->PP;
   const int ha_n = h->cfg.h_alpha, hr_n = h->cfg.h_rgb;
   ChainLayout L = make_layout(h, M, 1);
   int rc;
-  for (int i = 4; i < (int)h->slots.size(); ++i)
-    CFN_CHECK_ARG(grads[i] != nullptr, "cfn_network_bwd: grads[%d] (%s) is null", i, h->slots[i].name.c_str());
+  const bool want_w = grads != nullptr;
+  const int ld_enc = chain_input_grad_width(h);
+  if (want_w)
+    for (int i = 4; i < (int)h->slots.size(); ++i)
+      CFN_CHECK_ARG(grads[i] != nullptr, "cfn_network_bwd: grads[%d] (%s) is null", i, h->slots[i].name.c_str());
   float* dAm = ws + L.dAm;                       // (rows, cols) gathered weight grads
   float* dAb = dAm + (int64_t)PP * (ha_n > hr_n ? ha_n : hr_n);   // (rows) gathered bias grads
 
@@ -580,7 +591,7 @@ int chain_network_bwd(const CfnHandle* h, const float* g_flow_params, int64_t B,
   // Gradient tensors laid out back to back in slot order (cfnerf_b200.dist.FusedTrainStep's flat bucket): ONE memset
   // replaces the ~40 per-tensor ones of the split-K wgrads (each a graph node / launch of its own at 512 rays per step)
   Zeroed zeroed;
-  {
+  if (want_w) {
     bool flat = true;
     for (size_t i = 5; i < h->slots.size(); ++i)
       flat = flat && (grads[i] == grads[4] + (h->slots[i].offset - h->slots[4].offset));
@@ -592,21 +603,23 @@ int chain_network_bwd(const CfnHandle* h, const float* g_flow_params, int64_t B,
     }
   }
   // zero every flow-conditioning gradient: rows the path never reads keep an exact 0 (SURVEY §0 fact 5)
-  if (!zeroed.lo)
+  if (want_w && !zeroed.lo)
     for (int base : {h->s_frgb, h->s_falpha})
       for (int j = 0; j < 8; ++j)
         CFN_CUDA(cudaMemsetAsync(grads[base + j], 0, h->slots[base + j].numel * sizeof(float), s));
 
   // gradient pointers of every slot, handed to the scatter kernels by value
   GradPtrs table;
-  for (size_t i = 0; i < 64; ++i) table.p[i] = i < h->slots.size() ? grads[i] : nullptr;
+  for (size_t i = 0; i < 64; ++i) table.p[i] = (want_w && i < h->slots.size()) ? grads[i] : nullptr;
 
   // 2. alpha conditioning branch
   {
     // gathered dAmA = GP[:, :3F]^T ha ; bias = colsum
-    if ((rc = wgrad(h, GPa, ldGP, 3 * F, ws + L.ha, ha_n, ha_n, M, dAm, dAb, zeroed, s))) return rc;
-    scatter_rows_kernel<<<3 * F, 64, 0, s>>>(dAm, dAb, ha_n, h->gatherA_dev, 3 * F, table);
-    CFN_LAUNCH_CHECK();
+    if (want_w) {
+      if ((rc = wgrad(h, GPa, ldGP, 3 * F, ws + L.ha, ha_n, ha_n, M, dAm, dAb, zeroed, s))) return rc;
+      scatter_rows_kernel<<<3 * F, 64, 0, s>>>(dAm, dAb, ha_n, h->gatherA_dev, 3 * F, table);
+      CFN_LAUNCH_CHECK();
+    }
     // g_ha = GP[:, :3F] amA
     GemmArgs g{};
     g.A = GPa; g.a_rs = ldGP; g.a_cs = 1;
@@ -614,28 +627,32 @@ int chain_network_bwd(const CfnHandle* h, const float* g_flow_params, int64_t B,
     g.C = gha; g.c_rs = ld_gha; g.M = M; g.N = ha_n; g.K = 3 * F; g.split_k = 1;
     g.ab_bf16 = g.c_bf16 = h->chain_bf16;
     if ((rc = gemm(h, g, 1, s))) return rc;
-    if ((rc = wgrad_slot(h, h->s_halpha, gha, ld_gha, h7, ld7, M, grads[h->s_halpha], grads[h->s_halpha + 1], dWp, zeroed, s))) return rc;
+    if (want_w && (rc = wgrad_slot(h, h->s_halpha, gha, ld_gha, h7, ld7, M, grads[h->s_halpha], grads[h->s_halpha + 1], dWp, zeroed, s))) return rc;
     // g_h7 (unmasked, first contribution) = g_ha W_halpha  -- or, fused, left for the K-concatenated GEMM of step 3
     if (!fuse_heads && (rc = dgrad(h, h->s_halpha, gha, ld_gha, 0, W, G1, W, M, nullptr, 0, 0, s))) return rc;
   }
   // 3. rgb conditioning branch
   {
-    if ((rc = wgrad(h, GPc, ldGP, 15 * F, ws + L.hr, hr_n, hr_n, M, dAm, dAb, zeroed, s))) return rc;
-    scatter_rows_kernel<<<15 * F, 64, 0, s>>>(dAm, dAb, hr_n, h->gatherC_dev, 15 * F, table);
-    CFN_LAUNCH_CHECK();
+    if (want_w) {
+      if ((rc = wgrad(h, GPc, ldGP, 15 * F, ws + L.hr, hr_n, hr_n, M, dAm, dAb, zeroed, s))) return rc;
+      scatter_rows_kernel<<<15 * F, 64, 0, s>>>(dAm, dAb, hr_n, h->gatherC_dev, 15 * F, table);
+      CFN_LAUNCH_CHECK();
+    }
     GemmArgs g{};
     g.A = GPc; g.a_rs = ldGP; g.a_cs = 1;
     g.B = h->amC_g; g.b_rs = hr_n; g.b_cs = 1;
     g.C = gh; g.c_rs = hr_n; g.M = M; g.N = hr_n; g.K = 15 * F; g.split_k = 1;
     g.ab_bf16 = g.c_bf16 = h->chain_bf16;
     if ((rc = gemm(h, g, 1, s))) return rc;
-    if ((rc = wgrad_slot(h, h->s_hrgb, gh, hr_n, ws + L.v, W / 2, M, grads[h->s_hrgb], grads[h->s_hrgb + 1], dWp, zeroed, s))) return rc;
+    if (want_w && (rc = wgrad_slot(h, h->s_hrgb, gh, hr_n, ws + L.v, W / 2, M, grads[h->s_hrgb], grads[h->s_hrgb + 1], dWp, zeroed, s))) return rc;
     // g_v = (g_hr W_hrgb) * relu'(v)
     if ((rc = dgrad(h, h->s_hrgb, gh, hr_n, 0, W / 2, gv, W / 2, M, ws + L.v, W / 2, 0, s, mbv, L.bwv))) return rc;
-    if ((rc = wgrad_slot(h, h->s_views, gv, W / 2, ws + L.V, L.ldv, M, grads[h->s_views], grads[h->s_views + 1], dWp, zeroed, s))) return rc;
-    // g_feat = g_v W_view[:, :W]   (gamma(d) columns need no gradient)
+    if (want_w && (rc = wgrad_slot(h, h->s_views, gv, W / 2, ws + L.V, L.ldv, M, grads[h->s_views], grads[h->s_views + 1], dWp, zeroed, s))) return rc;
+    // g_gamma(d) = g_v W_view[:, W:W+in_dir], only when the input gradients are asked for
+    if (g_enc && (rc = dgrad(h, h->s_views, gv, W / 2, W, h->gd, g_enc + 2 * h->gp, ld_enc, M, nullptr, 0, 0, s, nullptr, 0, true))) return rc;
+    // g_feat = g_v W_view[:, :W]
     if ((rc = dgrad(h, h->s_views, gv, W / 2, 0, W, G2, ld_g2, M, nullptr, 0, 0, s))) return rc;
-    if ((rc = wgrad_slot(h, h->s_feat, G2, ld_g2, h7, ld7, M, grads[h->s_feat], grads[h->s_feat + 1], dWp, zeroed, s))) return rc;
+    if (want_w && (rc = wgrad_slot(h, h->s_feat, G2, ld_g2, h7, ld7, M, grads[h->s_feat], grads[h->s_feat + 1], dWp, zeroed, s))) return rc;
     if (fuse_heads) {
       // g_h7 = ([g_feat | g_ha] [W_feat ; W_halpha]) * relu'(h7): one GEMM over the concatenated K instead of a second,
       // accumulating one (its read-modify-write of g_h7 cost three times a plain dgrad)
@@ -659,7 +676,12 @@ int chain_network_bwd(const CfnHandle* h, const float* g_flow_params, int64_t B,
   for (int i = D - 1; i >= 0; --i) {
     LayerIO io = trunk_io(h, L, ws, M, i, 1);
     const int slot = h->s_pts(i, 0);
-    if ((rc = wgrad_slot(h, slot, gout, W, io.in, io.ld_in, M, grads[slot], grads[slot + 1], dWp, zeroed, s))) return rc;
+    if (want_w && (rc = wgrad_slot(h, slot, gout, W, io.in, io.ld_in, M, grads[slot], grads[slot + 1], dWp, zeroed, s))) return rc;
+    if (g_enc && (i == 0 || (h->skip >= 0 && i == h->skip + 1))) {
+      // g_gamma(p) = dY_i W_i[:, 0:in_pos] (+ gap / pad columns, zero weights): layer 0, and the skip layer whose input is
+      // cat[gamma(p), h]; separate column blocks (the bf16 chain has no accumulating GEMM), added by the ray kernel
+      if ((rc = dgrad(h, slot, gout, W, 0, h->gp, g_enc + (i == 0 ? 0 : h->gp), ld_enc, M, nullptr, 0, 0, s, nullptr, 0, true))) return rc;
+    }
     if (i == 0) break;
     // gradient w.r.t. the previous layer's (post-ReLU) output, masked by its ReLU
     LayerIO prev = trunk_io(h, L, ws, M, i - 1, 1);
@@ -667,6 +689,8 @@ int chain_network_bwd(const CfnHandle* h, const float* g_flow_params, int64_t B,
     if ((rc = dgrad(h, slot, gout, W, col0, W, gin, W, M, prev.out, prev.ld_out, 0, s, MBl(i - 1), L.bw))) return rc;
     float* t = gout; gout = gin; gin = t;
   }
+  if (g_enc && h->skip < 0)
+    CFN_CUDA(cudaMemset2DAsync(g_enc + h->gp, (size_t)ld_enc * 4, 0, (size_t)h->gp * 4, (size_t)M, s));
   return CFN_OK;
 }
 

@@ -107,6 +107,104 @@ int launch_rays_from_pose(int H, int W, double focal, const float* c2w12, double
   return CFN_OK;
 }
 
+// F7: the adjoint of rays_from_pose_kernel.  g_rays (H*W,11) -> g_c2w (3,4) through o = t, d = R dir_cam, the viewdir
+// normalisation (taken before the warp) and, with ndc, the NDC warp (helpers:360-377); near / far are constants.  Every
+// thread walks a fixed set of pixels, each block joins its 256 threads' 12 sums by a fixed tree, and one final block adds
+// the kPoseBwdBlocks partials in order: the result is bitwise repeatable.  c2w is read from device memory.
+constexpr int kPoseBwdBlocks = CFN_POSE_BWD_PARTIALS / 12;
+
+__global__ void __launch_bounds__(256)
+rays_from_pose_bwd_kernel(int H, int W, float focal, const float* __restrict__ c2w, int ndc, float ndc_near, float sW,
+                          float sH, float two_near, const float* __restrict__ g_rays, float* __restrict__ partials) {
+  __shared__ float red[12][256];
+  float m[12];
+#pragma unroll
+  for (int i = 0; i < 12; ++i) m[i] = c2w[i];
+  float acc[12];
+#pragma unroll
+  for (int i = 0; i < 12; ++i) acc[i] = 0.f;
+  const int n = H * W;
+  for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < n; p += gridDim.x * blockDim.x) {
+    const int row = p / W, col = p - row * W;
+    const float dir[3] = {__fdiv_rn(__fsub_rn((float)col, (float)W * 0.5f), focal),
+                          -__fdiv_rn(__fsub_rn((float)row, (float)H * 0.5f), focal), -1.0f};
+    float dx[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k)
+      dx[k] = __fadd_rn(__fadd_rn(__fmul_rn(dir[0], m[4 * k + 0]), __fmul_rn(dir[1], m[4 * k + 1])), __fmul_rn(dir[2], m[4 * k + 2]));
+    const float* g = g_rays + (int64_t)p * 11;
+    float go[3] = {g[0], g[1], g[2]}, gd[3] = {g[3], g[4], g[5]};
+    // viewdir v = d / |d|:  g_d += (g_v - v (v . g_v)) / |d|
+    const float nrm = sqrtf(dx[0] * dx[0] + dx[1] * dx[1] + dx[2] * dx[2]);
+    const float v[3] = {dx[0] / nrm, dx[1] / nrm, dx[2] / nrm};
+    const float vg = v[0] * g[8] + v[1] * g[9] + v[2] * g[10];
+    float gdx[3], gt[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) gdx[k] = (g[8 + k] - v[k] * vg) / nrm;
+    if (ndc) {
+      // forward: tt = -(near + t_z) / d_z, q = t + tt d, o' = (sW q0/q2, sH q1/q2, 1 + 2n/q2),
+      //          d' = (sW (d0/d2 - q0/q2), sH (d1/d2 - q1/q2), -2n/q2)
+      const float tt = -(ndc_near + m[11]) / dx[2];
+      const float q[3] = {m[3] + tt * dx[0], m[7] + tt * dx[1], m[11] + tt * dx[2]};
+      const float iq2 = 1.0f / q[2], iq22 = iq2 * iq2, id2 = 1.0f / dx[2];
+      float gq[3];
+      gq[0] = (go[0] - gd[0]) * sW * iq2;
+      gq[1] = (go[1] - gd[1]) * sH * iq2;
+      gq[2] = ((gd[0] - go[0]) * sW * q[0] + (gd[1] - go[1]) * sH * q[1] + (gd[2] - go[2]) * two_near) * iq22;
+      float gdd[3];
+      gdd[0] = gd[0] * sW * id2;
+      gdd[1] = gd[1] * sH * id2;
+      gdd[2] = -(gd[0] * sW * dx[0] + gd[1] * sH * dx[1]) * id2 * id2;
+      const float gtt = gq[0] * dx[0] + gq[1] * dx[1] + gq[2] * dx[2];
+#pragma unroll
+      for (int k = 0; k < 3; ++k) { gt[k] = gq[k]; gdx[k] += gdd[k] + gq[k] * tt; }
+      // tt = -(near + t_z) / d_z
+      gt[2] += -gtt * id2;
+      gdx[2] += -gtt * tt * id2;
+    } else {
+#pragma unroll
+      for (int k = 0; k < 3; ++k) { gt[k] = go[k]; gdx[k] += gd[k]; }
+    }
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+#pragma unroll
+      for (int c = 0; c < 3; ++c) acc[4 * k + c] += gdx[k] * dir[c];
+      acc[4 * k + 3] += gt[k];
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < 12; ++i) red[i][threadIdx.x] = acc[i];
+  __syncthreads();
+  for (int w = 128; w > 0; w >>= 1) {
+    if (threadIdx.x < w)
+#pragma unroll
+      for (int i = 0; i < 12; ++i) red[i][threadIdx.x] += red[i][threadIdx.x + w];
+    __syncthreads();
+  }
+  if (threadIdx.x < 12) partials[blockIdx.x * 12 + threadIdx.x] = red[threadIdx.x][0];
+}
+
+__global__ void pose_bwd_finish_kernel(const float* __restrict__ partials, int n_blocks, float* __restrict__ g_c2w) {
+  const int i = threadIdx.x;
+  if (i >= 12) return;
+  float s = 0.f;
+  for (int b = 0; b < n_blocks; ++b) s += partials[b * 12 + i];
+  g_c2w[i] = s;
+}
+
+int launch_rays_from_pose_bwd(int H, int W, double focal, const float* c2w, int ndc, double ndc_near, const float* g_rays,
+                              float* partials, float* g_c2w, cudaStream_t s) {
+  CFN_CHECK_ARG(H > 0 && W > 0 && focal > 0 && (int64_t)H * W < (1ll << 31), "rays_from_pose_bwd: bad image size");
+  const float sW = (float)(-1.0 / ((double)W / (2.0 * focal))), sH = (float)(-1.0 / ((double)H / (2.0 * focal)));
+  const float two_near = (float)(2.0 * ndc_near);
+  rays_from_pose_bwd_kernel<<<kPoseBwdBlocks, 256, 0, s>>>(H, W, (float)focal, c2w, ndc, (float)ndc_near, sW, sH, two_near,
+                                                          g_rays, partials);
+  CFN_LAUNCH_CHECK();
+  pose_bwd_finish_kernel<<<1, 32, 0, s>>>(partials, kPoseBwdBlocks, g_c2w);
+  CFN_LAUNCH_CHECK();
+  return CFN_OK;
+}
+
 // ------------------------------------------------------------------------------------------------
 // A8: raw2outputs (run_nerf_uncertainty_NF.py:411-454).  raw (B,N,K,4) is streamed exactly once:
 // one warp owns (ray, group of 32 latent samples); lane k walks the N samples front to back carrying the

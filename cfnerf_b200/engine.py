@@ -189,14 +189,23 @@ class Engine:
         return out
 
     def flow_composite_bwd(self,flow_params, z_vals, rays_d, rays_d_stride, eps_alpha, eps_rgb, white_bkgd,
-                           g_rgb, g_depth, g_ld, *, trans, eps_group_rays: int = 0, seg_sums=None):
+                           g_rgb, g_depth, g_ld, *, trans, eps_group_rays: int = 0, seg_sums=None, ray_terms=False):
         """g_ld: device tensor (B,2) = d loss / d (per-ray sums of the alpha / rgb log-dets); stays on the device (no
         host sync).  trans / seg_sums: what the training forward (flow_composite(..., want_trans=True)) wrote.
-        -> g_flow_params (B*N,18F), g_globals_partial (B*S,8) (sum the rows)."""
+        -> g_flow_params (B*N,18F), g_globals_partial (B*S,8) (sum the rows); with ray_terms also g_zdirect (B,N) and
+        g_delta (B,N), the per-sample sums the ray gradient needs (cfn_flow_composite_bwd_rays)."""
         B, N = z_vals.shape
         S = seg_sums.shape[1] if seg_sums is not None else 1
         g_fp = torch.empty_like(flow_params)
         g_glob = torch.empty(B * S, 8, dtype=torch.float32, device=self.device)
+        if ray_terms:
+            g_zd = torch.empty(B, N, dtype=torch.float32, device=self.device)
+            g_dl = torch.empty(B, N, dtype=torch.float32, device=self.device)
+            check(self.lib.cfn_flow_composite_bwd_rays(
+                self.h, _ptr(flow_params), _ptr(z_vals), _ptr(rays_d), rays_d_stride, _ptr(eps_alpha), _ptr(eps_rgb),
+                int(eps_group_rays), B, N, int(white_bkgd), _ptr(g_rgb), _ptr(g_depth), _ptr(g_ld), _ptr(trans),
+                _ptr(seg_sums), S, _ptr(g_fp), _ptr(g_glob), _ptr(g_zd), _ptr(g_dl), _stream()), "cfn_flow_composite_bwd_rays")
+            return g_fp, g_glob, g_zd, g_dl
         check(self.lib.cfn_flow_composite_bwd(self.h, _ptr(flow_params), _ptr(z_vals), _ptr(rays_d), rays_d_stride,
                                               _ptr(eps_alpha), _ptr(eps_rgb), int(eps_group_rays), B, N, int(white_bkgd),
                                               _ptr(g_rgb), _ptr(g_depth), _ptr(g_ld), _ptr(trans), _ptr(seg_sums), S,
@@ -214,6 +223,29 @@ class Engine:
         check(self.lib.cfn_network_bwd(self.h, _ptr(g_flow_params), B, N, _ptr(ws), ws.numel(), arr, len(grads),
                                        _stream()), "cfn_network_bwd")
         return grads
+
+
+    def network_bwd_inputs(self, g_flow_params, B: int, N: int, ws, weights: bool = True):
+        """network_bwd that also returns g_enc (B*N, cfn_input_grad_width): the gradients of the encoded inputs
+        (cfn_network_bwd_inputs).  weights=False: a frozen network, no weight gradient is computed -> (None, g_enc)."""
+        g_enc = torch.empty(B * N, self.lib.cfn_input_grad_width(self.h), dtype=torch.float32, device=self.device)
+        grads, arr = None, None
+        if weights:
+            grads = [None] * 4 + [torch.empty_like(p, dtype=torch.float32, memory_format=torch.contiguous_format)
+                                  for p in self.params[4:]]
+            arr = (C.c_void_p * len(grads))(*[(g.data_ptr() if (g is not None and i >= 4) else 0) for i, g in enumerate(grads)])
+        check(self.lib.cfn_network_bwd_inputs(self.h, _ptr(g_flow_params), B, N, _ptr(ws), ws.numel(), arr, len(self.params),
+                                              _ptr(g_enc), _stream()), "cfn_network_bwd_inputs")
+        return grads, g_enc
+
+    def ray_grad(self, rays, z_vals, t_vals, t_rand, lindisp: bool, g_enc, g_zdirect, g_delta):
+        """-> g_rays (B,11) = d loss / d [o d near far viewdir] (cfn_ray_grad_f32)."""
+        B, N = z_vals.shape
+        out = torch.empty(B, 11, dtype=torch.float32, device=self.device)
+        check(self.lib.cfn_ray_grad_f32(self.h, _ptr(rays), _ptr(z_vals), _ptr(t_vals), _ptr(t_rand), int(bool(lindisp)),
+                                        _ptr(g_enc), _ptr(g_zdirect), _ptr(g_delta), B, N, _ptr(out), _stream()),
+              "cfn_ray_grad_f32")
+        return out
 
 
 _ENGINES: "weakref.WeakKeyDictionary" = weakref.WeakKeyDictionary()

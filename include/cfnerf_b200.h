@@ -233,6 +233,50 @@ int cfn_sparsification_f32(const float* uncertainty, const float* sq_err, const 
 int cfn_field_stats_f32(const CfnHandle* h, const float* flow_params, const float* eps_alpha, const float* eps_rgb,
                         int64_t M, float* out, void* stream);
 
+/* ---- F7: gradients with respect to the rays and the camera pose (INTEGRATION.md §2) -------------------------------- */
+/* Added without a cfn_version() change: callers detect the feature by the presence of these symbols.  Every entry
+ * point checks its arguments before any CUDA call.  The calls chain to d loss / d ray_batch for one single-network
+ * training-path pass (cfn_network_fwd with save_for_backward + the training flavour of cfn_flow_composite_fwd):
+ *   cfn_flow_composite_bwd_rays -> cfn_network_bwd_inputs -> cfn_ray_grad_f32 [-> cfn_rays_from_pose_bwd_f32].
+ *
+ * cfn_flow_composite_bwd with the same arguments and results, plus two per-sample sums over k (written, not added):
+ * g_zdirect (B,N) = sum_k d loss/d depth_map[b,k] * weights[b,n,k] (the depth map's direct z term) and g_delta (B,N) =
+ * sum_k d loss / d delta[b,n,k] with delta = dist * |d| the sample distance of raw2outputs (main:427-429).  Both REQUIRED. */
+int cfn_flow_composite_bwd_rays(CfnHandle* h, const float* flow_params, const float* z_vals, const float* rays_d,
+                                int rays_d_stride, const float* eps_alpha, const float* eps_rgb, int64_t eps_group_rays,
+                                int64_t B, int N, int white_bkgd, const float* g_rgb_map, const float* g_depth_map,
+                                const float* g_logdet, const float* trans, const float* seg_sums, int n_segments,
+                                float* g_flow_params, float* g_globals_partial, float* g_zdirect, float* g_delta,
+                                void* stream);
+
+/* Columns of one g_enc row of cfn_network_bwd_inputs: 2 * round8(3 + 6 L_pos) + round8(3 + 6 L_dir) (160 for the
+ * canonical network).  0 for a null handle. */
+int cfn_input_grad_width(const CfnHandle* h);
+
+/* cfn_network_bwd that also writes the gradients of the encoded network inputs: g_enc (B*N, cfn_input_grad_width), fp32,
+ * row m = [d loss/d gamma(p) through layer 0 | through the skip layer (zeros without one) | d loss/d gamma(d) through the
+ * view layer], each block padded to a multiple of 8 columns (pad columns are 0).  The two gamma(p) blocks are kept apart
+ * (cfn_ray_grad_f32 adds them).  grads may be NULL: then no weight gradient is computed and nothing in grads is touched
+ * (a frozen network: about half the backward's dense work); otherwise it is exactly the grads argument of the plain
+ * backward. */
+int cfn_network_bwd_inputs(CfnHandle* h, const float* g_flow_params, int64_t B, int N, void* workspace,
+                           size_t workspace_bytes, float* const* grads, int n_params, float* g_enc, void* stream);
+
+/* g_rays (B,11) = d loss / d rays [o d near far viewdir] from g_enc (cfn_network_bwd_inputs) and g_zdirect / g_delta
+ * (cfn_flow_composite_bwd_rays) of the same pass.  rays, t_vals, t_rand, lindisp and z_vals are what cfn_zvals_f32 was
+ * given and wrote (t_rand NULL = no stratified jitter; it is data and gets no gradient).  One warp per ray, fixed-order
+ * sums: bitwise repeatable. */
+int cfn_ray_grad_f32(const CfnHandle* h, const float* rays, const float* z_vals, const float* t_vals, const float* t_rand,
+                     int lindisp, const float* g_enc, const float* g_zdirect, const float* g_delta, int64_t B, int N,
+                     float* g_rays, void* stream);
+
+/* Adjoint of cfn_rays_from_pose_f32 with the same H, W, focal, ndc, ndc_near: g_rays (H*W,11) -> g_c2w (3,4), the rows
+ * of d loss / d c2w[:3,:4] (near / far are constants).  c2w (12 floats) is in DEVICE memory here.  partials: device
+ * scratch of CFN_POSE_BWD_PARTIALS floats.  Fixed-order block sums and a fixed-order final pass: bitwise repeatable. */
+#define CFN_POSE_BWD_PARTIALS 3072
+int cfn_rays_from_pose_bwd_f32(int H, int W, double focal, const float* c2w, int ndc, double ndc_near, const float* g_rays,
+                               float* partials, float* g_c2w, void* stream);
+
 /* ---- F3: fused optimiser step (torch.optim.Adam, run_nerf_uncertainty_NF.py:339, 1065-1077) ------------------- */
 /* One launch over all n_tensors parameter tensors.  The four pointer arrays and numels live in HOST memory and hold
  * DEVICE pointers / element counts; `step` is the 1-based step count (bias correction), `lr` the already decayed
@@ -281,7 +325,8 @@ int cfn_gemm_f32(int engine, const float* A, int64_t a_rs, int64_t a_cs, const f
  * per row and 32 columns, bits_ld words per row; column n at bit 8 * (n % 4) + (n % 32) / 4) and epilogue 3 reads such a mask (aux_bits) instead of an fp32 aux.
  * split_k > 1: fp32 atomics into a pre-zeroed fp32 C; rowsum (optional, pre-zeroed, M floats) += sum_k A(m,k).
  * Instantiated flavours = the ones the training chain issues (else CFN_EINVAL): K-major x K-major {none, ReLU -> bf16;
- * tanh-mask -> fp32}, K-major x N-major {none, bit-mask -> bf16}, M-major x N-major split-K -> fp32. */
+ * tanh-mask -> fp32}, K-major x N-major {none -> bf16 or fp32 (the input
+ * gradients of cfn_network_bwd_inputs), bit-mask -> bf16}, M-major x N-major split-K -> fp32. */
 int cfn_gemm_bf16(const void* A, int64_t a_rs, int64_t a_cs, const void* B, int64_t b_rs, int64_t b_cs, void* C,
                   int64_t c_rs, int c_bf16, const float* bias, const float* aux, uint32_t* mask_out,
                   const uint32_t* aux_bits, int64_t bits_ld, int64_t M, int N, int64_t K, int epilogue, int split_k,
