@@ -40,6 +40,7 @@ SYMBOLS = {
     "cfn_raw2outputs_f32": (_i32, [_f32p, _f32p, _f32p, _i32, _i32, _f32p, _f32p, _f32p, _f32p, _i64, _i32, _i32, _vp]),
     "cfn_sample_pdf_f32": (_i32, [_f32p, _f32p, _f32p, _f32p, _vp, _i64, _i32, _i32, _vp]),
     "cfn_merge_sorted_f32": (_i32, [_f32p, _f32p, _f32p, _i64, _i32, _i32, _vp]),
+    "cfn_merge_sorted_src_f32": (_i32, [_f32p, _f32p, _f32p, _vp, _i64, _i32, _i32, _vp]),
     "cfn_mean_over_k_f32": (_i32, [_f32p, _f32p, _i64, _i32, _vp]),
     "cfn_trainer_loss_f32": (_i32, [_f32p, _f32p, _f32p, _f32p, _i64, _i64, _i32, C.c_float, C.c_float, _f32p, _f32p, _f32p,
                                     _vp]),
@@ -53,6 +54,8 @@ SYMBOLS = {
     "cfn_input_grad_width": (_i32, [_vp]),
     "cfn_network_bwd_inputs": (_i32, [_vp, _f32p, _i64, _i32, _vp, _sz, C.POINTER(_vp), _i32, _f32p, _vp]),
     "cfn_ray_grad_f32": (_i32, [_vp, _f32p, _f32p, _f32p, _f32p, _i32, _f32p, _f32p, _f32p, _i64, _i32, _f32p, _vp]),
+    "cfn_ray_grad_merged_f32": (_i32, [_vp, _f32p, _f32p, _vp, _i32, _f32p, _f32p, _i32, _f32p, _f32p, _f32p, _i64, _i32,
+                                       _f32p, _vp]),
     "cfn_rays_from_pose_bwd_f32": (_i32, [_i32, _i32, C.c_double, _f32p, _i32, C.c_double, _f32p, _f32p, _f32p, _vp]),
     "cfn_adam_step_f32":(_i32, [_i32, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_i64),
                           C.c_float, C.c_float, C.c_float, C.c_float, _i32, C.c_float, _vp]),

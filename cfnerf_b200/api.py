@@ -111,8 +111,9 @@ def sample_pdf(bins, weights, N_samples, det=False, pytest=False, *, u=None, ret
     return (out, below) if return_below else out
 
 
-def merge_sorted(z_a, z_b):
-    """sort(cat[z_a, z_b], -1) per ray."""
+def merge_sorted(z_a, z_b, *, return_src=False):
+    """sort(cat[z_a, z_b], -1) per ray.  return_src: also the permutation src (B,Na+Nb) int32, the index into
+    cat[z_a, z_b] of every output slot (torch.sort(stable=True).indices) -> (out, src)."""
     lib = _lib.load()
     dev = z_a.device
     z_a, z_b = _f32c(z_a, dev), _f32c(z_b, dev)
@@ -120,6 +121,11 @@ def merge_sorted(z_a, z_b):
     Nb = z_b.shape[1]
     out = torch.empty(B, Na + Nb, dtype=torch.float32, device=dev)
     with torch.cuda.device(dev):
+        if return_src:
+            src = torch.empty(B, Na + Nb, dtype=torch.int32, device=dev)
+            check(lib.cfn_merge_sorted_src_f32(_ptr(z_a), _ptr(z_b), _ptr(out), _ptr(src), B, Na, Nb, _stream()),
+                  "cfn_merge_sorted_src_f32")
+            return out, src
         check(lib.cfn_merge_sorted_f32(_ptr(z_a), _ptr(z_b), _ptr(out), B, Na, Nb, _stream()), "cfn_merge_sorted_f32")
     return out
 
@@ -142,9 +148,11 @@ class _RenderTrainFn(torch.autograd.Function):
     """forward: cfn_network_fwd(save) + cfn_flow_composite_fwd(train); backward: cfn_flow_composite_bwd +
     cfn_network_bwd.  The parameters are inputs so that autograd writes into the reference module's own .grad.
     eps_a (G,K) / eps_c (G,K,3): one latent draw per group of `group_rays` rays (0: G = 1).
-    sched = (t_vals, t_rand or None, lindisp): what made z_vals from the rays.  When the rays need a gradient the
-    backward runs the ray flavour instead (cfn_flow_composite_bwd_rays + cfn_network_bwd_inputs + cfn_ray_grad_f32),
-    without any weight gradient when no parameter needs one."""
+    sched = (t_vals, t_rand or None, lindisp, merged): what made z_vals from the rays.  merged is None for a grid
+    cfn_zvals_f32 made, or (src, Nc) for the fine pass's merged grid (src from merge_sorted(..., return_src=True), kept
+    alive here for the backward; t_vals / t_rand are then the coarse pass's).  When the rays need a gradient the
+    backward runs the ray flavour instead (cfn_flow_composite_bwd_rays + cfn_network_bwd_inputs + cfn_ray_grad_f32 or
+    cfn_ray_grad_merged_f32), without any weight gradient when no parameter needs one."""
 
     @staticmethod
     def forward(ctx, eng: Engine, rays, z_vals, eps_a, eps_c, white_bkgd, want_weights, group_rays, sched, *params):
@@ -183,8 +191,8 @@ class _RenderTrainFn(torch.autograd.Function):
                     eps_group_rays=ctx.group_rays, seg_sums=sg if sg.numel() else None, ray_terms=True)
                 need_w = any(ctx.needs_input_grad[9:])
                 grads, g_enc = eng.network_bwd_inputs(g_fp, B, N, ws, weights=need_w)
-                t_vals, t_rand, lindisp = ctx.sched
-                g_rays = eng.ray_grad(rays, z_vals, t_vals, t_rand, lindisp, g_enc, g_zd, g_dl)
+                t_vals, t_rand, lindisp, merged = ctx.sched
+                g_rays = eng.ray_grad(rays, z_vals, t_vals, t_rand, lindisp, g_enc, g_zd, g_dl, merged=merged)
                 if not need_w:
                     return (None, g_rays) + (None,) * (7 + len(eng.params))
         gg = g_glob.sum(0)
@@ -321,7 +329,8 @@ def run_network(inputs, viewdirs, fn, is_val, is_test, embed_fn=None, embeddirs_
 def render_rays(ray_batch, network_fn, network_query_fn=None, N_samples=128, is_train=False, uniformsample=False,
                 retraw=False, lindisp=False, K_samples=0, perturb=0., N_importance=0, network_fine=None,
                 white_bkgd=False, raw_noise_std=0., verbose=False, pytest=False, *, t_rand=None, eps_alpha=None,
-                eps_rgb=None, u=None, precision=None, want_weights=False, want_kstats=False, netchunk=None):
+                eps_rgb=None, u=None, precision=None, want_weights=False, want_kstats=False, netchunk=None,
+                detach_z_samples=False):
     """main:457-553, plus the coarse+fine extension when N_importance > 0 and network_fine is given (SURVEY A9/A10).
 
     Returns the reference dict: rgb_map (B,3,K), disp_map (B,K), depth_map (B,K); when is_train also raw
@@ -333,16 +342,23 @@ def render_rays(ray_batch, network_fn, network_query_fn=None, N_samples=128, is_
     network call of netchunk points draws its own latent noise (models.py:233-251) and returns its own entropy scalar,
     so a training batch of more than netchunk / N rays uses one (eps_alpha, eps_rgb) pair per group of netchunk / N
     rays, drawn in the reference's order, and `loss_entropy` carries one scalar per group.  `eps_alpha` / `eps_rgb` may
-    be passed as (K,1) / (K,3) (one call) or (G,K,1) / (G,K,3) (one pair per call)."""
+    be passed as (K,1) / (K,3) (one call) or (G,K,1) / (G,K,3) (one pair per call).
+
+    A ray_batch that requires a gradient makes the maps differentiable in it (F7).  For the coarse+fine pass this needs
+    detach_z_samples=True: upstream nerf-pytorch's hierarchical step, in which the resampled depths (sample_pdf of the
+    detached coarse weights) are constants and the coarse depths keep their gradient through the sort.  Both passes
+    then add their terms to ray_batch.grad; about 26 KB of saved activations per point on the tf32 chain, for the coarse
+    and the fine points alike."""
     module = _unwrap(network_fn)
     dev = ray_batch.device
     hier = N_importance > 0 and network_fine is not None
     # F7: the rays need a gradient -> the training kernels run in test mode too (the reference's render_rays is one
-    # autograd graph from ray_batch in both modes); single-network passes only
+    # autograd graph from ray_batch in both modes); the coarse+fine pass only with the resampled depths held constant
     ray_grad = ray_batch.requires_grad and torch.is_grad_enabled()
-    if ray_grad and hier:
-        raise ValueError("ray gradients cover single-network passes: the coarse+fine pass (N_importance > 0 with "
-                         "network_fine) is not differentiable in ray_batch")
+    if ray_grad and hier and not detach_z_samples:
+        raise ValueError("ray gradients cover single-network passes by default: the coarse+fine pass (N_importance > 0 "
+                         "with network_fine) is differentiable in ray_batch only with detach_z_samples=True (the "
+                         "resampled depths held constant, as upstream nerf-pytorch)")
     if ray_grad and want_kstats:
         raise ValueError("want_kstats is not available together with ray gradients (ray_batch.requires_grad)")
     prec = precision or DEFAULT_PRECISION
@@ -388,12 +404,12 @@ def render_rays(ray_batch, network_fn, network_query_fn=None, N_samples=128, is_
             # the reference draws noise here and never adds it (main:432-442); same count keeps the RNG stream aligned
             torch.randn(B, N_samples, eng.K, device=dev)
 
-        def one_pass(net, z, train, need_w):
+        def one_pass(net, z, train, need_w, merged=None):
             e = engine_for(net, dev, prec)
             N = z.shape[1]
             if train or ray_grad:
                 rgb, disp, depth, raw, ld, w = _RenderTrainFn.apply(e, rays, z, eps_a, eps_c, bool(white_bkgd),
-                                                                    need_w, group_rays, sched, *e.params)
+                                                                    need_w, group_rays, sched + (merged,), *e.params)
                 if not train:       # test mode with ray gradients: the maps (and weights), as the reference returns
                     return dict(rgb_map=rgb, disp_map=disp, depth_map=depth, weights=w if need_w else None)
                 ent = _entropy_rows(_unwrap(net), eps_a, eps_c, ld, B, N, e.K, group_rays)    # models.py:286-291
@@ -423,8 +439,11 @@ def render_rays(ray_batch, network_fn, network_query_fn=None, N_samples=128, is_
                 z_mid = .5 * (z_vals[..., 1:] + z_vals[..., :-1])
                 z_samples = sample_pdf(z_mid, w_mean[..., 1:-1], N_importance, det=(perturb == 0.), pytest=pytest,
                                        u=u)
-                z_all = merge_sorted(z_vals, z_samples)
-            o = one_pass(network_fine, z_all, is_train, want_weights)
+                if ray_grad:        # the fine pass's ray gradient routes each slot back through the permutation
+                    z_all, src = merge_sorted(z_vals, z_samples, return_src=True)
+                else:
+                    z_all = merge_sorted(z_vals, z_samples)
+            o = one_pass(network_fine, z_all, is_train, want_weights, (src, N_samples) if ray_grad else None)
             ret = {"rgb_map": o["rgb_map"], "disp_map": o["disp_map"], "depth_map": o["depth_map"],
                    "rgb0": oc["rgb_map"], "disp0": oc["disp_map"], "depth0": oc["depth_map"],
                    "z_samples": z_samples, "z_vals": z_all}

@@ -392,7 +392,15 @@ extern "C" int cfn_merge_sorted_f32(const float* a, const float* b, float* out, 
                                     void* stream) {
   CFN_CHECK_ARG(B >= 0 && Na >= 0 && Nb >= 0, "cfn_merge_sorted_f32: negative size");
   CFN_CHECK_ARG(B == 0 || ((a || Na == 0) && (b || Nb == 0) && (out || Na + Nb == 0)), "cfn_merge_sorted_f32: null argument");
-  return launch_merge_sorted(a, b, out, B, Na, Nb, (cudaStream_t)stream);
+  return launch_merge_sorted(a, b, out, nullptr, B, Na, Nb, (cudaStream_t)stream);
+}
+
+extern "C" int cfn_merge_sorted_src_f32(const float* a, const float* b, float* out, int32_t* src, int64_t B, int Na, int Nb,
+                                        void* stream) {
+  CFN_CHECK_ARG(B >= 0 && Na >= 0 && Nb >= 0, "cfn_merge_sorted_src_f32: negative size");
+  CFN_CHECK_ARG(B == 0 || Na + Nb == 0 || ((a || Na == 0) && (b || Nb == 0) && out && src),
+                "cfn_merge_sorted_src_f32: null argument");
+  return launch_merge_sorted(a, b, out, src, B, Na, Nb, (cudaStream_t)stream);
 }
 
 extern "C" int cfn_mean_over_k_f32(const float* w, float* out, int64_t rows, int K, void* stream) {
@@ -554,6 +562,19 @@ extern "C" int cfn_ray_grad_f32(const CfnHandle* h, const float* rays, const flo
   CFN_CHECK_ARG(B == 0 || (rays && z_vals && t_vals && g_enc && g_zdirect && g_delta && g_rays), "cfn_ray_grad_f32: null argument");
   return launch_ray_grad(rays, z_vals, t_vals, t_rand, lindisp, g_enc, chain_input_grad_width(h), h->gp, h->skip >= 0 ? 1 : 0,
                          h->cfg.L_pos, h->cfg.L_dir, g_zdirect, g_delta, B, N, g_rays, (cudaStream_t)stream);
+}
+
+extern "C" int cfn_ray_grad_merged_f32(const CfnHandle* h, const float* rays, const float* z_vals, const int32_t* src, int Nc,
+                                       const float* t_vals, const float* t_rand, int lindisp, const float* g_enc,
+                                       const float* g_zdirect, const float* g_delta, int64_t B, int N, float* g_rays,
+                                       void* stream) {
+  CFN_CHECK_ARG(B >= 0 && N >= 1, "cfn_ray_grad_merged_f32: bad shape (B %lld, N %d)", (long long)B, N);
+  CFN_CHECK_ARG(Nc > 0 && Nc <= N, "cfn_ray_grad_merged_f32: Nc %d out of range (0, N = %d]", Nc, N);
+  CFN_CHECK_ARG(h != nullptr, "cfn_ray_grad_merged_f32: null handle");
+  CFN_CHECK_ARG(B == 0 || (rays && z_vals && src && t_vals && g_enc && g_zdirect && g_delta && g_rays),
+                "cfn_ray_grad_merged_f32: null argument");
+  return launch_ray_grad(rays, z_vals, t_vals, t_rand, lindisp, g_enc, chain_input_grad_width(h), h->gp, h->skip >= 0 ? 1 : 0,
+                         h->cfg.L_pos, h->cfg.L_dir, g_zdirect, g_delta, B, N, g_rays, (cudaStream_t)stream, src, Nc);
 }
 
 extern "C" int cfn_rays_from_pose_bwd_f32(int H, int W, double focal, const float* c2w, int ndc, double ndc_near,

@@ -92,7 +92,8 @@ int launch_raw2outputs(const float* raw, const float* z_vals, const float* rays_
                        cudaStream_t s);
 int launch_sample_pdf(const float* bins, const float* weights, const float* u, float* samples, int32_t* below,
                       int64_t B, int M, int Nf, cudaStream_t s);
-int launch_merge_sorted(const float* a, const float* b, float* out, int64_t B, int Na, int Nb, cudaStream_t s);
+int launch_merge_sorted(const float* a, const float* b, float* out, int32_t* src, int64_t B, int Na, int Nb,
+                        cudaStream_t s);
 int launch_trainer_loss(const float* rgb_map, const float* depth_map, const float* target_rgb, const float* target_depth,
                         int64_t B_rgb, int64_t B_depth, int K, float nll_scale, float depth_scale, float* partial, float* g_rgb,
                         float* g_depth, cudaStream_t s);
@@ -115,7 +116,8 @@ int launch_field_stats(int fast_math, int F, int K, const float* globals, const 
 
 int launch_ray_grad(const float* rays, const float* z_vals, const float* t_vals, const float* t_rand, int lindisp,
                     const float* g_enc, int ld_enc, int gp, int has_skip, int L_pos, int L_dir, const float* g_zdirect,
-                    const float* g_delta, int64_t B, int N, float* g_rays, cudaStream_t s);
+                    const float* g_delta, int64_t B, int N, float* g_rays, cudaStream_t s,
+                    const int32_t* src = nullptr, int Nc = 0);
 int launch_rays_from_pose_bwd(int H, int W, double focal, const float* c2w, int ndc, double ndc_near, const float* g_rays,
                               float* partials, float* g_c2w, cudaStream_t s);
 

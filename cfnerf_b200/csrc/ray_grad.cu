@@ -6,7 +6,8 @@
 //   g_o     = sum_n g_p_n
 //   g_d     = sum_n z_n g_p_n + (sum_n g_delta_n dist_n) d / |d|                            (dist_{N-1} = 10)
 //   near/far: g_z_n through zvals_kernel's schedule (linear or lindisp; the stratified mids / lower / upper when t_rand is
-//             given; t_rand itself is data)
+//             given; t_rand itself is data); on a merged coarse+fine grid only the slots taken from the coarse grid,
+//             through the coarse schedule (the MERGED flavour)
 //   viewdir: J_gamma(vd)^T sum_n g_gamma(d)_n                                              (vd is constant along a ray)
 // One warp per ray, lane = sample; every sum runs in a fixed order (lane-sequential, then a fixed xor butterfly), so the
 // result is bitwise repeatable.  The points are recomputed in the forward encoder's fp32 operation order and the
@@ -33,11 +34,17 @@ __device__ __forceinline__ void zsched_grad(float near, float far, float t, int 
   cf = zz * t / (far * far);
 }
 
+// MERGED: z_vals is a merged grid (the fine pass of a coarse+fine render) whose slot n holds element src[b,n] of
+// cat[coarse z (Nc), resampled z]; t_vals (Nc) and t_rand (B,Nc) are the coarse pass's.  A slot taken from the coarse
+// grid chains its g_z through coarse slot src's schedule (stratified neighbours src -+ 1 of the coarse grid); a
+// resampled slot is a constant (sample_pdf is not differentiated) and adds nothing to near / far.  src and Nc come last
+// so that the plain flavour keeps its parameter layout.
+template <bool MERGED>
 __global__ void __launch_bounds__(128)
 ray_grad_kernel(const float* __restrict__ rays, const float* __restrict__ z_vals, const float* __restrict__ t_vals,
                 const float* __restrict__ t_rand, int lindisp, const float* __restrict__ g_enc, int ld_enc, int gp,
                 int has_skip, int L_pos, int L_dir, const float* __restrict__ g_zdirect, const float* __restrict__ g_delta,
-                int64_t B, int N, float* __restrict__ g_rays) {
+                int64_t B, int N, float* __restrict__ g_rays, const int32_t* __restrict__ src, int Nc) {
   __shared__ float s_gd[4][kRayGradMaxDir];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t b = (int64_t)blockIdx.x * 4 + warp;
@@ -79,19 +86,24 @@ ray_grad_kernel(const float* __restrict__ rays, const float* __restrict__ z_vals
 #pragma unroll
     for (int c = 0; c < 3; ++c) { acc[c] += gpt[c]; acc[3 + c] += z * gpt[c]; }
     acc[6] += dl * dist;
-    // z_n through the schedule: lower + (upper - lower) * t_rand with lower / upper the neighbouring mids
-    float cn, cf;
-    zsched_grad(near, far, t_vals[n], lindisp, cn, cf);
-    if (t_rand) {
-      float pn = cn, pf = cf, qn = cn, qf = cf;   // d lower, d upper
-      if (n > 0) { float an, af; zsched_grad(near, far, t_vals[n - 1], lindisp, an, af); pn = 0.5f * (cn + an); pf = 0.5f * (cf + af); }
-      if (n < N - 1) { float an, af; zsched_grad(near, far, t_vals[n + 1], lindisp, an, af); qn = 0.5f * (an + cn); qf = 0.5f * (af + cf); }
-      const float u = t_rand[b * N + n];
-      cn = pn + (qn - pn) * u;
-      cf = pf + (qf - pf) * u;
+    // z_n through the schedule: lower + (upper - lower) * t_rand with lower / upper the neighbouring mids; on a merged
+    // grid the schedule slot is the coarse slot m the sample came from (Ns = Nc slots)
+    const int m = MERGED ? src[b * N + n] : n;
+    const int Ns = MERGED ? Nc : N;
+    if (!MERGED || m < Nc) {
+      float cn, cf;
+      zsched_grad(near, far, t_vals[m], lindisp, cn, cf);
+      if (t_rand) {
+        float pn = cn, pf = cf, qn = cn, qf = cf;   // d lower, d upper
+        if (m > 0) { float an, af; zsched_grad(near, far, t_vals[m - 1], lindisp, an, af); pn = 0.5f * (cn + an); pf = 0.5f * (cf + af); }
+        if (m < Ns - 1) { float an, af; zsched_grad(near, far, t_vals[m + 1], lindisp, an, af); qn = 0.5f * (an + cn); qf = 0.5f * (af + cf); }
+        const float u = t_rand[b * Ns + m];
+        cn = pn + (qn - pn) * u;
+        cf = pf + (qf - pf) * u;
+      }
+      acc[7] += gz * cn;
+      acc[8] += gz * cf;
     }
-    acc[7] += gz * cn;
-    acc[8] += gz * cf;
   }
 #pragma unroll
   for (int j = 0; j < 9; ++j)
@@ -131,11 +143,16 @@ ray_grad_kernel(const float* __restrict__ rays, const float* __restrict__ z_vals
 
 int launch_ray_grad(const float* rays, const float* z_vals, const float* t_vals, const float* t_rand, int lindisp,
                     const float* g_enc, int ld_enc, int gp, int has_skip, int L_pos, int L_dir, const float* g_zdirect,
-                    const float* g_delta, int64_t B, int N, float* g_rays, cudaStream_t s) {
+                    const float* g_delta, int64_t B, int N, float* g_rays, cudaStream_t s, const int32_t* src, int Nc) {
   if (B == 0) return CFN_OK;
   CFN_CHECK_ARG(3 + 6 * L_dir <= kRayGradMaxDir, "ray_grad: multires_views %d unsupported", L_dir);
-  ray_grad_kernel<<<(unsigned)((B + 3) / 4), 128, 0, s>>>(rays, z_vals, t_vals, t_rand, lindisp, g_enc, ld_enc, gp, has_skip,
-                                                         L_pos, L_dir, g_zdirect, g_delta, B, N, g_rays);
+  const unsigned grid = (unsigned)((B + 3) / 4);
+  if (src)
+    ray_grad_kernel<true><<<grid, 128, 0, s>>>(rays, z_vals, t_vals, t_rand, lindisp, g_enc, ld_enc, gp, has_skip, L_pos,
+                                               L_dir, g_zdirect, g_delta, B, N, g_rays, src, Nc);
+  else
+    ray_grad_kernel<false><<<grid, 128, 0, s>>>(rays, z_vals, t_vals, t_rand, lindisp, g_enc, ld_enc, gp, has_skip, L_pos,
+                                                L_dir, g_zdirect, g_delta, B, N, g_rays, nullptr, 0);
   CFN_LAUNCH_CHECK();
   return CFN_OK;
 }

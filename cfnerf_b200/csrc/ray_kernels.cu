@@ -352,9 +352,13 @@ int launch_sample_pdf(const float* bins, const float* weights, const float* u, f
   return CFN_OK;
 }
 
-// sort(cat[a,b]) per ray by ranking: element i goes to position #{j : v_j < v_i or (v_j == v_i and j < i)}.
+// sort(cat[a,b]) per ray by ranking: element i goes to position #{j : v_j < v_i or (v_j == v_i and j < i)}, which is
+// torch.sort(stable=True).  SRC also writes src[rank] = i, the index into cat[a,b] of every output slot (the ray
+// gradient of a merged grid routes each slot's g_z back through it); src is the last parameter so that the values-only
+// flavour keeps its parameter layout.
+template <bool SRC>
 __global__ void merge_sorted_kernel(const float* __restrict__ a, const float* __restrict__ b, float* __restrict__ out,
-                                    int Na, int Nb) {
+                                    int Na, int Nb, int32_t* __restrict__ src) {
   extern __shared__ float v[];
   int64_t ray = blockIdx.x;
   int T = Na + Nb;
@@ -368,15 +372,20 @@ __global__ void merge_sorted_kernel(const float* __restrict__ a, const float* __
       rank += (y < x) || (y == x && j < i);
     }
     out[ray * T + rank] = x;
+    if (SRC) src[ray * T + rank] = i;
   }
 }
 
-int launch_merge_sorted(const float* a, const float* b, float* out, int64_t B, int Na, int Nb, cudaStream_t s) {
+int launch_merge_sorted(const float* a, const float* b, float* out, int32_t* src, int64_t B, int Na, int Nb,
+                        cudaStream_t s) {
   int T = Na + Nb;
   if (B == 0 || T == 0) return CFN_OK;
   CFN_CHECK_ARG(T >= 1 && T <= 8192, "merge_sorted: unsupported size %d", T);
   int threads = T < 256 ? ((T + 31) / 32) * 32 : 256;
-  merge_sorted_kernel<<<(unsigned)B, threads, (size_t)T * sizeof(float), s>>>(a, b, out, Na, Nb);
+  if (src)
+    merge_sorted_kernel<true><<<(unsigned)B, threads, (size_t)T * sizeof(float), s>>>(a, b, out, Na, Nb, src);
+  else
+    merge_sorted_kernel<false><<<(unsigned)B, threads, (size_t)T * sizeof(float), s>>>(a, b, out, Na, Nb, nullptr);
   CFN_LAUNCH_CHECK();
   return CFN_OK;
 }

@@ -238,10 +238,18 @@ class Engine:
                                               _ptr(g_enc), _stream()), "cfn_network_bwd_inputs")
         return grads, g_enc
 
-    def ray_grad(self, rays, z_vals, t_vals, t_rand, lindisp: bool, g_enc, g_zdirect, g_delta):
-        """-> g_rays (B,11) = d loss / d [o d near far viewdir] (cfn_ray_grad_f32)."""
+    def ray_grad(self, rays, z_vals, t_vals, t_rand, lindisp: bool, g_enc, g_zdirect, g_delta, merged=None):
+        """-> g_rays (B,11) = d loss / d [o d near far viewdir] (cfn_ray_grad_f32).  merged=(src, Nc): z_vals is the fine
+        pass's merged grid, src (B,N) int32 its permutation (merge_sorted(..., return_src=True)) and t_vals / t_rand the
+        coarse pass's (cfn_ray_grad_merged_f32)."""
         B, N = z_vals.shape
         out = torch.empty(B, 11, dtype=torch.float32, device=self.device)
+        if merged is not None:
+            src, Nc = merged
+            check(self.lib.cfn_ray_grad_merged_f32(self.h, _ptr(rays), _ptr(z_vals), _ptr(src), int(Nc), _ptr(t_vals),
+                                                   _ptr(t_rand), int(bool(lindisp)), _ptr(g_enc), _ptr(g_zdirect),
+                                                   _ptr(g_delta), B, N, _ptr(out), _stream()), "cfn_ray_grad_merged_f32")
+            return out
         check(self.lib.cfn_ray_grad_f32(self.h, _ptr(rays), _ptr(z_vals), _ptr(t_vals), _ptr(t_rand), int(bool(lindisp)),
                                         _ptr(g_enc), _ptr(g_zdirect), _ptr(g_delta), B, N, _ptr(out), _stream()),
               "cfn_ray_grad_f32")

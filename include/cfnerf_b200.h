@@ -182,6 +182,11 @@ int cfn_sample_pdf_f32(const float* bins, const float* weights, const float* u, 
                        int64_t B, int M, int Nf, void* stream);
 /* out (B,Na+Nb) = sort(cat[a (B,Na), b (B,Nb)]) per row (values only). */
 int cfn_merge_sorted_f32(const float* a, const float* b, float* out, int64_t B, int Na, int Nb, void* stream);
+/* cfn_merge_sorted_f32 that also writes src (B,Na+Nb) int32: the index into cat[a, b] of every output slot (ties keep
+ * the a-before-b order, i.e. torch.sort(stable=True)); out holds the same values bit for bit.  The permutation a ray
+ * gradient on a merged grid needs (cfn_ray_grad_merged_f32, F7).  Detected by the symbol (cfn_version() stays 103). */
+int cfn_merge_sorted_src_f32(const float* a, const float* b, float* out, int32_t* src, int64_t B, int Na, int Nb,
+                             void* stream);
 /* mean over K of weights (B,N,K) -> (B,N)  (the shared fine grid decision, SURVEY.md A9) */
 int cfn_mean_over_k_f32(const float* w, float* out, int64_t rows, int K, void* stream);
 
@@ -238,6 +243,10 @@ int cfn_field_stats_f32(const CfnHandle* h, const float* flow_params, const floa
  * point checks its arguments before any CUDA call.  The calls chain to d loss / d ray_batch for one single-network
  * training-path pass (cfn_network_fwd with save_for_backward + the training flavour of cfn_flow_composite_fwd):
  *   cfn_flow_composite_bwd_rays -> cfn_network_bwd_inputs -> cfn_ray_grad_f32 [-> cfn_rays_from_pose_bwd_f32].
+ * A coarse+fine render is two such passes whose g_rays add up.  The coarse pass chains as above.  The fine pass runs on
+ * z_all = cfn_merge_sorted_src_f32(coarse z_vals, z_samples) -> (z_all, src), with the resampled depths z_samples
+ * (cfn_sample_pdf_f32) held constant, and ends in the merged-grid reduction:
+ *   cfn_flow_composite_bwd_rays -> cfn_network_bwd_inputs -> cfn_ray_grad_merged_f32(src, Nc, coarse t_vals / t_rand).
  *
  * cfn_flow_composite_bwd with the same arguments and results, plus two per-sample sums over k (written, not added):
  * g_zdirect (B,N) = sum_k d loss/d depth_map[b,k] * weights[b,n,k] (the depth map's direct z term) and g_delta (B,N) =
@@ -269,6 +278,16 @@ int cfn_network_bwd_inputs(CfnHandle* h, const float* g_flow_params, int64_t B, 
 int cfn_ray_grad_f32(const CfnHandle* h, const float* rays, const float* z_vals, const float* t_vals, const float* t_rand,
                      int lindisp, const float* g_enc, const float* g_zdirect, const float* g_delta, int64_t B, int N,
                      float* g_rays, void* stream);
+
+/* cfn_ray_grad_f32 for the fine pass of a coarse+fine render: z_vals (B,N) is the merged grid and src (B,N) the
+ * permutation cfn_merge_sorted_src_f32 wrote with a = the coarse z_vals (B,Nc), 0 < Nc <= N.  t_vals (Nc), t_rand (B,Nc or
+ * NULL) and lindisp are what made the coarse z_vals.  A slot with src < Nc chains its d loss / d z through coarse slot
+ * src's schedule (stratified neighbours src -+ 1 of the coarse grid); a slot with src >= Nc is a resampled depth, a
+ * constant: it adds nothing to near / far.  o, d and viewdir get the terms of every slot.  Fixed-order sums: bitwise
+ * repeatable. */
+int cfn_ray_grad_merged_f32(const CfnHandle* h, const float* rays, const float* z_vals, const int32_t* src, int Nc,
+                            const float* t_vals, const float* t_rand, int lindisp, const float* g_enc, const float* g_zdirect,
+                            const float* g_delta, int64_t B, int N, float* g_rays, void* stream);
 
 /* Adjoint of cfn_rays_from_pose_f32 with the same H, W, focal, ndc, ndc_near: g_rays (H*W,11) -> g_c2w (3,4), the rows
  * of d loss / d c2w[:3,:4] (near / far are constants).  c2w (12 floats) is in DEVICE memory here.  partials: device
